@@ -2,7 +2,7 @@
 """bench.py — SE env-steps/s of the NES inner loop (BASELINE.json metric) on N B200s of one node.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload NAME] [--extras all|none]
-                    [--scaling weak|strong] [--population P]
+                    [--scaling weak|strong] [--population P] [--dump-outputs DIR]
 
 One "step" = one NES generation's population evaluation over one batch of synthetic input: every member's SE is
 perturbed from the Philox stream (theta, theta+eps, theta-eps) and every resulting lane runs a complete, bounded
@@ -343,10 +343,42 @@ class Dist(object):
             self.dist.destroy_process_group()
 
 
-def measure_vary_hp(D, steps, warmup, members_per_gpu=0, ffma_peak=None):
+DUMP_BYTES = 64 << 20          # all files of one --dump-outputs directory together
+
+
+def lane_fields(res, order=None):
+    """The fields of a lane-result structured array (ops.lane_out_dtype) as separate arrays, optionally re-ordered."""
+    return {"lane_" + k: res[k] if order is None else res[k][order] for k in res.dtype.names}
+
+
+def dump_outputs(out_dir, arrays):
+    """Writes each array as out_dir/<name>.npy: float32 stays float32, every other dtype becomes float64.  The files share
+    DUMP_BYTES: arrays are taken smallest first, each may use an equal share of what is left, and one that does not fit keeps
+    a sample of its rows (elements for 1-D arrays) drawn from a fixed seed, with the row indices in <name>_rows.npy, so that
+    two builds run with the same arguments are compared on the same elements."""
+    header = 128                                                   # bytes of one .npy header
+    arrays = {k: np.asarray(a) for k, a in arrays.items()}
+    arrays = {k: a.astype(np.float32 if a.dtype == np.float32 else np.float64) for k, a in arrays.items()}
+    os.makedirs(out_dir, exist_ok=True)
+    left = DUMP_BYTES
+    for n, name in enumerate(sorted(arrays, key=lambda k: (arrays[k].nbytes, k))):
+        a = arrays[name]
+        share = left // (len(arrays) - n) - header
+        if a.nbytes > share:
+            k = max((share - header) // (a.nbytes // a.shape[0] + 8), 1)
+            rows = np.sort(np.random.RandomState(0).choice(a.shape[0], k, replace=False))
+            a = a[rows]
+            np.save(os.path.join(out_dir, name + "_rows.npy"), rows.astype(np.float64))
+            left -= rows.nbytes + header
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+        left -= a.nbytes + header
+
+
+def measure_vary_hp(D, steps, warmup, members_per_gpu=0, ffma_peak=None, outputs=None):
     """BASELINE config 4.  One step = every agent of this rank trained on the SE (virtual-env plateau rule) and tested on
     the real env: one launch per kernel family (register kernel sets by hidden width, general kernel for the rest), per-lane
-    le_lane_cfg; the lane queue of every launch is ordered longest-first."""
+    le_lane_cfg; the lane queue of every launch is ordered longest-first.  `outputs` (a dict) receives the lane results of
+    the last timed step in agent order."""
     import torch
     from learning_environments_b200 import default_configs, ops, vary_hp
     from learning_environments_b200.rng import lane_keys
@@ -395,6 +427,9 @@ def measure_vary_hp(D, steps, warmup, members_per_gpu=0, ffma_peak=None):
                 flop += float(st) * a + float(li) * b
     D.barrier()
     clocks = sampler.stop()
+    if outputs is not None:
+        res = np.concatenate([gr["bufs"].results() for gr in groups])
+        outputs.update(lane_fields(res, np.argsort(np.concatenate([gr["idx"] for gr in groups]))))
     mx, sm = D.max_sum([dev_ms, float(steps_done), flop])
     dev_ms, steps_all, flop_all = mx[0], sm[1], sm[2]
     # end to end through the public API: sampling, H2D of theta / keys / per-lane cfgs, all launches, D2H of the results
@@ -429,9 +464,10 @@ def measure_vary_hp(D, steps, warmup, members_per_gpu=0, ffma_peak=None):
     }
 
 
-def measure_td3(D, steps, warmup, lanes_per_gpu=0, ffma_peak=None):
+def measure_td3(D, steps, warmup, lanes_per_gpu=0, ffma_peak=None, outputs=None):
     """TD3_discrete_vary lanes through le_td3_run_host (HOST buffers in and out: the timed region holds the H2D of the SE / initial
-    nets / keys, the persistent kernel and the D2H of the lane results), wall clock around the call, max over ranks."""
+    nets / keys, the persistent kernel and the D2H of the lane results), wall clock around the call, max over ranks.
+    `outputs` (a dict) receives the arrays le_td3_run_host returned in the last timed step."""
     import copy
     import torch
     from learning_environments_b200 import agents as A, default_configs, ops
@@ -475,6 +511,9 @@ def measure_td3(D, steps, warmup, lanes_per_gpu=0, ffma_peak=None):
     D.barrier()
     sec = time.perf_counter() - t0
     clocks = sampler.stop()
+    if outputs is not None:
+        outputs.update(lane_fields(res["out"]))
+        outputs.update({k: res[k] for k in ("rewards", "lengths", "test_rewards", "actor_final")})
     mx, sm = D.max_sum([sec, float(steps_done), float(learns)])
     sec, steps_all, learns_all = mx[0], sm[1], sm[2]
     achieved = (steps_all * (f_env + f_a) + learns_all * f_learn) / D.world / sec / 1e12
@@ -497,9 +536,12 @@ def measure_td3(D, steps, warmup, lanes_per_gpu=0, ffma_peak=None):
     }
 
 
-def measure_nes(D, workload, steps, warmup, members_per_gpu=0, population=0, lane_override=(), ffma_peak=None, with_e2e=True):
+def measure_nes(D, workload, steps, warmup, members_per_gpu=0, population=0, lane_override=(), ffma_peak=None, with_e2e=True,
+                outputs=None):
     """One NES-generation workload on this process group: device-timed `value`, the generation including the score exchange
-    and the NES update (`with_update`), and (with_e2e) the end-to-end figure through the host API.  Returns the JSON fields."""
+    and the NES update (`with_update`), and (with_e2e) the end-to-end figure through the host API.  Returns the JSON fields.
+    `outputs` (a dict) receives what the last step of the device-timed population evaluation computed: the lane results, the
+    per-episode train and test rings and the perturbed SE / RN parameters the lanes ran on."""
     import torch
     from learning_environments_b200 import ops
     from learning_environments_b200.engine import PopulationEvaluator
@@ -593,6 +635,12 @@ def measure_nes(D, workload, steps, warmup, members_per_gpu=0, population=0, lan
     # ---------------- device-resident: population evaluation only (value) ----------------
     dev_ms, steps_all, learn_all, clocks = timed(launch_resident, 0)
     value = steps_all / (dev_ms * 1e-3)
+    if outputs is not None:
+        b = ev.bufs
+        outputs.update(lane_fields(b.results()))
+        outputs.update(episode_rewards=b.rewards.cpu().numpy(), episode_lengths=b.lengths.cpu().numpy(),
+                       test_rewards=b.test_rewards.cpu().numpy(), test_lengths=b.test_lengths.cpu().numpy(),
+                       env_theta=ev._thetas.cpu().numpy())
 
     # ---------------- device-resident generation INCLUDING the collective and the NES update ----------------
     def generation_with_update(gen):
@@ -671,23 +719,34 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--lane-override", action="append", default=[], metavar="FIELD=VALUE",
                     help="profiling aid: override an le_lane_cfg field (e.g. max_steps=100); recorded in config.overrides")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the timed path of --workload computed in its last timed step as DIR/<name>.npy "
+                         "(rank 0's lanes; at most 64 MB, larger arrays as a seeded row sample)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
+        if args.dump_outputs:
+            ap.error("--dump-outputs writes the outputs of --impl ours")
         return run_reference_arm(args)
     D = Dist()
     from learning_environments_b200 import ops
     ffma_peak = ops.bench_ffma()
     plain = args.workload == "cartpole_se" and not args.lane_override and not args.members_per_gpu and args.scaling == "weak"
     extras = args.extras == "all" or (args.extras == "auto" and plain and not args.no_cpu_baseline)
+    outputs = {} if args.dump_outputs else None
     if args.workload == "vary_hp":
-        line = measure_vary_hp(D, args.steps, args.warmup, args.members_per_gpu, ffma_peak)
+        line = measure_vary_hp(D, args.steps, args.warmup, args.members_per_gpu, ffma_peak, outputs)
         cfg = None
     elif args.workload == "td3_discrete":
-        line = measure_td3(D, args.steps, args.warmup, args.members_per_gpu, ffma_peak)
+        line = measure_td3(D, args.steps, args.warmup, args.members_per_gpu, ffma_peak, outputs)
         cfg = None
     else:
         pop = (args.population or STRONG_POPULATION) if args.scaling == "strong" else 0
-        line, cfg = measure_nes(D, args.workload, args.steps, args.warmup, args.members_per_gpu, pop, args.lane_override, ffma_peak)
+        line, cfg = measure_nes(D, args.workload, args.steps, args.warmup, args.members_per_gpu, pop, args.lane_override, ffma_peak,
+                                outputs=outputs)
+    if outputs is not None and D.rank == 0:
+        dump_outputs(args.dump_outputs, outputs)
     if extras:
         wl = {}
         for name in EXTRA_WORKLOADS:

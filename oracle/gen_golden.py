@@ -155,9 +155,35 @@ def gen_td_update(yaml_name, tag, seed, steps=5, agent=None, **overrides):
     st = agent.optimizer.state_dict()["state"]
     m = np.concatenate([st[i]["exp_avg"].numpy().reshape(-1) for i in range(len(st))])
     v = np.concatenate([st[i]["exp_avg_sq"].numpy().reshape(-1) for i in range(len(st))])
-    np.savez(os.path.join(GOLDEN, "td_update_%s.npz" % tag), q_init=q0, rows=rows, thetas=np.stack(thetas),
-             targets=np.stack(targets), losses=np.array(losses, np.float32), adam_m=m, adam_v=v, yaml=yaml_name,
-             cfg=cfg_bytes(cfg, agent_name, ENV_RN if "reward_env" in yaml_name else ENV_SE))
+    save_td_update(tag, dict(q_init=q0, rows=rows, losses=np.array(losses, np.float32), yaml=yaml_name,
+                             cfg=cfg_bytes(cfg, agent_name, ENV_RN if "reward_env" in yaml_name else ENV_SE)),
+                   dict(thetas=np.stack(thetas), targets=np.stack(targets), adam_m=m, adam_v=v))
+
+
+GOLDEN_FILE_BYTES = 1000000     # no fixture is larger
+
+
+def save_td_update(tag, inputs, after):
+    """Writes td_update_<tag>.npz.  `inputs` (q_init, rows, losses, yaml, cfg) are stored whole.  `after` holds the parameter
+    vectors after the steps (thetas, targets [steps, P], adam_m, adam_v [P]); when storing them whole would make the file larger
+    than GOLDEN_FILE_BYTES they are kept at the sorted parameter indices `param_idx` instead: every bias and the same seeded
+    fraction of every weight matrix, as many as fit."""
+    from learning_environments_b200._abi import LaneCfg
+    size = sum(np.asarray(a).nbytes for a in list(inputs.values()) + list(after.values())) + 4096     # + npy headers
+    if size > GOLDEN_FILE_BYTES:
+        dims = LaneCfg.from_buffer_copy(inputs["cfg"].tobytes()).q_layer_dims()
+        n_bias, n_weight = sum(o for _, o in dims), sum(i * o for i, o in dims)
+        per_index = 4 + sum(a.nbytes // a.shape[-1] for a in after.values())
+        room = (GOLDEN_FILE_BYTES - 4096 - sum(np.asarray(a).nbytes for a in inputs.values())) // per_index - n_bias
+        rng = np.random.RandomState(0)
+        idx, off = [], 0
+        for i, o in dims:
+            idx += [off + np.sort(rng.choice(i * o, max(1, room * i * o // n_weight), replace=False)), off + i * o + np.arange(o)]
+            off += i * o + o
+        assert off == inputs["q_init"].size
+        param_idx = np.concatenate(idx).astype(np.int32)
+        after = dict({k: a[..., param_idx] for k, a in after.items()}, param_idx=param_idx)
+    np.savez(os.path.join(GOLDEN, "td_update_%s.npz" % tag), **inputs, **after)
 
 
 def gen_td3_learn(seed, steps=5, tag="cartpole", yaml_name="default_config_cartpole_syn_env.yaml", **overrides):
@@ -235,6 +261,78 @@ def gen_td3_learn(seed, steps=5, tag="cartpole", yaml_name="default_config_cartp
              expo_target=np.stack(expo_target), expo_actor=np.stack(expo_actor),
              **{"init_" + n: init[n] for n in nets}, **{"after_" + n: np.stack(per_step[n]) for n in nets})
     print("td3_learn: steps", steps, "policy updates", updated, "temps", temps[:2])
+
+
+class _RingRestatement(object):
+    """utils.ReplayBuffer.add / get_all restated (utils.py:24-32: write row ptr, ptr = (ptr + 1) % max_size,
+    size = min(size + 1, max_size); every field stored as float32 rows).  Used only where the reference tree is absent."""
+
+    def __init__(self, dims, max_size):
+        self.rows = [np.zeros((max_size, d), np.float32) for d in dims]
+        self.ptr = self.size = 0
+        self.max_size = max_size
+
+    def add(self, *values):
+        for r, x in zip(self.rows, values):
+            r[self.ptr] = np.asarray(x, np.float32).reshape(-1)
+        self.ptr = (self.ptr + 1) % self.max_size
+        self.size = min(self.size + 1, self.max_size)
+
+    def get_all(self):
+        return [r[:self.size] for r in self.rows]
+
+
+class _MeterRestatement(object):
+    """utils.AverageMeter.get_mean / get_mean_last restated (utils.py:75-105): the mean of the last `num` values, or of the `num`
+    before them, as sum / (count + 1e-9) over however many exist.  Used only where the reference tree is absent."""
+
+    def __init__(self):
+        self.vals = []
+
+    def update(self, v, print_rate=10):
+        self.vals.append(v)
+
+    def _mean(self, num, skip):
+        hi = max(len(self.vals) - skip, 0)
+        w = self.vals[max(hi - num, 0):hi]
+        return sum(w) / (len(w) + 1e-9)
+
+    def get_mean(self, num=10):
+        return self._mean(num, 0)
+
+    def get_mean_last(self, num=10):
+        return self._mean(num, num)
+
+
+def gen_utils_semantics(seed=0, adds=9, max_size=4, updates=25):
+    """utils.ReplayBuffer (ptr / size after every add, get_all()) and utils.AverageMeter (get_mean(10), get_mean_last(10) after
+    every update) on seeded inputs, which are stored with the results.  The reference's own classes where its tree is present;
+    elsewhere the restatements above, and `source` says which."""
+    rng = np.random.RandomState(seed)
+    rb_in = np.zeros((adds, 9), np.float32)          # state[3] action[1] next_state[3] reward[1] done[1]
+    for i in range(adds):
+        rb_in[i] = np.concatenate([rng.rand(3), [i % 2], rng.rand(3), [i], [i % 3 == 0]]).astype(np.float32)
+    meter_in = rng.rand(updates)
+    if rh.reference_available():
+        import torch
+        ref = rh.import_reference()["utils"]
+        rb, meter, source = ref.ReplayBuffer(3, 1, "cpu", max_size=max_size), ref.AverageMeter(""), "reference"
+        cols = [(0, 3), (3, 4), (4, 7), (7, 8)]
+        add = lambda r: rb.add(*[torch.from_numpy(r[a:b].copy()) for a, b in cols], torch.tensor(float(r[8])))
+    else:
+        rb, meter, source = _RingRestatement((3, 1, 3, 1, 1), max_size), _MeterRestatement(), "restatement"
+        add = lambda r: rb.add(r[0:3], r[3:4], r[4:7], r[7:8], r[8:9])
+    ptr_size = []
+    for r in rb_in:
+        add(r)
+        ptr_size.append((rb.ptr, rb.size))
+    out = {"rb_" + k: np.asarray(x, np.float32) for k, x in zip(("state", "action", "next_state", "reward", "done"), rb.get_all())}
+    means = []
+    for v in meter_in:
+        meter.update(v, print_rate=10 ** 9)
+        means.append((meter.get_mean(10), meter.get_mean_last(10)))
+    np.savez(os.path.join(GOLDEN, "utils_semantics.npz"), rb_inputs=rb_in, rb_max_size=max_size, ptr_size=np.array(ptr_size, np.int64),
+             meter_inputs=meter_in, means=np.array(means, np.float64), source=source, **out)
 
 
 def gen_real_env(seed):
@@ -507,6 +605,7 @@ def main():
                                                                          hidden_layer=2, batch_size=16, policy_delay=2, vary_hp=False,
                                                                          same_action_num=2), trace_cap=300, env_kind="real")),
         ("real_env", lambda: gen_real_env(7)),
+        ("utils_semantics", gen_utils_semantics),
         ("trajectory_cartpole_se", lambda: gen_trajectory(CP, "cartpole_se", 11, (0x1234, 0xABCD), "se",
                                                           dict(train_episodes=5, test_episodes=3, init_episodes=1), trace_cap=400)),
         ("trajectory_acrobot_se", lambda: gen_trajectory(AC, "acrobot_se", 12, (0x77, 0x99), "se",

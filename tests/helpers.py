@@ -13,6 +13,12 @@ def load_golden(name):
     return np.load(os.path.join(GOLDEN, name), allow_pickle=False)
 
 
+def param_index(g):
+    """Indices into the parameter vector at which a td_update fixture stores thetas / targets / adam_m / adam_v: all of them,
+    or the fixed sample `param_idx` of a fixture that would otherwise exceed 1 MB (oracle/gen_golden.py save_td_update)."""
+    return g["param_idx"] if "param_idx" in g.files else slice(None)
+
+
 def cfg_from_bytes(arr):
     c = LaneCfg()
     raw = np.ascontiguousarray(arr, np.uint8).tobytes()

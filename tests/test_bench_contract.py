@@ -1,9 +1,12 @@
-"""bench.py contract checks that need no GPU: the reference arm's JSON line and the static structure of our arm's line."""
+"""bench.py contract checks: the reference arm's JSON line, the static structure of our arm's line and --dump-outputs (its last
+check runs our arm on the GPU)."""
 import json
 import os
 import re
 import subprocess
 import sys
+
+import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
@@ -46,3 +49,55 @@ def test_our_arm_line_carries_every_contract_key():
     for key in ("bound", "achieved", "peak", "unit", "frac", "traffic"):
         assert re.search(r'"%s":' % key, body[body.index('"roofline"'):]), key
     assert "no CPU fallback" in src           # our arm refuses to run without a CUDA device
+
+
+def test_dump_outputs_writes_float_arrays_within_the_size_limit(tmp_path, monkeypatch):
+    """--dump-outputs: float32 kept, other dtypes as float64, the directory within DUMP_BYTES, and an array that does not fit cut
+    to the same seeded row sample every time."""
+    import bench
+    import numpy as np
+    monkeypatch.setattr(bench, "DUMP_BYTES", 16 << 10)
+    big = np.arange(8192, dtype=np.float32).reshape(-1, 16)                   # 32 KB, twice the budget
+    arrays = {"lane_train_steps": np.arange(5, dtype=np.int64), "score": np.linspace(0, 1, 5), "big": big}
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), arrays)
+    a, b = tmp_path / "a", tmp_path / "b"
+    assert sorted(p.name for p in a.iterdir()) == ["big.npy", "big_rows.npy", "lane_train_steps.npy", "score.npy"]
+    steps = np.load(a / "lane_train_steps.npy")
+    assert steps.dtype == np.float64 and steps.tolist() == [0, 1, 2, 3, 4]
+    assert np.load(a / "score.npy").dtype == np.float64
+    sample, rows = np.load(a / "big.npy"), np.load(a / "big_rows.npy").astype(np.int64)
+    assert sample.dtype == np.float32 and sample.shape[0] > 100 and np.array_equal(sample, big[rows])
+    assert np.array_equal(rows, np.load(b / "big_rows.npy")) and np.array_equal(sample, np.load(b / "big.npy"))
+    assert sum(p.stat().st_size for p in a.iterdir()) <= bench.DUMP_BYTES
+
+
+def test_steps_below_one_are_refused():
+    out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "0"], cwd=ROOT, capture_output=True, text=True,
+                         timeout=120)
+    assert out.returncode == 2 and "--steps must be at least 1" in out.stderr
+
+
+@pytest.mark.gpu
+def test_dump_outputs_hold_the_timed_step_and_repeat_exactly(tmp_path):
+    """With one timed step the dumped lane results are that step's: their train steps are the JSON line's value x time.  A second
+    run with the same arguments writes the same arrays bit for bit."""
+    import numpy as np
+    lines = []
+    for run in ("a", "b"):
+        out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--workload", "cartpole_se_pop16", "--steps", "1", "--warmup",
+                              "1", "--extras", "none", "--no-cpu-baseline", "--dump-outputs", str(tmp_path / run)], cwd=ROOT,
+                             capture_output=True, text=True, timeout=600)
+        assert out.returncode == 0, out.stderr[-2000:]
+        lines.append(json.loads([l for l in out.stdout.splitlines() if l.startswith("{")][-1]))
+    d, a, b = lines[0], tmp_path / "a", tmp_path / "b"
+    steps = np.load(a / "lane_train_steps.npy")
+    assert steps.shape == (48,) and steps.dtype == np.float64 and steps.min() > 0
+    assert abs(steps.sum() - d["value"] * d["ms_per_step"] * 1e-3) <= 1e-6 * steps.sum()
+    theta = np.load(a / "env_theta.npy")
+    assert theta.dtype == np.float32 and theta.shape[0] == 48 and np.isfinite(theta).all()
+    assert np.allclose(theta[1] + theta[2], 2 * theta[0], atol=1e-6)          # member 0: theta, theta + eps, theta - eps
+    names = sorted(p.name for p in a.iterdir())
+    assert names == sorted(p.name for p in b.iterdir()) and len(names) >= 11
+    for n in names:
+        assert np.array_equal(np.load(a / n), np.load(b / n)), n

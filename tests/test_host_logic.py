@@ -93,25 +93,22 @@ def test_replay_buffer_ring_semantics():
     assert rb.get_all()[0].shape == (5, 2)
 
 
-@pytest.mark.reference
-def test_replay_buffer_and_average_meter_against_the_reference_classes():
-    from oracle import ref_harness as rh
-    ref = rh.import_reference()["utils"]
-    a, b = utils.ReplayBuffer(3, 1, "cpu", max_size=4), ref.ReplayBuffer(3, 1, "cpu", max_size=4)
-    rng = np.random.RandomState(0)
-    for i in range(9):
-        args = [torch.from_numpy(rng.rand(3).astype(np.float32)), torch.tensor([float(i % 2)]),
-                torch.from_numpy(rng.rand(3).astype(np.float32)), torch.tensor([float(i)]), torch.tensor(float(i % 3 == 0))]
-        a.add(*args)
-        b.add(*args)
-        assert (a.ptr, a.size) == (b.ptr, b.size)
-    for x, y in zip(a.get_all(), b.get_all()):
-        assert torch.equal(x, y)
-    ma, mb = utils.AverageMeter(""), ref.AverageMeter("")
-    for v in rng.rand(25):
-        ma.update(v, print_rate=10 ** 9)
-        mb.update(v, print_rate=10 ** 9)
-        assert ma.get_mean(10) == mb.get_mean(10) and ma.get_mean_last(10) == mb.get_mean_last(10)
+def test_replay_buffer_and_average_meter_against_the_reference_classes(golden_dir):
+    """utils.ReplayBuffer and utils.AverageMeter against what the reference's classes return on the same seeded inputs
+    (tests/golden/utils_semantics.npz, oracle/gen_golden.py): ptr / size after every add, get_all(), and get_mean(10) /
+    get_mean_last(10) after every update, all exact."""
+    g = np.load(os.path.join(golden_dir, "utils_semantics.npz"))
+    a = utils.ReplayBuffer(3, 1, "cpu", max_size=int(g["rb_max_size"]))
+    for r, want in zip(g["rb_inputs"], g["ptr_size"]):
+        a.add(torch.from_numpy(r[0:3].copy()), torch.tensor([r[3]]), torch.from_numpy(r[4:7].copy()), torch.tensor([r[7]]),
+              torch.tensor(r[8]))
+        assert [a.ptr, a.size] == want.tolist()
+    for x, k in zip(a.get_all(), ("state", "action", "next_state", "reward", "done")):
+        assert torch.equal(x, torch.from_numpy(g["rb_" + k])), k
+    m = utils.AverageMeter("")
+    for v, want in zip(g["meter_inputs"], g["means"]):
+        m.update(v, print_rate=10 ** 9)
+        assert m.get_mean(10) == want[0] and m.get_mean_last(10) == want[1]
 
 
 def test_vary_hyperparameters_ranges():

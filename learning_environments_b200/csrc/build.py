@@ -14,7 +14,8 @@ SOURCES = ["le_api.cu", "le_general.cu", "le_td3.cu", "le_tc.cu", "le_inst_cp_ta
 HEADERS = ["le_common.cuh", "le_lane.cuh", "le_envpack.cuh", "le_inner_loop.cuh", "le_instance.cuh", "le_general.cuh", "le_tc.cuh", "le_general_api.h", "le_td3_api.h",
            os.path.join("..", "..", "include", "le_b200.h")]
 OUT = os.path.join(HERE, os.environ.get("LE_LIB_NAME", "lible_b200.so"))
-# variant libraries (LE_LIB_NAME + LE_NVCC_EXTRA: A/B kernel experiments) keep their objects apart from the default build
+# a library built under another name (LE_LIB_NAME, e.g. an older build kept for an A/B run, selected by the same variable at run
+# time) keeps its objects apart from the default build
 OBJDIR = os.path.join(HERE, "build") if os.path.basename(OUT) == "lible_b200.so" else os.path.join(HERE, "build", os.path.basename(OUT) + ".d")
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 EXTRA = os.environ.get("LE_NVCC_EXTRA", "").split()

@@ -559,9 +559,8 @@ int le_inner_loop_run(const le_lane_cfg* cfg_dev, int n_cfg, const le_lane_cfg* 
     else if (pl.mw) {
         // the member's SE / RN pack is staged in the CTA's shared memory by one TMA bulk copy per lane when it fits beside the lane state
         const int64_t pack_bytes = c->env_kind == LE_ENV_REAL ? 0 : pl.pack_stride_f * 4;
-        const char* e = getenv("LE_MW_PACK");
         const int64_t lane_smem = pl.mwc ? pl.ops->mwc_smem_bytes : pl.ops->mw_smem_bytes;
-        if (pack_bytes > 0 && lane_smem + pack_bytes <= 227 * 1024 && !(e && e[0] == '0')) P.mw_pack_f4 = (int)(pack_bytes / 16);
+        if (pack_bytes > 0 && lane_smem + pack_bytes <= 227 * 1024) P.mw_pack_f4 = (int)(pack_bytes / 16);
         if (pl.mwc) LE_CUDA_CHECK(pl.ops->launch_inner_mwc(P, pl.slots, st));
         else LE_CUDA_CHECK(pl.ops->launch_inner_mw(P, pl.grid, st));
     }

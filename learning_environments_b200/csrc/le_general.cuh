@@ -83,15 +83,12 @@ struct GActFn {
 // nets with the minibatch as rows, and their input / weight gradients) go to the tcgen05 tensor cores (le_tc.cuh, 3xTF32,
 // fp32 accumulate in TMEM); everything with a short side (first layers K = sd, heads N <= 4, row counts <= 16) stays on
 // the FFMA paths below.  `tcx` is null in kernels that do not own a TMEM allocation (TD3 lanes, single-row forward).
-#ifndef LE_GENERAL_TC
-#define LE_GENERAL_TC 1
-#endif
 // TCX is tc::Ctx* in the tensor-core instantiations of the lane kernels and std::nullptr_t everywhere else: kernels that do
 // not own a TMEM allocation contain no tcgen05 code at all (a kernel that allocates TMEM is limited to ONE resident CTA per SM
 // by the runtime, measured with tools/ubench/occ_tmem.cu, so the FFMA instantiations keep their two CTAs per SM).
 template <typename TCX>
 __device__ __forceinline__ bool g_use_tc(TCX tcx, int I, int J, int L) {
-    if constexpr (std::is_same<TCX, tc::Ctx*>::value) return LE_GENERAL_TC && tcx != nullptr && I >= 64 && J >= 32 && L >= 32;
+    if constexpr (std::is_same<TCX, tc::Ctx*>::value) return tcx != nullptr && I >= 64 && J >= 32 && L >= 32;
     else return false;
 }
 template <typename TCX, typename... Args>

@@ -26,20 +26,16 @@ struct RunParams {
     le_trace trace; int trace_lane;
 };
 
-#ifndef LE_WARPS_PER_CTA
-#define LE_WARPS_PER_CTA 4
-#endif
-constexpr int kWarpsPerCta = LE_WARPS_PER_CTA;
+constexpr int kWarpsPerCta = 4;
 // Fused kernel: U <= 2 -> 2 CTAs x 4 warps per SM (<= 255 registers each); U = 4 needs all 255 registers per thread, so ONE
 // CTA of 8 warps fills the register file (8 x 32 x 255) and still gives every scheduler two warps to alternate between.
-#ifndef LE_WARPS_U4
-#define LE_WARPS_U4 8
-#endif
-template <int U> constexpr int inner_warps() { return U <= 2 ? kWarpsPerCta : LE_WARPS_U4; }
+constexpr int kWarpsU4 = 8;
+constexpr int kMinCtasU2 = 2;
+template <int U> constexpr int inner_warps() { return U <= 2 ? kWarpsPerCta : kWarpsU4; }
 
 
 // Per-warp shared memory: [stage rows | test-phase weight image (aliased)] [Adam m, v] [lane configuration] [reduction]
-template <int SD, int AD, int U, int ROW = -1>
+template <int SD, int AD, int U, bool ROW = false>
 struct SmemWarp {
     using SL = StageLayout<SD>;
     static constexpr int PUP = SD + 1 + AD;           // per-unit record of the test-phase weight image (scalar reads, broadcast)
@@ -49,7 +45,6 @@ struct SmemWarp {
     static constexpr int BUF_F = STAGE_F > QW_F ? STAGE_F : QW_F;
     static constexpr int MV_F = 2 * (U * (SD + 1 + AD) + AD) * 32;
     static constexpr int CFG_F = (sizeof(le_lane_cfg) + 15) / 16 * 4;
-    static constexpr int RED_R = (U <= 2 ? LE_R_U2 : 4);
     static constexpr int RED_F = LaneCore<SD, AD, U, QACT_TANH, ROW>::SMEM_RED_F;   // reduction buffers, or the row-owner region
     static constexpr int FLOATS = BUF_F + MV_F + CFG_F + RED_F;
     static constexpr int OFF_MV = BUF_F, OFF_CFG = BUF_F + MV_F, OFF_RED = BUF_F + MV_F + CFG_F;
@@ -131,9 +126,9 @@ struct FusedLane {
     static constexpr int NPART = CL == 1 ? W : 2 * (W - 1);          // participants of a learn(): pass p goes to participant p % NPART
     static constexpr int NEXS = CL == 1 ? W - 1 : NPART;             // exchange slots (CL == 1: the leader keeps its share in registers)
     static __device__ __forceinline__ void lane_bar(int id) { if constexpr (CL == 1) mw_bar<W>(id); else cluster_bar(); }
-    using Core = LaneCore<SD, AD, U, ACT, (W > 1 ? 1 : -1)>;
+    using Core = LaneCore<SD, AD, U, ACT, (W > 1)>;
     using RL = RowLayout<SD>;
-    using SW = SmemWarp<SD, AD, U, (W > 1 ? 1 : -1)>;
+    using SW = SmemWarp<SD, AD, U, (W > 1)>;
     using SL0 = StageLayout<SD>;
     // multi-warp lanes: per-worker shared memory = a 32-row stage + the row-owner scratch; exchange = gradients, bias gradients, loss
     static constexpr int MW_STAGE_F = 32 * SL0::STAGE_F;
@@ -581,11 +576,8 @@ struct FusedLane {
     }
 };
 
-#ifndef LE_MIN_CTAS_U2
-#define LE_MIN_CTAS_U2 2
-#endif
 template <int SD, int AD, int U, int ACT>
-__global__ void __launch_bounds__(inner_warps<U>() * 32, (U <= 2 ? LE_MIN_CTAS_U2 : 1)) inner_loop_kernel(const RunParams P) {
+__global__ void __launch_bounds__(inner_warps<U>() * 32, (U <= 2 ? kMinCtasU2 : 1)) inner_loop_kernel(const RunParams P) {
     using SW = SmemWarp<SD, AD, U>;
     extern __shared__ __align__(16) float smem_dyn[];
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;

@@ -11,7 +11,7 @@ import sys
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 SOURCES = ["le_api.cu", "le_general.cu", "le_td3.cu", "le_tc.cu", "le_inst_cp_tanh.cu", "le_inst_cp_leaky.cu", "le_inst_ac_tanh.cu", "le_inst_ac_leaky.cu"]
-HEADERS = ["le_common.cuh", "le_lane.cuh", "le_envpack.cuh", "le_inner_loop.cuh", "le_instance.cuh", "le_general.cuh", "le_tc.cuh", "le_general_api.h", "le_td3_api.h",
+HEADERS = ["le_common.cuh", "le_lane.cuh", "le_envpack.cuh", "le_inner_loop.cuh", "le_instance.cuh", "le_cta_lane.cuh", "le_general.cuh", "le_tc.cuh", "le_general_api.h", "le_td3_api.h",
            os.path.join("..", "..", "include", "le_b200.h")]
 OUT = os.path.join(HERE, os.environ.get("LE_LIB_NAME", "lible_b200.so"))
 # a library built under another name (LE_LIB_NAME, e.g. an older build kept for an A/B run, selected by the same variable at run

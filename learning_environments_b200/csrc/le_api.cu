@@ -289,6 +289,35 @@ static bool use_mwc_lanes(const InstanceOps* ops, int n_lanes, int sms) {
     return !(c && c[0] == '0');
 }
 
+// replay ring rows: rb_size, but never more than a lane can add (every episode at max_steps, or the step budget plus one episode)
+static int ring_capacity(const le_lane_cfg* c) {
+    int64_t max_total = (int64_t)c->train_episodes * c->max_steps;
+    if (c->step_budget > 0 && c->step_budget + c->max_steps < max_total) max_total = c->step_budget + c->max_steps;
+    if (max_total < 1) max_total = 1;
+    return (int)((int64_t)c->rb_size < max_total ? c->rb_size : max_total);
+}
+
+// parameters of one SE / RN env network (envs/virtual_env.py, envs/reward_env.py); 0 for the real envs
+static int env_param_count(const le_lane_cfg* c) {
+    const int H = c->env_hidden;
+    if (c->env_kind == LE_ENV_SE) return 3 * H * (c->sd + c->ad + 1) + H * (c->sd + 2) + c->sd + 2;
+    if (c->env_kind == LE_ENV_RN) return H * (c->sd + 2) + 1;
+    return 0;
+}
+
+// n_env SE / RN parameter vectors -> the packed layout the lane kernels read (stride_f floats per env); real envs: nothing
+static cudaError_t pack_env(const InstanceOps* ops, const le_lane_cfg* c, const float* theta, int n_env, float* pack, int64_t stride_f,
+                            cudaStream_t st) {
+    if (c->env_kind == LE_ENV_SE) {
+        float slopes[3];
+        for (int i = 0; i < 3; ++i) slopes[i] = act_slope(c->env_act, c->env_slope[i]);
+        return ops->launch_pack_se(theta, env_param_count(c), n_env, c->env_hidden, slopes, pack, stride_f, st);
+    }
+    if (c->env_kind == LE_ENV_RN)
+        return ops->launch_pack_rn(theta, env_param_count(c), n_env, c->env_hidden, act_slope(c->env_act, c->env_slope[0]), pack, stride_f, st);
+    return cudaSuccess;
+}
+
 static int make_plan(const le_lane_cfg* c, int n_lanes, int n_env, Plan* pl) {
     { const int rc0 = check_env_cfg(c); if (rc0 != LE_OK) return rc0; }
     if (c->batch_size < 1 || c->rb_size < 1 || c->train_episodes < 0 || c->test_episodes < 1 || c->max_steps < 1 || n_lanes < 1) {
@@ -307,10 +336,7 @@ static int make_plan(const le_lane_cfg* c, int n_lanes, int n_env, Plan* pl) {
     int dev = 0, sms = 0;
     LE_CUDA_CHECK(cudaGetDevice(&dev));
     LE_CUDA_CHECK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
-    int64_t max_total = (int64_t)c->train_episodes * c->max_steps;
-    if (c->step_budget > 0 && c->step_budget + c->max_steps < max_total) max_total = c->step_budget + c->max_steps;
-    if (max_total < 1) max_total = 1;
-    pl->ring_cap = (int)((int64_t)c->rb_size < max_total ? c->rb_size : max_total);
+    pl->ring_cap = ring_capacity(c);
     pl->ops = ops;
     if (pl->general) {
         const int rc = general_plan(c, n_lanes, pl->ring_cap, sms, &pl->gp);
@@ -351,12 +377,45 @@ static int make_plan(const le_lane_cfg* c, int n_lanes, int n_env, Plan* pl) {
 using namespace le;
 
 // Owns the private stream and the device arena of a *_host entry point: every early return (LE_CUDA_CHECK) releases both.
+// The arena holds one 256-byte aligned segment per host array (add) and the call's device-only regions (reserve).
 struct HostCall {
+    struct Seg { const void* src; void* dst_host; size_t bytes; size_t off; };
     cudaStream_t st = nullptr;
     char* arena = nullptr;
+    std::vector<Seg> segs;
+    size_t total = 0;
     ~HostCall() {
         if (arena) cudaFreeAsync(arena, st);
         if (st) { cudaStreamSynchronize(st); cudaStreamDestroy(st); }
+    }
+    // segment of `bytes`: filled from host `src` before the run, copied to host `dst` after it (either may be null)
+    size_t add(const void* src, void* dst, size_t bytes) {
+        segs.push_back(Seg{src, dst, bytes, total});
+        total += (bytes + 255) / 256 * 256;
+        return segs.size() - 1;
+    }
+    size_t reserve(size_t bytes) { const size_t off = total; total += bytes; return off; }
+    char* dp(size_t i) const { return segs[i].bytes ? arena + segs[i].off : nullptr; }
+    // creates the stream, allocates the arena and copies the inputs in
+    int stage_in() {
+        LE_CUDA_CHECK(cudaStreamCreateWithFlags(&st, cudaStreamNonBlocking));
+        LE_CUDA_CHECK(cudaMallocAsync((void**)&arena, total, st));
+        for (auto& s : segs)
+            if (s.src && s.bytes) LE_CUDA_CHECK(cudaMemcpyAsync(arena + s.off, s.src, s.bytes, cudaMemcpyHostToDevice, st));
+        return LE_OK;
+    }
+    // after a run that returned rc: copies the outputs out (rc == LE_OK) and waits for the stream
+    int stage_out(int rc, const char* who) {
+        if (rc == LE_OK) {
+            for (auto& s : segs)
+                if (s.dst_host && s.bytes) {
+                    cudaError_t e = cudaMemcpyAsync(s.dst_host, arena + s.off, s.bytes, cudaMemcpyDeviceToHost, st);
+                    if (e != cudaSuccess) { le_set_error("D2H copy failed: %s", cudaGetErrorString(e)); rc = LE_ECUDA; break; }
+                }
+        }
+        cudaError_t e = cudaStreamSynchronize(st);
+        if (e != cudaSuccess && rc == LE_OK) { le_set_error("%s: %s", who, cudaGetErrorString(e)); rc = LE_ECUDA; }
+        return rc;
     }
 };
 
@@ -416,14 +475,13 @@ int le_se_forward(const le_lane_cfg* cfg, const float* theta_dev, int pop, int l
     const InstanceOps* ops = le_find_instance(cfg->sd, cfg->ad, 1, QACT_TANH);
     if (!ops) { le_set_error("no compiled kernel set for state_dim=%d action_dim=%d", cfg->sd, cfg->ad); return LE_EUNSUPPORTED; }
     cudaStream_t st = (cudaStream_t)stream;
-    const int H = cfg->env_hidden;
+    le_lane_cfg c = *cfg;
+    c.env_kind = LE_ENV_SE;
+    const int H = c.env_hidden;
     const int64_t stride_f = ops->se_pack_vec4(H) * 4;
-    const int P_env = 3 * H * (cfg->sd + cfg->ad + 1) + H * (cfg->sd + 2) + cfg->sd + 2;
     float* pack = nullptr;
     LE_CUDA_CHECK(cudaMallocAsync((void**)&pack, (size_t)pop * stride_f * 4, st));
-    float slopes[3];
-    for (int i = 0; i < 3; ++i) slopes[i] = act_slope(cfg->env_act, cfg->env_slope[i]);
-    LE_CUDA_CHECK(ops->launch_pack_se(theta_dev, P_env, pop, H, slopes, pack, stride_f, st));
+    LE_CUDA_CHECK(pack_env(ops, &c, theta_dev, pop, pack, stride_f, st));
     LE_CUDA_CHECK(ops->launch_se_forward((const float4*)pack, stride_f / 4, H, cfg->env_act == LE_ACT_TANH, lanes_per_member, state_dev,
                                          action_dev, next_state_dev, reward_dev, done_dev, pop * lanes_per_member, st));
     LE_CUDA_CHECK(cudaFreeAsync(pack, st));
@@ -442,10 +500,9 @@ int le_rn_reward(const le_lane_cfg* cfg, const float* theta_dev, int pop, int la
     cudaStream_t st = (cudaStream_t)stream;
     const int H = c.env_hidden;
     const int64_t stride_f = ops->rn_pack_vec4(H) * 4;
-    const int P_env = H * (c.sd + 2) + 1;
     float* pack = nullptr;
     LE_CUDA_CHECK(cudaMallocAsync((void**)&pack, (size_t)pop * stride_f * 4, st));
-    LE_CUDA_CHECK(ops->launch_pack_rn(theta_dev, P_env, pop, H, act_slope(c.env_act, c.env_slope[0]), pack, stride_f, st));
+    LE_CUDA_CHECK(pack_env(ops, &c, theta_dev, pop, pack, stride_f, st));
     LE_CUDA_CHECK(ops->launch_rn_reward((const float4*)pack, stride_f / 4, H, c.env_act == LE_ACT_TANH, c.rn_type, (float)c.gamma,
                                         lanes_per_member, state_dev, next_state_dev, real_reward_dev, reward_dev, pop * lanes_per_member, st));
     LE_CUDA_CHECK(cudaFreeAsync(pack, st));
@@ -530,16 +587,7 @@ int le_inner_loop_run(const le_lane_cfg* cfg_dev, int n_cfg, const le_lane_cfg* 
     char* ws = (char*)workspace_dev;
     float* pack = (float*)ws;
     const le_lane_cfg* c = cfg_host0;
-    if (c->env_kind == LE_ENV_SE) {
-        float slopes[3];
-        for (int i = 0; i < 3; ++i) slopes[i] = act_slope(c->env_act, c->env_slope[i]);
-        const int P_env = 3 * c->env_hidden * (c->sd + c->ad + 1) + c->env_hidden * (c->sd + 2) + c->sd + 2;
-        LE_CUDA_CHECK(pl.ops->launch_pack_se(env_theta_dev, P_env, n_env, c->env_hidden, slopes, pack, pl.pack_stride_f, st));
-    } else if (c->env_kind == LE_ENV_RN) {
-        const int P_env = c->env_hidden * (c->sd + 2) + 1;
-        LE_CUDA_CHECK(pl.ops->launch_pack_rn(env_theta_dev, P_env, n_env, c->env_hidden, act_slope(c->env_act, c->env_slope[0]), pack,
-                                             pl.pack_stride_f, st));
-    }
+    LE_CUDA_CHECK(pack_env(pl.ops, c, env_theta_dev, n_env, pack, pl.pack_stride_f, st));
     int* counter = (int*)(ws + pl.off_counter);
     LE_CUDA_CHECK(cudaMemsetAsync(counter, 0, sizeof(int), st));
     RunParams P;
@@ -594,48 +642,27 @@ int le_inner_loop_run_host(const le_lane_cfg* cfgs, int n_cfg, const float* env_
     int rc = make_plan(c, n_lanes, n_env, &pl);
     if (rc != LE_OK) return rc;
     const int Pq = q_params_of(c);
-    const int P_env = c->env_kind == LE_ENV_SE ? 3 * c->env_hidden * (c->sd + c->ad + 1) + c->env_hidden * (c->sd + 2) + c->sd + 2
-                                              : (c->env_kind == LE_ENV_RN ? c->env_hidden * (c->sd + 2) + 1 : 0);
     const int rs = c->train_episodes > 0 ? c->train_episodes : 1;
     HostCall hc;
-    LE_CUDA_CHECK(cudaStreamCreateWithFlags(&hc.st, cudaStreamNonBlocking));
-    cudaStream_t st = hc.st;
-    // one device arena for every array of the call
-    struct Seg { const void* src; void* dst_host; size_t bytes; size_t off; };
-    std::vector<Seg> segs;
-    size_t total = 0;
-    auto add = [&](const void* src, void* dst, size_t bytes) { Seg s{src, dst, bytes, total}; total += (bytes + 255) / 256 * 256; segs.push_back(s); return segs.size() - 1; };
-    const size_t i_cfg = add(cfgs, nullptr, sizeof(le_lane_cfg) * n_cfg);
-    const size_t i_th = add(env_theta, nullptr, P_env > 0 && env_theta ? sizeof(float) * (size_t)P_env * n_env : 0);
-    const size_t i_ei = add(env_index, nullptr, env_index ? sizeof(int32_t) * n_lanes : 0);
-    const size_t i_key = add(keys, nullptr, sizeof(uint32_t) * 2 * n_lanes);
-    const size_t i_qi = add(q_init, nullptr, q_init ? sizeof(float) * (size_t)Pq * n_lanes : 0);
-    const size_t i_qf = add(nullptr, q_final, q_final ? sizeof(float) * (size_t)Pq * n_lanes : 0);
-    const size_t i_out = add(nullptr, out, sizeof(le_lane_out) * n_lanes);
-    const size_t i_rw = add(nullptr, rewards, sizeof(double) * (size_t)rs * n_lanes);
-    const size_t i_ln = add(nullptr, lengths, sizeof(int32_t) * (size_t)rs * n_lanes);
-    const size_t i_tr = add(nullptr, test_rewards, sizeof(double) * (size_t)c->test_episodes * n_lanes);
-    const size_t off_ws = total;
-    total += (size_t)pl.total_bytes;
-    LE_CUDA_CHECK(cudaMallocAsync((void**)&hc.arena, total, st));
-    char* arena = hc.arena;
-    for (auto& s : segs)
-        if (s.src && s.bytes) LE_CUDA_CHECK(cudaMemcpyAsync(arena + s.off, s.src, s.bytes, cudaMemcpyHostToDevice, st));
-    LE_CUDA_CHECK(cudaMemsetAsync(arena + segs[i_rw].off, 0, segs[i_rw].bytes + segs[i_ln].bytes, st));
-    auto dp = [&](size_t i) -> char* { return segs[i].bytes ? arena + segs[i].off : nullptr; };
-    rc = le_inner_loop_run((const le_lane_cfg*)dp(i_cfg), n_cfg, c, (const float*)dp(i_th), n_env, (const int32_t*)dp(i_ei),
-                           (const uint32_t*)dp(i_key), (const float*)dp(i_qi), (float*)dp(i_qf), n_lanes, (le_lane_out*)dp(i_out),
-                           (double*)dp(i_rw), (int32_t*)dp(i_ln), (double*)dp(i_tr), nullptr, arena + off_ws, pl.total_bytes, nullptr, 0, st);
-    if (rc == LE_OK) {
-        for (auto& s : segs)
-            if (s.dst_host && s.bytes) {
-                cudaError_t e = cudaMemcpyAsync(s.dst_host, arena + s.off, s.bytes, cudaMemcpyDeviceToHost, st);
-                if (e != cudaSuccess) { le_set_error("D2H copy failed: %s", cudaGetErrorString(e)); rc = LE_ECUDA; break; }
-            }
-    }
-    cudaError_t e = cudaStreamSynchronize(st);
-    if (e != cudaSuccess && rc == LE_OK) { le_set_error("le_inner_loop_run_host: %s", cudaGetErrorString(e)); rc = LE_ECUDA; }
-    return rc;   // ~HostCall frees the arena and destroys the stream
+    const size_t i_cfg = hc.add(cfgs, nullptr, sizeof(le_lane_cfg) * n_cfg);
+    const size_t i_th = hc.add(env_theta, nullptr, env_theta ? sizeof(float) * (size_t)env_param_count(c) * n_env : 0);
+    const size_t i_ei = hc.add(env_index, nullptr, env_index ? sizeof(int32_t) * n_lanes : 0);
+    const size_t i_key = hc.add(keys, nullptr, sizeof(uint32_t) * 2 * n_lanes);
+    const size_t i_qi = hc.add(q_init, nullptr, q_init ? sizeof(float) * (size_t)Pq * n_lanes : 0);
+    const size_t i_qf = hc.add(nullptr, q_final, q_final ? sizeof(float) * (size_t)Pq * n_lanes : 0);
+    const size_t i_out = hc.add(nullptr, out, sizeof(le_lane_out) * n_lanes);
+    const size_t i_rw = hc.add(nullptr, rewards, sizeof(double) * (size_t)rs * n_lanes);
+    const size_t i_ln = hc.add(nullptr, lengths, sizeof(int32_t) * (size_t)rs * n_lanes);
+    const size_t i_tr = hc.add(nullptr, test_rewards, sizeof(double) * (size_t)c->test_episodes * n_lanes);
+    const size_t off_ws = hc.reserve((size_t)pl.total_bytes);
+    rc = hc.stage_in();
+    if (rc != LE_OK) return rc;
+    LE_CUDA_CHECK(cudaMemsetAsync(hc.arena + hc.segs[i_rw].off, 0, hc.segs[i_rw].bytes + hc.segs[i_ln].bytes, hc.st));
+    rc = le_inner_loop_run((const le_lane_cfg*)hc.dp(i_cfg), n_cfg, c, (const float*)hc.dp(i_th), n_env, (const int32_t*)hc.dp(i_ei),
+                           (const uint32_t*)hc.dp(i_key), (const float*)hc.dp(i_qi), (float*)hc.dp(i_qf), n_lanes, (le_lane_out*)hc.dp(i_out),
+                           (double*)hc.dp(i_rw), (int32_t*)hc.dp(i_ln), (double*)hc.dp(i_tr), nullptr, hc.arena + off_ws, pl.total_bytes, nullptr, 0,
+                           hc.st);
+    return hc.stage_out(rc, "le_inner_loop_run_host");   // ~HostCall frees the arena and destroys the stream
 }
 
 // ---- TD3_discrete_vary lanes ----------------------------------------------------------------------------
@@ -670,88 +697,60 @@ int le_td3_run_host(const le_td3_cfg* cfg, const float* env_theta, int n_env, co
     LE_CUDA_CHECK(cudaSetDevice(device));
     int sms = 0;
     LE_CUDA_CHECK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device));
-    int64_t max_total = (int64_t)c->train_episodes * c->max_steps;
-    if (c->step_budget > 0 && c->step_budget + c->max_steps < max_total) max_total = c->step_budget + c->max_steps;
-    if (max_total < 1) max_total = 1;
-    const int ring_cap = (int)((int64_t)c->rb_size < max_total ? c->rb_size : max_total);
+    const int ring_cap = ring_capacity(c);
     Td3Plan tp;
     rc = td3_plan(cfg, n_lanes, ring_cap, sms, &tp);
     if (rc != LE_OK) return rc;
-    const int P_env = c->env_kind == LE_ENV_SE ? 3 * c->env_hidden * (c->sd + c->ad + 1) + c->env_hidden * (c->sd + 2) + c->sd + 2 : 0;
     if (c->env_kind == LE_ENV_SE && (!env_theta || n_env < 1)) { le_set_error("le_td3_run_host: env_theta is required for SE lanes"); return LE_EINVAL; }
     const int64_t pack_stride_f = (c->env_kind == LE_ENV_SE ? ops->se_pack_vec4(c->env_hidden) : 1) * 4;
     const int rs = c->train_episodes > 0 ? c->train_episodes : 1;
     const int tcap = trace_host ? trace_host->cap : 0;
     HostCall hc;
-    LE_CUDA_CHECK(cudaStreamCreateWithFlags(&hc.st, cudaStreamNonBlocking));
-    cudaStream_t st = hc.st;
-    struct Seg { const void* src; void* dst_host; size_t bytes; size_t off; };
-    std::vector<Seg> segs;
-    size_t total = 0;
-    auto add = [&](const void* src, void* dst, size_t bytes) { Seg s{src, dst, bytes, total}; total += (bytes + 255) / 256 * 256; segs.push_back(s); return segs.size() - 1; };
-    const size_t i_th = add(env_theta, nullptr, P_env > 0 ? sizeof(float) * (size_t)P_env * n_env : 0);
-    const size_t i_ei = add(env_index, nullptr, env_index ? sizeof(int32_t) * n_lanes : 0);
-    const size_t i_key = add(keys, nullptr, sizeof(uint32_t) * 2 * n_lanes);
-    const size_t i_a = add(actor_init, nullptr, sizeof(float) * (size_t)tp.p_actor * n_init);
-    const size_t i_c1 = add(critic1_init, nullptr, sizeof(float) * (size_t)tp.p_critic * n_init);
-    const size_t i_c2 = add(critic2_init, nullptr, sizeof(float) * (size_t)tp.p_critic * n_init);
-    const size_t i_af = add(nullptr, actor_final, actor_final ? sizeof(float) * (size_t)tp.p_actor * n_lanes : 0);
-    const size_t i_out = add(nullptr, out, sizeof(le_lane_out) * n_lanes);
-    const size_t i_rw = add(nullptr, rewards, sizeof(double) * (size_t)rs * n_lanes);
-    const size_t i_ln = add(nullptr, lengths, sizeof(int32_t) * (size_t)rs * n_lanes);
-    const size_t i_tr = add(nullptr, test_rewards, sizeof(double) * (size_t)c->test_episodes * n_lanes);
-    const size_t i_ta = add(nullptr, tcap ? trace_host->action : nullptr, sizeof(int32_t) * (size_t)tcap);
-    const size_t i_te = add(nullptr, tcap ? trace_host->explore : nullptr, sizeof(int32_t) * (size_t)tcap);
-    const size_t i_tn = add(nullptr, tcap ? trace_host->next_state : nullptr, sizeof(float) * (size_t)tcap * c->sd);
-    const size_t i_trw = add(nullptr, tcap ? trace_host->reward : nullptr, sizeof(float) * (size_t)tcap);
-    const size_t i_td = add(nullptr, tcap ? trace_host->done : nullptr, sizeof(float) * (size_t)tcap);
-    const size_t i_tl = add(nullptr, tcap ? trace_host->loss : nullptr, sizeof(float) * (size_t)tcap);
-    const size_t off_pack = total;
-    total += ((size_t)(n_env > 0 ? n_env : 1) * pack_stride_f * 4 + 255) / 256 * 256;
-    const size_t off_counter = total;
-    total += 256;
-    const size_t off_slots = total;
-    total += (size_t)tp.grid * tp.slot_floats * sizeof(float);
-    LE_CUDA_CHECK(cudaMallocAsync((void**)&hc.arena, total, st));
+    const size_t i_th = hc.add(env_theta, nullptr, sizeof(float) * (size_t)env_param_count(c) * n_env);
+    const size_t i_ei = hc.add(env_index, nullptr, env_index ? sizeof(int32_t) * n_lanes : 0);
+    const size_t i_key = hc.add(keys, nullptr, sizeof(uint32_t) * 2 * n_lanes);
+    const size_t i_a = hc.add(actor_init, nullptr, sizeof(float) * (size_t)tp.p_actor * n_init);
+    const size_t i_c1 = hc.add(critic1_init, nullptr, sizeof(float) * (size_t)tp.p_critic * n_init);
+    const size_t i_c2 = hc.add(critic2_init, nullptr, sizeof(float) * (size_t)tp.p_critic * n_init);
+    const size_t i_af = hc.add(nullptr, actor_final, actor_final ? sizeof(float) * (size_t)tp.p_actor * n_lanes : 0);
+    const size_t i_out = hc.add(nullptr, out, sizeof(le_lane_out) * n_lanes);
+    const size_t i_rw = hc.add(nullptr, rewards, sizeof(double) * (size_t)rs * n_lanes);
+    const size_t i_ln = hc.add(nullptr, lengths, sizeof(int32_t) * (size_t)rs * n_lanes);
+    const size_t i_tr = hc.add(nullptr, test_rewards, sizeof(double) * (size_t)c->test_episodes * n_lanes);
+    const size_t i_ta = hc.add(nullptr, tcap ? trace_host->action : nullptr, sizeof(int32_t) * (size_t)tcap);
+    const size_t i_te = hc.add(nullptr, tcap ? trace_host->explore : nullptr, sizeof(int32_t) * (size_t)tcap);
+    const size_t i_tn = hc.add(nullptr, tcap ? trace_host->next_state : nullptr, sizeof(float) * (size_t)tcap * c->sd);
+    const size_t i_trw = hc.add(nullptr, tcap ? trace_host->reward : nullptr, sizeof(float) * (size_t)tcap);
+    const size_t i_td = hc.add(nullptr, tcap ? trace_host->done : nullptr, sizeof(float) * (size_t)tcap);
+    const size_t i_tl = hc.add(nullptr, tcap ? trace_host->loss : nullptr, sizeof(float) * (size_t)tcap);
+    const size_t off_pack = hc.reserve(((size_t)(n_env > 0 ? n_env : 1) * pack_stride_f * 4 + 255) / 256 * 256);
+    const size_t off_counter = hc.reserve(256);
+    const size_t off_slots = hc.reserve((size_t)tp.grid * tp.slot_floats * sizeof(float));
+    rc = hc.stage_in();
+    if (rc != LE_OK) return rc;
     char* arena = hc.arena;
-    for (auto& s : segs)
-        if (s.src && s.bytes) LE_CUDA_CHECK(cudaMemcpyAsync(arena + s.off, s.src, s.bytes, cudaMemcpyHostToDevice, st));
-    LE_CUDA_CHECK(cudaMemsetAsync(arena + segs[i_rw].off, 0, segs[i_rw].bytes + segs[i_ln].bytes, st));
-    if (tcap) LE_CUDA_CHECK(cudaMemsetAsync(arena + segs[i_ta].off, 0xff, off_pack - segs[i_ta].off, st));   /* untouched trace slots: -1 / NaN */
-    LE_CUDA_CHECK(cudaMemsetAsync(arena + off_counter, 0, 256, st));
-    auto dp = [&](size_t i) -> char* { return segs[i].bytes ? arena + segs[i].off : nullptr; };
-    if (c->env_kind == LE_ENV_SE) {
-        float slopes[3];
-        for (int i = 0; i < 3; ++i) slopes[i] = act_slope(c->env_act, c->env_slope[i]);
-        LE_CUDA_CHECK(ops->launch_pack_se((const float*)dp(i_th), P_env, n_env, c->env_hidden, slopes, (float*)(arena + off_pack), pack_stride_f, st));
-    }
+    LE_CUDA_CHECK(cudaMemsetAsync(arena + hc.segs[i_rw].off, 0, hc.segs[i_rw].bytes + hc.segs[i_ln].bytes, hc.st));
+    if (tcap) LE_CUDA_CHECK(cudaMemsetAsync(arena + hc.segs[i_ta].off, 0xff, off_pack - hc.segs[i_ta].off, hc.st));   /* untouched trace slots: -1 / NaN */
+    LE_CUDA_CHECK(cudaMemsetAsync(arena + off_counter, 0, 256, hc.st));
+    LE_CUDA_CHECK(pack_env(ops, c, (const float*)hc.dp(i_th), n_env, (float*)(arena + off_pack), pack_stride_f, hc.st));
     RunParams P;
     memset(&P, 0, sizeof(P));
     P.env_pack = (const float4*)(arena + off_pack); P.env_pack_stride = pack_stride_f / 4;
-    P.env_index = (const int32_t*)dp(i_ei); P.keys = (const uint32_t*)dp(i_key);
-    P.n_lanes = n_lanes; P.out = (le_lane_out*)dp(i_out); P.rewards = (double*)dp(i_rw); P.lengths = (int32_t*)dp(i_ln);
-    P.test_rewards = (double*)dp(i_tr);
+    P.env_index = (const int32_t*)hc.dp(i_ei); P.keys = (const uint32_t*)hc.dp(i_key);
+    P.n_lanes = n_lanes; P.out = (le_lane_out*)hc.dp(i_out); P.rewards = (double*)hc.dp(i_rw); P.lengths = (int32_t*)hc.dp(i_ln);
+    P.test_rewards = (double*)hc.dp(i_tr);
     P.rew_stride = rs; P.test_stride = c->test_episodes;
     P.ring_cap = ring_cap;
     P.work_counter = (int*)(arena + off_counter);
     if (tcap) {
-        P.trace.cap = tcap; P.trace.action = (int32_t*)dp(i_ta); P.trace.explore = (int32_t*)dp(i_te); P.trace.next_state = (float*)dp(i_tn);
-        P.trace.reward = (float*)dp(i_trw); P.trace.done = (float*)dp(i_td); P.trace.loss = (float*)dp(i_tl);
+        P.trace.cap = tcap; P.trace.action = (int32_t*)hc.dp(i_ta); P.trace.explore = (int32_t*)hc.dp(i_te); P.trace.next_state = (float*)hc.dp(i_tn);
+        P.trace.reward = (float*)hc.dp(i_trw); P.trace.done = (float*)hc.dp(i_td); P.trace.loss = (float*)hc.dp(i_tl);
         P.trace_lane = trace_lane;
     }
-    cudaError_t le = td3_launch(cfg, P, (float*)(arena + off_slots), tp, (const float*)dp(i_a), (const float*)dp(i_c1), (const float*)dp(i_c2),
-                                n_init == n_lanes && n_lanes > 1, (float*)dp(i_af), st);
+    cudaError_t le = td3_launch(cfg, P, (float*)(arena + off_slots), tp, (const float*)hc.dp(i_a), (const float*)hc.dp(i_c1),
+                                (const float*)hc.dp(i_c2), n_init == n_lanes && n_lanes > 1, (float*)hc.dp(i_af), hc.st);
     if (le != cudaSuccess) { le_set_error("td3 launch failed: %s", cudaGetErrorString(le)); rc = LE_ECUDA; }
-    if (rc == LE_OK) {
-        for (auto& s : segs)
-            if (s.dst_host && s.bytes) {
-                cudaError_t e = cudaMemcpyAsync(s.dst_host, arena + s.off, s.bytes, cudaMemcpyDeviceToHost, st);
-                if (e != cudaSuccess) { le_set_error("D2H copy failed: %s", cudaGetErrorString(e)); rc = LE_ECUDA; break; }
-            }
-    }
-    cudaError_t e = cudaStreamSynchronize(st);
-    if (e != cudaSuccess && rc == LE_OK) { le_set_error("le_td3_run_host: %s", cudaGetErrorString(e)); rc = LE_ECUDA; }
-    return rc;   // ~HostCall frees the arena and destroys the stream
+    return hc.stage_out(rc, "le_td3_run_host");   // ~HostCall frees the arena and destroys the stream
 }
 
 // ---- NES ----------------------------------------------------------------------------------------------

@@ -5,20 +5,19 @@
 // lane slot's HBM workspace (<= 2.5 MB per slot) and every dense layer with more than 16 rows is a 128x64x16
 // shared-memory-tiled GEMM with an 8x4 register tile of packed fp32x2 accumulators per thread, operands streamed by cp.async
 // (forward NT, input-gradient NN, weight-gradient TN through one strided routine; LE_TC=1: the tcgen05 routine of le_tc.cuh);
-// <= 16 rows (acting, batched test rollouts) take a thin thread-per-column path.  The control flow (episodes, eps-greedy, env step, replay ring, tests, early-out) mirrors
-// le_inner_loop.cuh; scalars are computed redundantly by all threads (uniform), warp 0 runs the SE/RN mat-vec.
+// <= 16 rows (acting, batched test rollouts) take a thin thread-per-column path.  The agent loop (episodes, env step, replay ring, tests, early-out) is
+// cta_lane_loop of le_cta_lane.cuh, shared with the TD3 lanes; GeneralAgent supplies the DDQN pieces.
 //
 // Dueling coupling (models/actor_critic.py:121): q = V + (A - A.mean()) with the mean over the WHOLE batch tensor, so
 // the forward needs a CTA-wide reduction before the TD error and the backward seeds dA = dq*[a=a_r] - sum(dq)/(B*AD).
 #pragma once
 #include <cstddef>
 #include <type_traits>
-#include "le_inner_loop.cuh"
+#include "le_cta_lane.cuh"
 #include "le_tc.cuh"
 
 namespace le {
 
-constexpr int kGThreads = 256;
 constexpr int kGTileM = 128, kGTileN = 64, kGChunk = 16, kGPad = 4;
 constexpr int kGSmemFloats = 2 * kGChunk * (kGTileM + kGPad + kGTileN + kGPad);
 
@@ -476,6 +475,44 @@ struct GSlot {
     int* astar;
 };
 
+// torch.optim.Adam step of one parameter vector (b1pow / b2pow: beta^t after the step count increment); with a target thT,
+// also the Polyak update thT <- tau * th + (1 - tau) * thT.  Same operation order as LaneCore::adam_polyak.
+static __device__ void g_adam(float* th, float* thT, float* m, float* v, const float* grad, int P, const LearnScalars& ls, double b1pow,
+                              double b2pow) {
+    const double bc1 = 1.0 - b1pow, bc2 = 1.0 - b2pow;
+    const float neg_step = (float)(-(ls.lr / bc1));
+    const float bc2s = (float)sqrt(bc2);
+    constexpr int UN = 8;   // parameters in flight per thread (5 loads each)
+    for (int p0 = threadIdx.x; p0 < P; p0 += UN * kGThreads) {
+        float g[UN], mo[UN], vo[UN], t[UN], tt[UN];
+#pragma unroll
+        for (int u = 0; u < UN; ++u) {
+            const int p = p0 + u * kGThreads < P ? p0 + u * kGThreads : p0;
+            g[u] = __ldcg(grad + p); mo[u] = __ldcg(m + p); vo[u] = __ldcg(v + p);
+            t[u] = __ldcg(th + p);
+            if (thT) tt[u] = __ldcg(thT + p);
+        }
+#pragma unroll
+        for (int u = 0; u < UN; ++u) {
+            const int p = p0 + u * kGThreads;
+            if (p < P) {
+                float mm = mo[u] + ls.w1 * (g[u] - mo[u]);
+                float vv = vo[u] * ls.beta2;
+                vv = vv + (ls.w2 * g[u]) * g[u];
+                __stcg(m + p, mm);
+                __stcg(v + p, vv);
+                bool exact = true;
+                float up = adam_update_core(mm, vv, neg_step, bc2s, ls.eps, &exact);
+                if (!exact) up = __fdiv_rn(neg_step * mm, __fdiv_rn(__fsqrt_rn(vv), bc2s) + ls.eps);
+                const float pn = t[u] + up;
+                __stcg(th + p, pn);
+                if (thT) __stcg(thT + p, ls.tau * pn + ls.one_minus_tau * tt[u]);
+            }
+        }
+    }
+    __syncthreads();
+}
+
 // DDQN.learn / DuelingDDQN.learn on the B rows staged in slot.xs / xs2 / misc (misc = [a, r, d, pad] per row)
 template <typename TCX = std::nullptr_t>
 static __device__ float g_td_update(const GNet& n, const GSlot& w, int B, LearnScalars& ls, float* sm, float* red, TCX tcx = nullptr) {
@@ -531,60 +568,20 @@ static __device__ float g_td_update(const GNet& n, const GSlot& w, int B, LearnS
         const int xs = i > 0 ? S : SDs;
         g_layer_bwd(l, w.theta, w.grad, X, xs, w.actA, w.dact, S, B, i > 0 ? w.dact + n.feat[i - 1].y_off : nullptr, S, false, n.slope, sm, tcx);
     }
-    // Adam + Polyak (same operation order as LaneCore::adam_polyak)
     ls.b1pow *= ls.beta1;
     ls.b2pow *= ls.beta2d;
-    const double bc1 = 1.0 - ls.b1pow, bc2 = 1.0 - ls.b2pow;
-    const float neg_step = (float)(-(ls.lr / bc1));
-    const float bc2s = (float)sqrt(bc2);
-    {
-        constexpr int UN = 8;   // parameters in flight per thread (5 loads each)
-        for (int p0 = threadIdx.x; p0 < n.P; p0 += UN * kGThreads) {
-            float g[UN], m[UN], v[UN], th[UN], tt[UN];
-#pragma unroll
-            for (int u = 0; u < UN; ++u) {
-                const int p = p0 + u * kGThreads < n.P ? p0 + u * kGThreads : p0;
-                g[u] = __ldcg(w.grad + p); m[u] = __ldcg(w.m + p); v[u] = __ldcg(w.v + p);
-                th[u] = __ldcg(w.theta + p); tt[u] = __ldcg(w.thetaT + p);
-            }
-#pragma unroll
-            for (int u = 0; u < UN; ++u) {
-                const int p = p0 + u * kGThreads;
-                if (p < n.P) {
-                    float mm = m[u] + ls.w1 * (g[u] - m[u]);
-                    float vv = v[u] * ls.beta2;
-                    vv = vv + (ls.w2 * g[u]) * g[u];
-                    __stcg(w.m + p, mm);
-                    __stcg(w.v + p, vv);
-                    bool exact = true;
-                    float up = adam_update_core(mm, vv, neg_step, bc2s, ls.eps, &exact);
-                    if (!exact) up = __fdiv_rn(neg_step * mm, __fdiv_rn(__fsqrt_rn(vv), bc2s) + ls.eps);
-                    const float pn = th[u] + up;
-                    __stcg(w.theta + p, pn);
-                    __stcg(w.thetaT + p, ls.tau * pn + ls.one_minus_tau * tt[u]);
-                }
-            }
-        }
-    }
-    __syncthreads();
+    g_adam(w.theta, w.thetaT, w.m, w.v, w.grad, n.P, ls, ls.b1pow, ls.b2pow);
     return loss;
 }
 
-// greedy action of ONE state row (select_train/test_action); result uniform across the CTA
-static __device__ int g_greedy_row(const GNet& n, const GSlot& w, const float* state_row /* [sd] in global memory */, float* sm, float* red,
-                            int* ibox) {
+// greedy action of ONE state row (select_train/test_action); every thread takes the argmax, so the result is uniform
+static __device__ int g_greedy_row(const GNet& n, const GSlot& w, const float* state_row /* [sd] in global memory */, float* sm, float* red) {
     g_net_forward(n, w.theta, state_row, n.sd, 1, w.actB, sm);
     g_q_values(n, w.actB, 1, w.q2, red);
-    if (threadIdx.x == 0) {
-        int best = 0;
-        for (int k = 1; k < n.ad; ++k)
-            if (w.q2[k] > w.q2[best]) best = k;
-        *ibox = best;
-    }
-    __syncthreads();
-    const int a = *ibox;
-    __syncthreads();
-    return a;
+    int best = 0;
+    for (int k = 1; k < n.ad; ++k)
+        if (w.q2[k] > w.q2[best]) best = k;
+    return best;
 }
 
 struct GRunParams {
@@ -630,53 +627,34 @@ static __device__ void g_init_layer(const GLayer& l, float* th, uint32_t k0, uin
     }
 }
 
-// TC = false: two CTAs per SM, every dense layer on the FFMA GEMM.  TC = true: the CTA owns 128 TMEM columns and the dense
-// hidden x hidden layers run on tcgen05 (one CTA per SM: the runtime's TMEM occupancy rule).
-template <int SD, int AD, bool TC>
-__global__ void __launch_bounds__(kGThreads, TC ? 1 : 2) general_loop_kernel(const GRunParams G) {
+// DDQN / DuelingDDQN agent (agents/DDQN.py, agents/DuelingDDQN.py) as the hooks of cta_lane_loop: eps-greedy acting on
+// the greedy row, replay rows in RowLayout<SD>, learn = g_td_update.  cfg / n: this lane's configuration and network in shared
+// memory (per-lane q_hidden / q_layers under vary_hp).
+template <int SD, int AD, typename TCX>
+struct GeneralAgent {
     using RL = RowLayout<SD>;
-    __shared__ __align__(16) float sm[kGSmemFloats];
-    __shared__ float red[32];
-    __shared__ __align__(16) float box[16];   // state row / env step results broadcast
-    __shared__ int ibox[4];
-    __shared__ double dred[kGThreads / 32];
-    __shared__ int sred[kGThreads / 32];
-    __shared__ le_lane_cfg cfg_sm;
-    __shared__ GNet net_sm;          // this lane's network (per-lane q_hidden / q_layers under vary_hp)
-    extern __shared__ __align__(128) unsigned char tc_smem[];   // TC: tc::kSmemBytes, operand parts of the tensor-core GEMM
-    tc::Ctx tcs;
-    if constexpr (TC) tcs = tc::ctx_create(tc_smem);
-    typename std::conditional<TC, tc::Ctx*, std::nullptr_t>::type tcx = nullptr;
-    if constexpr (TC) tcx = &tcs;
-    const RunParams& P = G.rp;
-    const GNet& n = net_sm;
-    const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-    const GSlot w = gslot_view(G.slots + (int64_t)blockIdx.x * G.slot_stride, G.net, P.ring_cap, RL::ROWF, G.bmax);   // sized for the maxima (cfg 0)
-    bool first_lane = true;   // the first lane of a CTA slot is static (lane_id == slot), the rest come from the queue counter
-    for (;;) {
-        __syncthreads();
-        if (tid == 0) ibox[0] = first_lane ? (int)blockIdx.x : (int)gridDim.x + atomicAdd(P.work_counter, 1);
-        __syncthreads();
-        const int lane_id = ibox[0];
-        first_lane = false;
-        if (lane_id >= P.n_lanes) break;
+    const RunParams& P;
+    const GSlot w;   // sized for the maxima (cfg 0)
+    le_lane_cfg& cfg;
+    GNet& n;
+    float* sm;
+    float* red;
+    TCX tcx;
+    uint32_t k0, k1;
+    LearnScalars ls;
+    double eps;
+
+    __device__ __forceinline__ const le_lane_cfg& begin_lane(int lane_id, uint32_t key0, uint32_t key1) {
+        const int tid = threadIdx.x;
+        k0 = key0; k1 = key1;
         {
             const uint32_t* src = reinterpret_cast<const uint32_t*>(P.cfg + (P.n_cfg == 1 ? 0 : lane_id));
-            uint32_t* dst = reinterpret_cast<uint32_t*>(&cfg_sm);
+            uint32_t* dst = reinterpret_cast<uint32_t*>(&cfg);
             for (int i = tid; i < (int)(sizeof(le_lane_cfg) / 4); i += kGThreads) dst[i] = src[i];
         }
         __syncthreads();
-        const le_lane_cfg& c = cfg_sm;
-        if (tid == 0) gnet_build(&cfg_sm, &net_sm);
+        if (tid == 0) gnet_build(&cfg, &n);
         __syncthreads();
-        const uint32_t k0 = P.keys[2 * lane_id], k1 = P.keys[2 * lane_id + 1];
-        const float4* pack = P.env_pack + (int64_t)(P.env_index ? P.env_index[lane_id] : 0) * P.env_pack_stride;
-        const bool env_tanh = c.env_act == LE_ACT_TANH;
-        double* rewards = P.rewards + (int64_t)lane_id * P.rew_stride;
-        int32_t* lengths = P.lengths + (int64_t)lane_id * P.rew_stride;
-        double* test_rewards = P.test_rewards + (int64_t)lane_id * P.test_stride;
-        const bool tracing = P.trace.cap > 0 && lane_id == P.trace_lane;
-        // ---- agent construction
         if (P.q_init) { for (int p = tid; p < n.P; p += kGThreads) w.theta[p] = P.q_init[(int64_t)lane_id * P.q_stride + p]; }
         else {
             for (int i = 0; i < n.nfeat; ++i) g_init_layer(n.feat[i], w.theta, k0, k1);
@@ -686,237 +664,97 @@ __global__ void __launch_bounds__(kGThreads, TC ? 1 : 2) general_loop_kernel(con
         __syncthreads();
         for (int p = tid; p < n.P; p += kGThreads) { w.thetaT[p] = w.theta[p]; w.m[p] = 0.f; w.v[p] = 0.f; }
         __syncthreads();
-        LearnScalars ls;
-        fill_learn_scalars(ls, c);
-
-        // greedy test rollouts on the real env, episodes = rows of one batched forward per step
-        auto run_test = [&](int test_call, double* ep_out, int32_t* len_out, int64_t& test_steps) -> double {
-            double total = 0.0;
-            for (int ep0 = 0; ep0 < c.test_episodes; ep0 += 64) {
-                const int M = min(64, c.test_episodes - ep0);
-                double st[4] = {0, 0, 0, 0};
-                float obs[SD];
-                int elapsed = 0, ep_steps = 0;
-                float ep_rew = 0.f;
-                bool running = tid < M;
-                if (tid < M) {
-                    real_reset(c.real_env, philox4x32_10((uint32_t)test_call, (uint32_t)(ep0 + tid), LE_P_RESET_TEST, 0u, k0, k1), st);
-                    real_obs<SD>(c.real_env, st, obs);
-#pragma unroll
-                    for (int i = 0; i < SD; ++i) w.obs[tid * SD + i] = obs[i];
-                }
-                const int K = c.same_action_num > 1 ? c.same_action_num : 1;
-                for (int t = 0; t < c.max_steps; t += K) {
-                    if (!__syncthreads_or(running ? 1 : 0)) break;
-                    g_net_forward(n, w.theta, w.obs, SD, M, w.actB, sm);
-                    g_q_values(n, w.actB, M, w.q2, red);
-                    if (running) {
-                        int best = 0;
-                        for (int k = 1; k < AD; ++k)
-                            if (w.q2[tid * AD + k] > w.q2[tid * AD + best]) best = k;
-                        float r, d;
-                        real_step<SD>(c.real_env, c.max_steps, st, elapsed, best, obs, r, d);
-                        if (K > 1) {
-                            double rsum = (double)r;
-                            for (int k = 1; k < K && !(d > 0.5f); ++k) {
-                                float rk;
-                                real_step<SD>(c.real_env, c.max_steps, st, elapsed, best, obs, rk, d);
-                                rsum += (double)rk;
-                            }
-                            r = (float)rsum;
-                        }
-#pragma unroll
-                        for (int i = 0; i < SD; ++i) w.obs[tid * SD + i] = obs[i];
-                        ep_rew += r;
-                        ep_steps += 1;
-                        if (d > 0.5f) running = false;
-                    }
-                }
-                __syncthreads();
-                float rsum = (tid < M) ? ep_rew : 0.f;
-                if (tid < M) {
-                    if (ep_out) ep_out[ep0 + tid] = (double)ep_rew;
-                    if (len_out) len_out[ep0 + tid] = ep_steps;
-                }
-                // episode rewards are small integers / short fp32 sums: an fp32 CTA sum would round; sum in double via shared memory
-                double dv = (double)rsum;
-                dv = warp_allreduce_sum(dv);
-                int sv = (tid < M) ? ep_steps : 0;
-#pragma unroll
-                for (int mm = 16; mm > 0; mm >>= 1) sv += __shfl_xor_sync(LE_FULL_MASK, sv, mm);
-                __syncthreads();
-                if (lane == 0) { dred[warp] = dv; sred[warp] = sv; }
-                __syncthreads();
-                for (int q = 0; q < kGThreads / 32; ++q) { total += dred[q]; test_steps += sred[q]; }
-                __syncthreads();
-            }
-            return total / (double)c.test_episodes;
-        };
-
-        int rb_ptr = 0, rb_size = 0;
-        int64_t train_steps = 0, learn_iters = 0, test_steps = 0;
-        int test_calls = 0, n_ep = 0, timed_out = 0;
-        double eps = c.eps_init;
-        const bool rule_virtual = (!c.use_test_env) && c.env_kind == LE_ENV_SE;
-        for (int episode = 0; episode < c.train_episodes; ++episode) {
-            if (c.step_budget > 0 && train_steps >= c.step_budget) { timed_out = 1; break; }
-            if (episode == 0) eps = c.eps_init;
-            else { eps *= c.eps_decay; if (eps < c.eps_min) eps = c.eps_min; }
-            double st[4];
-            real_reset(c.real_env, philox4x32_10((uint32_t)episode, 0u, LE_P_RESET_TRAIN, 0u, k0, k1), st);
-            float state[SD];
-            real_obs<SD>(c.real_env, st, state);
-            int elapsed = 0, ep_len = 0;
-            float ep_rew = 0.f;
-            const int K = c.same_action_num > 1 ? c.same_action_num : 1;
-            for (int t = 0; t < c.max_steps; t += K) {
-                const u32x4 wa = philox4x32_10((uint32_t)train_steps, 0u, LE_P_ACT, 0u, k0, k1);
-                const bool explore = ((double)(wa.x >> 8) * (1.0 / 16777216.0)) < eps;
-                int action;
-                float qgap = __int_as_float(0x7fc00000);
-                if (explore) action = (int)__umulhi(wa.y, (uint32_t)AD);
-                else {
-                    __syncthreads();
-                    if (tid < SD) __stcg(w.xs + tid, state[tid]);   // operand rows are read with ld.global.cg: stage in the slot
-                    __syncthreads();
-                    action = g_greedy_row(n, w, w.xs, sm, red, ibox);
-                    if (tracing) {
-                        float q[AD];
-#pragma unroll
-                        for (int k = 0; k < AD; ++k) q[k] = w.q2[k];
-                        qgap = relative_q_gap<AD>(q, action);
-                        __syncthreads();
-                    }
-                }
-                float ns[SD], r = 0.f, d = 0.f;
-                if (c.env_kind == LE_ENV_SE) {
-                    __syncthreads();
-                    if (warp == 0) {   // same_action_num chained SE steps, fp32 reward sum (envs/env_wrapper.py:24-30)
-                        float cur[SD], ns0[SD], r0 = 0.f, d0 = 0.f;
-#pragma unroll
-                        for (int i = 0; i < SD; ++i) cur[i] = state[i];
-                        for (int k = 0; k < K; ++k) {
-                            float rk;
-                            se_step_row<SD, AD>(pack, c.env_hidden, env_tanh, cur, action, lane, ns0, rk, d0);
-                            r0 = k == 0 ? rk : r0 + rk;
-#pragma unroll
-                            for (int i = 0; i < SD; ++i) cur[i] = ns0[i];
-                        }
-                        if (lane == 0) {
-#pragma unroll
-                            for (int i = 0; i < SD; ++i) box[i] = ns0[i];
-                            box[SD] = r0; box[SD + 1] = d0;
-                        }
-                    }
-                    __syncthreads();
-#pragma unroll
-                    for (int i = 0; i < SD; ++i) ns[i] = box[i];
-                    r = box[SD]; d = box[SD + 1];
-                    __syncthreads();
-                } else {   // real branch: python-float reward sum, break on done (envs/env_wrapper.py:56-61)
-                    float cur[SD];
-#pragma unroll
-                    for (int i = 0; i < SD; ++i) cur[i] = state[i];
-                    double rsum = 0.0;
-                    for (int k = 0; k < K; ++k) {
-                        float rr, rk;
-                        real_step<SD>(c.real_env, c.max_steps, st, elapsed, action, ns, rr, d);
-                        if (c.env_kind == LE_ENV_RN && c.rn_type != 0) {
-                            __syncthreads();
-                            if (warp == 0) {
-                                float ps, ps2;
-                                rn_phi2<SD>(pack, c.env_hidden, env_tanh, cur, ns, lane, ps, ps2);
-                                if (lane == 0) box[0] = rn_combine(c.rn_type, ls.gamma, rr, ps, ps2);
-                            }
-                            __syncthreads();
-                            rk = box[0];
-                            __syncthreads();
-                        } else rk = rr;
-                        rsum += (double)rk;
-                        r = K == 1 ? rk : (float)rsum;
-#pragma unroll
-                        for (int i = 0; i < SD; ++i) cur[i] = ns[i];
-                        if (d > 0.5f) break;
-                    }
-                }
-                {   // replay_buffer.add
-                    float rowv[RL::ROWF];
-#pragma unroll
-                    for (int i = 0; i < RL::ROWF; ++i) rowv[i] = 0.f;
-#pragma unroll
-                    for (int i = 0; i < SD; ++i) { rowv[RL::OFF_S + i] = state[i]; rowv[RL::OFF_S2 + i] = ns[i]; }
-                    rowv[RL::OFF_A] = __int_as_float(action); rowv[RL::OFF_R] = r; rowv[RL::OFF_D] = d;
-                    float4* dst = reinterpret_cast<float4*>(w.ring + (int64_t)rb_ptr * RL::ROWF);
-#pragma unroll
-                    for (int q = 0; q < RL::ROW_VEC; ++q)
-                        if (tid == q) __stcg(dst + q, make_float4(rowv[4 * q], rowv[4 * q + 1], rowv[4 * q + 2], rowv[4 * q + 3]));
-                    rb_ptr = (rb_ptr + 1 == P.ring_cap) ? 0 : rb_ptr + 1;
-                    rb_size = rb_size + 1 < P.ring_cap ? rb_size + 1 : P.ring_cap;
-                }
-#pragma unroll
-                for (int i = 0; i < SD; ++i) state[i] = ns[i];
-                ep_rew += r;
-                ep_len += K;
-                float loss = __int_as_float(0x7fc00000);
-                if (episode >= c.init_episodes) {
-                    __syncthreads();
-                    const int B = ls.batch;
-                    for (int b = tid; b < B; b += kGThreads) {   // replay_buffer.sample on the P_SAMPLE stream
-                        const u32x4 wv = philox4x32_10((uint32_t)learn_iters, (uint32_t)(b >> 2), LE_P_SAMPLE, 0u, k0, k1);
-                        const uint32_t idx = __umulhi(pick(wv, b & 3), (uint32_t)rb_size);
-                        const float4* src = reinterpret_cast<const float4*>(w.ring + (int64_t)idx * RL::ROWF);
-                        float rowv[RL::ROWF];
-#pragma unroll
-                        for (int q = 0; q < RL::ROW_VEC; ++q) { const float4 v4 = __ldcg(src + q); rowv[4 * q] = v4.x; rowv[4 * q + 1] = v4.y; rowv[4 * q + 2] = v4.z; rowv[4 * q + 3] = v4.w; }
-#pragma unroll
-                        for (int i = 0; i < SD; ++i) { w.xs[b * SD + i] = rowv[RL::OFF_S + i]; w.xs2[b * SD + i] = rowv[RL::OFF_S2 + i]; }
-                        w.misc[4 * b] = (float)__float_as_int(rowv[RL::OFF_A]); w.misc[4 * b + 1] = rowv[RL::OFF_R]; w.misc[4 * b + 2] = rowv[RL::OFF_D];
-                    }
-                    __syncthreads();
-                    loss = g_td_update(n, w, B, ls, sm, red, tcx);
-                    learn_iters += 1;
-                }
-                if (tracing && train_steps < P.trace.cap && tid == 0) {
-                    const int64_t i = train_steps;
-                    P.trace.action[i] = action; P.trace.explore[i] = explore ? 1 : 0;
-                    P.trace.reward[i] = r; P.trace.done[i] = d; P.trace.loss[i] = loss;
-                    if (P.trace.qgap) P.trace.qgap[i] = qgap;
-#pragma unroll
-                    for (int k = 0; k < SD; ++k) P.trace.next_state[i * SD + k] = ns[k];
-                }
-                train_steps += 1;
-                if (d > 0.5f) break;
-            }
-            double ep_value;
-            if (c.use_test_env) ep_value = run_test(test_calls++, nullptr, nullptr, test_steps);
-            else ep_value = (double)ep_rew;
-            __syncthreads();
-            if (tid == 0) { lengths[n_ep] = ep_len; rewards[n_ep] = ep_value; __threadfence_block(); }
-            n_ep += 1;
-            __syncthreads();
-            if (episode >= c.init_episodes) {
-                const double avg = mean_window(rewards, n_ep, c.early_out_num, 0);
-                bool solved;
-                if (rule_virtual) {
-                    const double avg_last = mean_window(rewards, n_ep, c.early_out_num, c.early_out_num);
-                    solved = (fabs(avg - avg_last) / (fabs(avg_last) + 1e-9) < c.early_out_virtual_diff) &&
-                             (episode >= c.init_episodes + c.early_out_num);
-                } else solved = avg >= c.solved_reward;
-                if (solved) break;
-            }
-        }
-        double score = 0.0;
-        if (c.final_test)
-            score = run_test(test_calls++, test_rewards, P.test_lengths ? P.test_lengths + (int64_t)lane_id * P.test_stride : nullptr, test_steps);
-        __syncthreads();
-        if (P.q_final) for (int p = tid; p < n.P; p += kGThreads) P.q_final[(int64_t)lane_id * P.q_stride + p] = w.theta[p];
-        if (tid == 0) {
-            le_lane_out o;
-            o.n_episodes = n_ep; o.timed_out = timed_out; o.train_steps = train_steps; o.learn_iters = learn_iters;
-            o.test_steps = test_steps; o.score = score;
-            P.out[lane_id] = o;
-        }
+        fill_learn_scalars(ls, cfg);
+        eps = cfg.eps_init;
+        return cfg;
     }
+
+    __device__ __forceinline__ void begin_episode(int episode) { eps = eps_schedule(eps, episode, cfg); }
+
+    __device__ __forceinline__ int train_action(const float (&state)[SD], int, int64_t train_steps, bool tracing, bool& explore, float& qgap,
+                                                float*) {
+        const u32x4 wa = philox4x32_10((uint32_t)train_steps, 0u, LE_P_ACT, 0u, k0, k1);
+        explore = ((double)(wa.x >> 8) * (1.0 / 16777216.0)) < eps;
+        if (explore) return (int)__umulhi(wa.y, (uint32_t)AD);
+        __syncthreads();
+        if (threadIdx.x < SD) __stcg(w.xs + threadIdx.x, state[threadIdx.x]);   // operand rows are read with ld.global.cg: stage in the slot
+        __syncthreads();
+        const int action = g_greedy_row(n, w, w.xs, sm, red);
+        if (tracing) {
+            float q[AD];
+#pragma unroll
+            for (int k = 0; k < AD; ++k) q[k] = w.q2[k];
+            qgap = relative_q_gap<AD>(q, action);
+            __syncthreads();
+        }
+        return action;
+    }
+
+    __device__ __forceinline__ void store_row(int row, const float (&state)[SD], int action, const float (&ns)[SD], float r, float d) {
+        float rowv[RL::ROWF];
+#pragma unroll
+        for (int i = 0; i < RL::ROWF; ++i) rowv[i] = 0.f;
+#pragma unroll
+        for (int i = 0; i < SD; ++i) { rowv[RL::OFF_S + i] = state[i]; rowv[RL::OFF_S2 + i] = ns[i]; }
+        rowv[RL::OFF_A] = __int_as_float(action); rowv[RL::OFF_R] = r; rowv[RL::OFF_D] = d;
+        float4* dst = reinterpret_cast<float4*>(w.ring + (int64_t)row * RL::ROWF);
+#pragma unroll
+        for (int q = 0; q < RL::ROW_VEC; ++q)
+            if (threadIdx.x == q) __stcg(dst + q, make_float4(rowv[4 * q], rowv[4 * q + 1], rowv[4 * q + 2], rowv[4 * q + 3]));
+    }
+
+    __device__ __forceinline__ float learn(int64_t learn_iters, int rb_size) {
+        __syncthreads();
+        const int B = ls.batch;
+        for (int b = threadIdx.x; b < B; b += kGThreads) {   // replay_buffer.sample on the P_SAMPLE stream
+            const u32x4 wv = philox4x32_10((uint32_t)learn_iters, (uint32_t)(b >> 2), LE_P_SAMPLE, 0u, k0, k1);
+            const uint32_t idx = __umulhi(pick(wv, b & 3), (uint32_t)rb_size);
+            const float4* src = reinterpret_cast<const float4*>(w.ring + (int64_t)idx * RL::ROWF);
+            float rowv[RL::ROWF];
+#pragma unroll
+            for (int q = 0; q < RL::ROW_VEC; ++q) { const float4 v4 = __ldcg(src + q); rowv[4 * q] = v4.x; rowv[4 * q + 1] = v4.y; rowv[4 * q + 2] = v4.z; rowv[4 * q + 3] = v4.w; }
+#pragma unroll
+            for (int i = 0; i < SD; ++i) { w.xs[b * SD + i] = rowv[RL::OFF_S + i]; w.xs2[b * SD + i] = rowv[RL::OFF_S2 + i]; }
+            w.misc[4 * b] = (float)__float_as_int(rowv[RL::OFF_A]); w.misc[4 * b + 1] = rowv[RL::OFF_R]; w.misc[4 * b + 2] = rowv[RL::OFF_D];
+        }
+        __syncthreads();
+        return g_td_update(n, w, B, ls, sm, red, tcx);
+    }
+
+    __device__ __forceinline__ float* test_obs() { return w.obs; }
+
+    // greedy action of test row threadIdx.x
+    __device__ __forceinline__ int test_action(int M, int, int, int, bool running) {
+        g_net_forward(n, w.theta, w.obs, SD, M, w.actB, sm);
+        g_q_values(n, w.actB, M, w.q2, red);
+        int best = 0;
+        if (running)
+            for (int k = 1; k < AD; ++k)
+                if (w.q2[threadIdx.x * AD + k] > w.q2[threadIdx.x * AD + best]) best = k;
+        return best;
+    }
+
+    __device__ __forceinline__ void end_lane(int lane_id) {
+        if (P.q_final) for (int p = threadIdx.x; p < n.P; p += kGThreads) P.q_final[(int64_t)lane_id * P.q_stride + p] = w.theta[p];
+    }
+};
+
+// TC = false: two CTAs per SM, every dense layer on the FFMA GEMM.  TC = true: the CTA owns 128 TMEM columns and the dense
+// hidden x hidden layers run on tcgen05 (one CTA per SM: the runtime's TMEM occupancy rule).
+template <int SD, int AD, bool TC>
+__global__ void __launch_bounds__(kGThreads, TC ? 1 : 2) general_loop_kernel(const GRunParams G) {
+    __shared__ __align__(16) float sm[kGSmemFloats];
+    __shared__ float red[32];
+    __shared__ le_lane_cfg cfg_sm;
+    __shared__ GNet net_sm;
+    extern __shared__ __align__(128) unsigned char tc_smem[];   // TC: tc::kSmemBytes, operand parts of the tensor-core GEMM
+    tc::Ctx tcs;
+    if constexpr (TC) tcs = tc::ctx_create(tc_smem);
+    typename std::conditional<TC, tc::Ctx*, std::nullptr_t>::type tcx = nullptr;
+    if constexpr (TC) tcx = &tcs;
+    GeneralAgent<SD, AD, decltype(tcx)> ag{G.rp, gslot_view(G.slots + (int64_t)blockIdx.x * G.slot_stride, G.net, G.rp.ring_cap, RowLayout<SD>::ROWF, G.bmax),
+                                           cfg_sm, net_sm, sm, red, tcx};
+    cta_lane_loop<SD, AD>(G.rp, ag);
     if constexpr (TC) tc::ctx_destroy(tcs);
 }
 
@@ -935,15 +773,9 @@ general_td_update_kernel(const le_lane_cfg* __restrict__ cfg_dev, GNet n, float*
     if constexpr (TC) tcx = &tcs;
     const int id = blockIdx.x, tid = threadIdx.x;
     const le_lane_cfg c = *cfg_dev;
-    int64_t offs[18];
-    gslot_floats(n, 0, 0, B, offs);
-    float* base = scratch + (int64_t)id * scratch_stride;
-    GSlot w;
-    w.ring = nullptr; w.theta = th + (int64_t)id * q_stride; w.thetaT = thT + (int64_t)id * q_stride;
+    GSlot w = gslot_view(scratch + (int64_t)id * scratch_stride, n, 0, 0, B);   // scratch arrays; parameters and Adam state are the caller's
+    w.theta = th + (int64_t)id * q_stride; w.thetaT = thT + (int64_t)id * q_stride;
     w.m = m + (int64_t)id * q_stride; w.v = v + (int64_t)id * q_stride;
-    w.grad = base + offs[5]; w.xs = base + offs[6]; w.xs2 = base + offs[7]; w.misc = base + offs[8]; w.actA = base + offs[9];
-    w.actB = base + offs[10]; w.dact = base + offs[11]; w.q = base + offs[12]; w.q2 = base + offs[13]; w.qT = base + offs[14];
-    w.dq = base + offs[15]; w.obs = base + offs[16]; w.astar = reinterpret_cast<int*>(base + offs[17]);
     constexpr int ROWP = 2 * SD + 3;
     const float* my_rows = rows + (int64_t)id * B * ROWP;
     for (int b = tid; b < B; b += kGThreads) {

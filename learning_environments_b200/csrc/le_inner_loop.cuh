@@ -72,6 +72,26 @@ __device__ __forceinline__ double mean_window(const double* vals, int len, int n
     return s / ((double)(hi - lo) + 1e-9);
 }
 
+// env_solved (agents/base_agent.py:49-62), checked after each episode past init_episodes: the mean of the last
+// early_out_num episode values reaches solved_reward; on a virtual (SE) env without a test env, the mean stops moving instead
+__device__ __forceinline__ bool env_solved(const double* rewards, int n_ep, int episode, const le_lane_cfg& c) {
+    if (episode < c.init_episodes) return false;
+    const double avg = mean_window(rewards, n_ep, c.early_out_num, 0);
+    if ((!c.use_test_env) && c.env_kind == LE_ENV_SE) {
+        const double avg_last = mean_window(rewards, n_ep, c.early_out_num, c.early_out_num);
+        return (fabs(avg - avg_last) / (fabs(avg_last) + 1e-9) < c.early_out_virtual_diff) &&
+               (episode >= c.init_episodes + c.early_out_num);
+    }
+    return avg >= c.solved_reward;
+}
+
+// eps-greedy schedule of the DDQN agents (agents/DDQN.py:112-117): eps_init in episode 0, then decayed and floored at eps_min
+__device__ __forceinline__ double eps_schedule(double eps, int episode, const le_lane_cfg& c) {
+    if (episode == 0) return c.eps_init;
+    eps *= c.eps_decay;
+    return eps < c.eps_min ? c.eps_min : eps;
+}
+
 // One replay row (registers, HBM layout) -> shared-memory stage (same layout)
 template <int SD>
 __device__ __forceinline__ void stage_row(float* dst, const float (&rowv)[RowLayout<SD>::ROWF]) {

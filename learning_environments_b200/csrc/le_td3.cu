@@ -1,8 +1,8 @@
 // le_td3.cu — TD3_discrete_vary lanes (agents/TD3_discrete_vary.py, models/actor_critic.py:22-36,69-76) on the CTA-per-lane
 // machinery of le_general.cuh: one 256-thread CTA owns one agent — actor, two critics, three target nets, Adam state, the
 // replay ring and the minibatch activations live in the lane slot's HBM workspace; every dense layer goes through the
-// strided GEMM / thin paths of le_general.cuh.  Control flow mirrors general_loop_kernel (BaseAgent.train / test,
-// agents/base_agent.py:64-227) with the TD3 pieces:
+// strided GEMM / thin paths of le_general.cuh.  td3_loop_kernel runs the agent loop shared with general_loop_kernel
+// (cta_lane_loop, le_cta_lane.cuh: BaseAgent.train / test, agents/base_agent.py:64-227); this file holds the TD3 hooks:
 //   select_train_action / select_test_action (:155-166): actor -> * max_action -> F.gumbel_softmax(tau, hard) + N(0,1)*action_std,
 //       the environment receives argmax (agents/base_agent.py:111-114), the replay ring the action VECTOR;
 //   learn (:62-119): target policy smoothing, twin target critics (min), two Adam optimizers, delayed policy update through
@@ -71,30 +71,6 @@ static __device__ void t_net_backward(const GNet& n, const float* th, float* gra
     }
 }
 
-// torch.optim.Adam step of one parameter vector (same op order as g_td_update); t = step count AFTER the increment
-static __device__ void t_adam(float* th, float* m, float* v, const float* grad, int P, const LearnScalars& ls, double b1pow, double b2pow) {
-    const double bc1 = 1.0 - b1pow, bc2 = 1.0 - b2pow;
-    const float neg_step = (float)(-(ls.lr / bc1)), bc2s = (float)sqrt(bc2);
-    for (int p = threadIdx.x; p < P; p += kGThreads) {
-        const float g = __ldcg(grad + p);
-        float mm = __ldcg(m + p), vv = __ldcg(v + p);
-        mm = mm + ls.w1 * (g - mm);
-        vv = vv * ls.beta2;
-        vv = vv + (ls.w2 * g) * g;
-        __stcg(m + p, mm);
-        __stcg(v + p, vv);
-        bool exact = true;
-        float up = adam_update_core(mm, vv, neg_step, bc2s, ls.eps, &exact);
-        if (!exact) up = __fdiv_rn(neg_step * mm, __fdiv_rn(__fsqrt_rn(vv), bc2s) + ls.eps);
-        __stcg(th + p, __ldcg(th + p) + up);
-    }
-    __syncthreads();
-}
-static __device__ void t_polyak(const float* th, float* thT, int P, const LearnScalars& ls) {
-    for (int p = threadIdx.x; p < P; p += kGThreads) __stcg(thT + p, ls.tau * __ldcg(th + p) + ls.one_minus_tau * __ldcg(thT + p));
-    __syncthreads();
-}
-
 struct TSlot {
     float *ring, *actor, *actorT, *m_a, *v_a, *g_a, *c1, *c1T, *m_c1, *v_c1, *c2, *c2T, *m_c2, *v_c2, *g_c, *X, *X2, *Xpi, *S2, *misc, *Y, *DX,
         *Aa, *A1, *D, *obs;
@@ -128,378 +104,259 @@ __host__ __device__ inline int64_t tslot_floats(const GNet& na, const GNet& nc, 
     return o;
 }
 
-template <int SD, int AD>
-__global__ void __launch_bounds__(kGThreads, 2) td3_loop_kernel(const TRunParams G) {
-    static_assert(AD <= 4, "action vectors are handled as register arrays");
-    __shared__ __align__(16) float sm[kGSmemFloats];
-    __shared__ float red[32];
-    __shared__ __align__(16) float box[16];
-    __shared__ int ibox[4];
-    __shared__ double dred[kGThreads / 32];
-    __shared__ int sred[kGThreads / 32];
-    const RunParams& P = G.rp;
-    const le_lane_cfg& c = G.tc.base;
-    const GNet& na = G.na;
-    const GNet& nc = G.nc;
-    constexpr int XI = SD + AD;
-    const int ROWF = G.rowf;     // ring row: [s(SD) | a(AD) | s'(SD) | r | d | pad]
-    const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-    const int Sa = na.sum_out, Sc = nc.sum_out, yo_a = na.feat[na.nfeat - 1].y_off, yo_c = nc.feat[nc.nfeat - 1].y_off;
-    const float max_action = (float)G.tc.max_action, action_std = (float)G.tc.action_std;
-    const float policy_std = (float)G.tc.policy_std, policy_clip = (float)G.tc.policy_std_clip;
-    const int hard = G.tc.gumbel_hard;
+__device__ inline TSlot tslot_view(float* base, const GNet& na, const GNet& nc, int sd, int ad, int ring_cap, int rowf, int bmax) {
+    int64_t offs[26];
+    tslot_floats(na, nc, sd, ad, ring_cap, rowf, bmax, offs);
     TSlot w;
-    {
-        int64_t offs[26];
-        tslot_floats(na, nc, SD, AD, P.ring_cap, ROWF, G.bmax, offs);
-        float* base = G.slots + (int64_t)blockIdx.x * G.slot_stride;
-        w.ring = base + offs[0]; w.actor = base + offs[1]; w.actorT = base + offs[2]; w.m_a = base + offs[3]; w.v_a = base + offs[4];
-        w.g_a = base + offs[5]; w.c1 = base + offs[6]; w.c1T = base + offs[7]; w.m_c1 = base + offs[8]; w.v_c1 = base + offs[9];
-        w.c2 = base + offs[10]; w.c2T = base + offs[11]; w.m_c2 = base + offs[12]; w.v_c2 = base + offs[13]; w.g_c = base + offs[14];
-        w.X = base + offs[15]; w.X2 = base + offs[16]; w.Xpi = base + offs[17]; w.S2 = base + offs[18]; w.misc = base + offs[19];
-        w.Y = base + offs[20]; w.DX = base + offs[21]; w.Aa = base + offs[22]; w.A1 = base + offs[23]; w.D = base + offs[24];
-        w.obs = base + offs[25];
-    }
-    for (;;) {
-        __syncthreads();
-        if (tid == 0) ibox[0] = atomicAdd(P.work_counter, 1);
-        __syncthreads();
-        const int lane_id = ibox[0];
-        if (lane_id >= P.n_lanes) break;
-        const uint32_t k0 = P.keys[2 * lane_id], k1 = P.keys[2 * lane_id + 1];
-        const float4* pack = P.env_pack + (int64_t)(P.env_index ? P.env_index[lane_id] : 0) * P.env_pack_stride;
-        const bool env_tanh = c.env_act == LE_ACT_TANH;
-        double* rewards = P.rewards + (int64_t)lane_id * P.rew_stride;
-        int32_t* lengths = P.lengths + (int64_t)lane_id * P.rew_stride;
-        double* test_rewards = P.test_rewards + (int64_t)lane_id * P.test_stride;
-        const bool tracing = P.trace.cap > 0 && lane_id == P.trace_lane;
-        // ---- agent construction: targets = copies, Adam state zero (agents/TD3_discrete_vary.py:41-52)
-        for (int p = tid; p < na.P; p += kGThreads) {
+    w.ring = base + offs[0]; w.actor = base + offs[1]; w.actorT = base + offs[2]; w.m_a = base + offs[3]; w.v_a = base + offs[4];
+    w.g_a = base + offs[5]; w.c1 = base + offs[6]; w.c1T = base + offs[7]; w.m_c1 = base + offs[8]; w.v_c1 = base + offs[9];
+    w.c2 = base + offs[10]; w.c2T = base + offs[11]; w.m_c2 = base + offs[12]; w.v_c2 = base + offs[13]; w.g_c = base + offs[14];
+    w.X = base + offs[15]; w.X2 = base + offs[16]; w.Xpi = base + offs[17]; w.S2 = base + offs[18]; w.misc = base + offs[19];
+    w.Y = base + offs[20]; w.DX = base + offs[21]; w.Aa = base + offs[22]; w.A1 = base + offs[23]; w.D = base + offs[24];
+    w.obs = base + offs[25];
+    return w;
+}
+
+// TD3_discrete_vary agent as the hooks of cta_lane_loop
+template <int SD, int AD>
+struct Td3Agent {
+    static constexpr int XI = SD + AD;
+    const TRunParams& G;
+    const TSlot w;
+    float* sm;
+    float* red;
+    uint32_t k0, k1;
+    LearnScalars ls;
+    double b1pow_a, b2pow_a, b1pow_c, b2pow_c;
+    float temp;        // self.gumbel_temp_annealed
+    int total_it;
+    float avec[AD];    // action vector of the current train step (its replay row)
+
+    __device__ __forceinline__ const le_lane_cfg& begin_lane(int lane_id, uint32_t key0, uint32_t key1) {
+        const int tid = threadIdx.x;
+        k0 = key0; k1 = key1;
+        // targets = copies, Adam state zero (agents/TD3_discrete_vary.py:41-52)
+        for (int p = tid; p < G.na.P; p += kGThreads) {
             const float v0 = G.actor_init[(int64_t)lane_id * G.init_stride_a + p];
             w.actor[p] = v0; w.actorT[p] = v0; w.m_a[p] = 0.f; w.v_a[p] = 0.f;
         }
-        for (int p = tid; p < nc.P; p += kGThreads) {
+        for (int p = tid; p < G.nc.P; p += kGThreads) {
             const float a1 = G.c1_init[(int64_t)lane_id * G.init_stride_c + p], a2 = G.c2_init[(int64_t)lane_id * G.init_stride_c + p];
             w.c1[p] = a1; w.c1T[p] = a1; w.m_c1[p] = 0.f; w.v_c1[p] = 0.f;
             w.c2[p] = a2; w.c2T[p] = a2; w.m_c2[p] = 0.f; w.v_c2[p] = 0.f;
         }
         __syncthreads();
-        LearnScalars ls;
-        fill_learn_scalars(ls, c);
-        double b1pow_a = 1.0, b2pow_a = 1.0, b1pow_c = 1.0, b2pow_c = 1.0;
-        const double T0 = G.tc.gumbel_temp, Tstep = (T0 / 20.0 - T0) / 1999.0;      // np.linspace(T0, T0/20, 2000)
-        float temp = (float)T0;                                                     // self.gumbel_temp_annealed
-        int total_it = 0;
-        const int K = c.same_action_num > 1 ? c.same_action_num : 1;
+        fill_learn_scalars(ls, G.tc.base);
+        b1pow_a = 1.0; b2pow_a = 1.0; b1pow_c = 1.0; b2pow_c = 1.0;
+        temp = (float)G.tc.gumbel_temp;
+        total_it = 0;
+        return G.tc.base;
+    }
 
-        // actor(rows) + Gumbel-softmax + action noise for M rows held in `Xrows` (row stride xs): thread m < M handles row m.
-        // Returns this thread's argmax; avec <- the action vector.
-        auto act_rows = [&](const float* Xrows, int xs, int M, uint32_t phase, uint32_t c0, uint32_t sub_of_thread, bool active,
-                            float (&avec)[AD]) -> int {
-            g_net_forward(na, w.actor, Xrows, xs, M, w.Aa, sm);
-            int best = 0;
-            if (active) {
+    __device__ __forceinline__ void begin_episode(int) {}
+
+    // actor(rows) + Gumbel-softmax + action noise for M rows held in `Xrows` (row stride xs): thread m < M handles row m.
+    // Returns this thread's argmax; av <- the action vector.
+    __device__ __forceinline__ int act_rows(const float* Xrows, int xs, int M, uint32_t phase, uint32_t c0, uint32_t sub_of_thread, bool active,
+                                            float (&av)[AD]) {
+        const int Sa = G.na.sum_out, yo_a = G.na.feat[G.na.nfeat - 1].y_off;
+        g_net_forward(G.na, w.actor, Xrows, xs, M, w.Aa, sm);
+        int best = 0;
+        if (active) {
+            float logits[AD], expo[AD], y[AD], ret[AD];
+#pragma unroll
+            for (int k = 0; k < AD; ++k) {
+                logits[k] = __ldcg(w.Aa + (int64_t)threadIdx.x * Sa + yo_a + k) * (float)G.tc.max_action;
+                expo[k] = td3_expo(k0, k1, phase, c0, sub_of_thread, k);
+            }
+            gumbel_softmax_row<AD>(logits, expo, temp, G.tc.gumbel_hard, y, ret);
+#pragma unroll
+            for (int k = 0; k < AD; ++k) {
+                av[k] = ret[k] + td3_normal(k0, k1, phase, c0, sub_of_thread, k) * (float)G.tc.action_std;
+                if (av[k] > av[best]) best = k;
+            }
+        }
+        return best;
+    }
+
+    // select_train_action (:155-162): random before init_episodes, then the actor on row 0; `box` broadcasts the action vector
+    __device__ __forceinline__ int train_action(const float (&state)[SD], int episode, int64_t train_steps, bool, bool& explore, float&,
+                                                float* box) {
+        explore = episode < G.tc.base.init_episodes;
+        if (explore) {
+            const u32x4 wa = philox4x32_10((uint32_t)train_steps, 0u, LE_P_ACT, 0u, k0, k1);
+            const int action = (int)__umulhi(wa.y, (uint32_t)AD);
+#pragma unroll
+            for (int k = 0; k < AD; ++k) avec[k] = k == action ? 1.f : 0.f;
+            return action;
+        }
+        const int tid = threadIdx.x;
+        __syncthreads();
+        if (tid < SD) __stcg(w.X + tid, state[tid]);      // row 0 of the staging area (free between learn() calls)
+        __syncthreads();
+        float av0[AD];
+        act_rows(w.X, XI, 1, 0u, (uint32_t)train_steps, 0u, tid == 0, av0);
+        if (tid == 0) {
+#pragma unroll
+            for (int k = 0; k < AD; ++k) box[k] = av0[k];
+        }
+        __syncthreads();
+        int action = 0;
+#pragma unroll
+        for (int k = 0; k < AD; ++k) { avec[k] = box[k]; if (avec[k] > avec[action]) action = k; }
+        __syncthreads();
+        return action;
+    }
+
+    // ring row: [s(SD) | a(AD) | s'(SD) | r | d | pad], with the action VECTOR
+    __device__ __forceinline__ void store_row(int rb_ptr, const float (&state)[SD], int, const float (&ns)[SD], float r, float d) {
+        if (threadIdx.x == 0) {
+            float* row = w.ring + (int64_t)rb_ptr * G.rowf;
+#pragma unroll
+            for (int i = 0; i < SD; ++i) { __stcg(row + i, state[i]); __stcg(row + SD + AD + i, ns[i]); }
+#pragma unroll
+            for (int k = 0; k < AD; ++k) __stcg(row + SD + k, avec[k]);
+            __stcg(row + 2 * SD + AD, r);
+            __stcg(row + 2 * SD + AD + 1, d);
+        }
+    }
+
+    // learn (:62-119)
+    __device__ __forceinline__ float learn(int64_t learn_iters, int rb_size) {
+        const GNet& na = G.na;
+        const GNet& nc = G.nc;
+        const int tid = threadIdx.x;
+        const int Sa = na.sum_out, Sc = nc.sum_out, yo_a = na.feat[na.nfeat - 1].y_off, yo_c = nc.feat[nc.nfeat - 1].y_off;
+        const float max_action = (float)G.tc.max_action, policy_std = (float)G.tc.policy_std, policy_clip = (float)G.tc.policy_std_clip;
+        const int hard = G.tc.gumbel_hard;
+        const double T0 = G.tc.gumbel_temp, Tstep = (T0 / 20.0 - T0) / 1999.0;      // np.linspace(T0, T0/20, 2000)
+        __syncthreads();
+        temp = (float)(total_it >= 1999 ? T0 / 20.0 : (double)total_it * Tstep + T0);
+        total_it += 1;
+        const int B = ls.batch;
+        for (int b = tid; b < B; b += kGThreads) {     // replay_buffer.sample on the P_SAMPLE stream
+            const u32x4 wv = philox4x32_10((uint32_t)learn_iters, (uint32_t)(b >> 2), LE_P_SAMPLE, 0u, k0, k1);
+            const float* src = w.ring + (int64_t)__umulhi(pick(wv, b & 3), (uint32_t)rb_size) * G.rowf;
+#pragma unroll
+            for (int i = 0; i < XI; ++i) w.X[b * XI + i] = __ldcg(src + i);
+#pragma unroll
+            for (int i = 0; i < SD; ++i) w.S2[b * SD + i] = __ldcg(src + XI + i);
+            w.misc[4 * b] = __ldcg(src + 2 * SD + AD);
+            w.misc[4 * b + 1] = __ldcg(src + 2 * SD + AD + 1);
+        }
+        __syncthreads();
+        // target policy smoothing: a' = gumbel_softmax(actor_target(s')) + clip(N * policy_std)
+        g_net_forward(na, w.actorT, w.S2, SD, B, w.Aa, sm);
+        for (int b = tid; b < B; b += kGThreads) {
+            float logits[AD], expo[AD], y[AD], ret[AD];
+#pragma unroll
+            for (int k = 0; k < AD; ++k) {
+                logits[k] = __ldcg(w.Aa + (int64_t)b * Sa + yo_a + k) * max_action;
+                expo[k] = td3_expo(k0, k1, 2u, (uint32_t)learn_iters, 0u, b * AD + k);
+            }
+            gumbel_softmax_row<AD>(logits, expo, temp, hard, y, ret);
+#pragma unroll
+            for (int i = 0; i < SD; ++i) w.X2[b * XI + i] = w.S2[b * SD + i];
+#pragma unroll
+            for (int k = 0; k < AD; ++k) {
+                float nz = td3_normal(k0, k1, 2u, (uint32_t)learn_iters, 0u, b * AD + k) * policy_std;
+                nz = nz < -policy_clip ? -policy_clip : (nz > policy_clip ? policy_clip : nz);
+                w.X2[b * XI + SD + k] = ret[k] + nz;
+            }
+        }
+        __syncthreads();
+        // target_Q = r + (1 - d) * gamma * min(Q1', Q2')
+        g_net_forward(nc, w.c1T, w.X2, XI, B, w.A1, sm);
+        for (int b = tid; b < B; b += kGThreads) w.misc[4 * b + 2] = __ldcg(w.A1 + (int64_t)b * Sc + yo_c);
+        __syncthreads();
+        g_net_forward(nc, w.c2T, w.X2, XI, B, w.A1, sm);
+        for (int b = tid; b < B; b += kGThreads) {
+            const float q1 = w.misc[4 * b + 2], q2 = __ldcg(w.A1 + (int64_t)b * Sc + yo_c);
+            w.misc[4 * b + 2] = w.misc[4 * b] + ((1.f - w.misc[4 * b + 1]) * ls.gamma) * fminf(q1, q2);
+        }
+        __syncthreads();
+        // critic loss and the two critic steps (one optimizer: shared step count)
+        b1pow_c *= ls.beta1; b2pow_c *= ls.beta2d;
+        float lsum = 0.f;
+        for (int which = 0; which < 2; ++which) {
+            float* cth = which ? w.c2 : w.c1;
+            g_net_forward(nc, cth, w.X, XI, B, w.A1, sm);
+            float lpart = 0.f;
+            for (int b = tid; b < B; b += kGThreads) {
+                const float e = __ldcg(w.A1 + (int64_t)b * Sc + yo_c) - w.misc[4 * b + 2];
+                lpart = fmaf(e, e, lpart);
+                __stcg(w.D + (int64_t)b * Sc + yo_c, ls.norm * e);
+            }
+            lsum += g_block_sum(lpart, red) / (float)B;
+            __syncthreads();
+            t_net_backward(nc, cth, w.g_c, w.X, XI, w.A1, w.D, B, nullptr, 0, sm);
+            g_adam(cth, nullptr, which ? w.m_c2 : w.m_c1, which ? w.v_c2 : w.v_c1, w.g_c, nc.P, ls, b1pow_c, b2pow_c);
+        }
+        if (total_it % G.tc.policy_delay == 0) {
+            // actor loss = -mean(critic_1(s, actor(s))) through the (updated) critic and the straight-through Gumbel-softmax
+            g_net_forward(na, w.actor, w.X, XI, B, w.Aa, sm);
+            for (int b = tid; b < B; b += kGThreads) {
                 float logits[AD], expo[AD], y[AD], ret[AD];
 #pragma unroll
                 for (int k = 0; k < AD; ++k) {
-                    logits[k] = __ldcg(w.Aa + (int64_t)tid * Sa + yo_a + k) * max_action;
-                    expo[k] = td3_expo(k0, k1, phase, c0, sub_of_thread, k);
+                    logits[k] = __ldcg(w.Aa + (int64_t)b * Sa + yo_a + k) * max_action;
+                    expo[k] = td3_expo(k0, k1, 3u, (uint32_t)learn_iters, 0u, b * AD + k);
                 }
                 gumbel_softmax_row<AD>(logits, expo, temp, hard, y, ret);
 #pragma unroll
-                for (int k = 0; k < AD; ++k) {
-                    avec[k] = ret[k] + td3_normal(k0, k1, phase, c0, sub_of_thread, k) * action_std;
-                    if (avec[k] > avec[best]) best = k;
-                }
+                for (int i = 0; i < SD; ++i) w.Xpi[b * XI + i] = w.X[b * XI + i];
+#pragma unroll
+                for (int k = 0; k < AD; ++k) { w.Xpi[b * XI + SD + k] = ret[k]; w.Y[4 * b + k] = y[k]; }
             }
-            return best;
-        };
-
-        // greedy-with-noise test rollouts on the real env, episodes = rows of one batched actor forward per step
-        auto run_test = [&](int test_call, double* ep_out, int64_t& test_steps) -> double {
-            double total = 0.0;
-            for (int ep0 = 0; ep0 < c.test_episodes; ep0 += 64) {
-                const int M = min(64, c.test_episodes - ep0);
-                double st[4] = {0, 0, 0, 0};
-                float obs[SD];
-                int elapsed = 0, ep_steps = 0;
-                float ep_rew = 0.f;
-                bool running = tid < M;
-                if (tid < M) {
-                    real_reset(c.real_env, philox4x32_10((uint32_t)test_call, (uint32_t)(ep0 + tid), LE_P_RESET_TEST, 0u, k0, k1), st);
-                    real_obs<SD>(c.real_env, st, obs);
-#pragma unroll
-                    for (int i = 0; i < SD; ++i) w.obs[tid * SD + i] = obs[i];
-                }
-                for (int t = 0; t < c.max_steps; t += K) {
-                    if (!__syncthreads_or(running ? 1 : 0)) break;
-                    float avec[AD];
-                    const int a = act_rows(w.obs, SD, M, 1u, ((uint32_t)test_call << 16) | (uint32_t)(t / K), (uint32_t)(ep0 + tid), running, avec);
-                    if (running) {
-                        float r, d;
-                        real_step<SD>(c.real_env, c.max_steps, st, elapsed, a, obs, r, d);
-                        if (K > 1) {
-                            double rsum = (double)r;
-                            for (int k = 1; k < K && !(d > 0.5f); ++k) { float rk; real_step<SD>(c.real_env, c.max_steps, st, elapsed, a, obs, rk, d); rsum += (double)rk; }
-                            r = (float)rsum;
-                        }
-#pragma unroll
-                        for (int i = 0; i < SD; ++i) w.obs[tid * SD + i] = obs[i];
-                        ep_rew += r;
-                        ep_steps += 1;
-                        if (d > 0.5f) running = false;
-                    }
-                }
-                __syncthreads();
-                if (tid < M && ep_out) ep_out[ep0 + tid] = (double)ep_rew;
-                double dv = warp_allreduce_sum((tid < M) ? (double)ep_rew : 0.0);
-                int sv = (tid < M) ? ep_steps : 0;
-#pragma unroll
-                for (int mm = 16; mm > 0; mm >>= 1) sv += __shfl_xor_sync(LE_FULL_MASK, sv, mm);
-                __syncthreads();
-                if (lane == 0) { dred[warp] = dv; sred[warp] = sv; }
-                __syncthreads();
-                for (int q = 0; q < kGThreads / 32; ++q) { total += dred[q]; test_steps += sred[q]; }
-                __syncthreads();
-            }
-            return total / (double)c.test_episodes;
-        };
-
-        int rb_ptr = 0, rb_size = 0;
-        int64_t train_steps = 0, learn_iters = 0, test_steps = 0;
-        int test_calls = 0, n_ep = 0, timed_out = 0;
-        const bool rule_virtual = (!c.use_test_env) && c.env_kind == LE_ENV_SE;
-        for (int episode = 0; episode < c.train_episodes; ++episode) {
-            if (c.step_budget > 0 && train_steps >= c.step_budget) { timed_out = 1; break; }
-            double st[4];
-            real_reset(c.real_env, philox4x32_10((uint32_t)episode, 0u, LE_P_RESET_TRAIN, 0u, k0, k1), st);
-            float state[SD];
-            real_obs<SD>(c.real_env, st, state);
-            int elapsed = 0, ep_len = 0;
-            float ep_rew = 0.f;
-            for (int t = 0; t < c.max_steps; t += K) {
-                // ---- select_train_action (:155-162)
-                float avec[AD];
-                int action;
-                if (episode < c.init_episodes) {
-                    const u32x4 wa = philox4x32_10((uint32_t)train_steps, 0u, LE_P_ACT, 0u, k0, k1);
-                    action = (int)__umulhi(wa.y, (uint32_t)AD);
-#pragma unroll
-                    for (int k = 0; k < AD; ++k) avec[k] = k == action ? 1.f : 0.f;
-                } else {
-                    __syncthreads();
-                    if (tid < SD) __stcg(w.X + tid, state[tid]);      // row 0 of the staging area (free between learn() calls)
-                    __syncthreads();
-                    float av0[AD];
-                    const int a0 = act_rows(w.X, XI, 1, 0u, (uint32_t)train_steps, 0u, tid == 0, av0);
-                    if (tid == 0) {
-                        ibox[1] = a0;
-#pragma unroll
-                        for (int k = 0; k < AD; ++k) box[8 + k] = av0[k];
-                    }
-                    __syncthreads();
-                    action = ibox[1];
-#pragma unroll
-                    for (int k = 0; k < AD; ++k) avec[k] = box[8 + k];
-                    __syncthreads();
-                }
-                // ---- env.step(action.argmax())
-                float ns[SD], r = 0.f, d = 0.f;
-                if (c.env_kind == LE_ENV_SE) {
-                    __syncthreads();
-                    if (warp == 0) {
-                        float cur[SD], ns0[SD], r0 = 0.f, d0 = 0.f;
-#pragma unroll
-                        for (int i = 0; i < SD; ++i) cur[i] = state[i];
-                        for (int k = 0; k < K; ++k) {
-                            float rk;
-                            se_step_row<SD, AD>(pack, c.env_hidden, env_tanh, cur, action, lane, ns0, rk, d0);
-                            r0 = k == 0 ? rk : r0 + rk;
-#pragma unroll
-                            for (int i = 0; i < SD; ++i) cur[i] = ns0[i];
-                        }
-                        if (lane == 0) {
-#pragma unroll
-                            for (int i = 0; i < SD; ++i) box[i] = ns0[i];
-                            box[SD] = r0; box[SD + 1] = d0;
-                        }
-                    }
-                    __syncthreads();
-#pragma unroll
-                    for (int i = 0; i < SD; ++i) ns[i] = box[i];
-                    r = box[SD]; d = box[SD + 1];
-                    __syncthreads();
-                } else {
-                    double rsum = 0.0;
-                    for (int k = 0; k < K; ++k) {
-                        float rr;
-                        real_step<SD>(c.real_env, c.max_steps, st, elapsed, action, ns, rr, d);
-                        rsum += (double)rr;
-                        r = K == 1 ? rr : (float)rsum;
-                        if (d > 0.5f) break;
-                    }
-                }
-                // ---- replay_buffer.add with the action vector
-                if (tid == 0) {
-                    float* row = w.ring + (int64_t)rb_ptr * ROWF;
-#pragma unroll
-                    for (int i = 0; i < SD; ++i) { __stcg(row + i, state[i]); __stcg(row + SD + AD + i, ns[i]); }
-#pragma unroll
-                    for (int k = 0; k < AD; ++k) __stcg(row + SD + k, avec[k]);
-                    __stcg(row + 2 * SD + AD, r);
-                    __stcg(row + 2 * SD + AD + 1, d);
-                }
-                rb_ptr = (rb_ptr + 1 == P.ring_cap) ? 0 : rb_ptr + 1;
-                rb_size = rb_size + 1 < P.ring_cap ? rb_size + 1 : P.ring_cap;
-#pragma unroll
-                for (int i = 0; i < SD; ++i) state[i] = ns[i];
-                ep_rew += r;
-                ep_len += K;
-                float loss = __int_as_float(0x7fc00000);
-                if (episode >= c.init_episodes) {
-                    // ---- learn (:62-119)
-                    __syncthreads();
-                    temp = (float)(total_it >= 1999 ? T0 / 20.0 : (double)total_it * Tstep + T0);
-                    total_it += 1;
-                    const int B = ls.batch;
-                    for (int b = tid; b < B; b += kGThreads) {     // replay_buffer.sample on the P_SAMPLE stream
-                        const u32x4 wv = philox4x32_10((uint32_t)learn_iters, (uint32_t)(b >> 2), LE_P_SAMPLE, 0u, k0, k1);
-                        const float* src = w.ring + (int64_t)__umulhi(pick(wv, b & 3), (uint32_t)rb_size) * ROWF;
-#pragma unroll
-                        for (int i = 0; i < XI; ++i) w.X[b * XI + i] = __ldcg(src + i);
-#pragma unroll
-                        for (int i = 0; i < SD; ++i) w.S2[b * SD + i] = __ldcg(src + XI + i);
-                        w.misc[4 * b] = __ldcg(src + 2 * SD + AD);
-                        w.misc[4 * b + 1] = __ldcg(src + 2 * SD + AD + 1);
-                    }
-                    __syncthreads();
-                    // target policy smoothing: a' = gumbel_softmax(actor_target(s')) + clip(N * policy_std)
-                    g_net_forward(na, w.actorT, w.S2, SD, B, w.Aa, sm);
-                    for (int b = tid; b < B; b += kGThreads) {
-                        float logits[AD], expo[AD], y[AD], ret[AD];
-#pragma unroll
-                        for (int k = 0; k < AD; ++k) {
-                            logits[k] = __ldcg(w.Aa + (int64_t)b * Sa + yo_a + k) * max_action;
-                            expo[k] = td3_expo(k0, k1, 2u, (uint32_t)learn_iters, 0u, b * AD + k);
-                        }
-                        gumbel_softmax_row<AD>(logits, expo, temp, hard, y, ret);
-#pragma unroll
-                        for (int i = 0; i < SD; ++i) w.X2[b * XI + i] = w.S2[b * SD + i];
-#pragma unroll
-                        for (int k = 0; k < AD; ++k) {
-                            float nz = td3_normal(k0, k1, 2u, (uint32_t)learn_iters, 0u, b * AD + k) * policy_std;
-                            nz = nz < -policy_clip ? -policy_clip : (nz > policy_clip ? policy_clip : nz);
-                            w.X2[b * XI + SD + k] = ret[k] + nz;
-                        }
-                    }
-                    __syncthreads();
-                    // target_Q = r + (1 - d) * gamma * min(Q1', Q2')
-                    g_net_forward(nc, w.c1T, w.X2, XI, B, w.A1, sm);
-                    for (int b = tid; b < B; b += kGThreads) w.misc[4 * b + 2] = __ldcg(w.A1 + (int64_t)b * Sc + yo_c);
-                    __syncthreads();
-                    g_net_forward(nc, w.c2T, w.X2, XI, B, w.A1, sm);
-                    for (int b = tid; b < B; b += kGThreads) {
-                        const float q1 = w.misc[4 * b + 2], q2 = __ldcg(w.A1 + (int64_t)b * Sc + yo_c);
-                        w.misc[4 * b + 2] = w.misc[4 * b] + ((1.f - w.misc[4 * b + 1]) * ls.gamma) * fminf(q1, q2);
-                    }
-                    __syncthreads();
-                    // critic loss and the two critic steps (one optimizer: shared step count)
-                    b1pow_c *= ls.beta1; b2pow_c *= ls.beta2d;
-                    float lsum = 0.f;
-                    for (int which = 0; which < 2; ++which) {
-                        float* cth = which ? w.c2 : w.c1;
-                        g_net_forward(nc, cth, w.X, XI, B, w.A1, sm);
-                        float lpart = 0.f;
-                        for (int b = tid; b < B; b += kGThreads) {
-                            const float e = __ldcg(w.A1 + (int64_t)b * Sc + yo_c) - w.misc[4 * b + 2];
-                            lpart = fmaf(e, e, lpart);
-                            __stcg(w.D + (int64_t)b * Sc + yo_c, ls.norm * e);
-                        }
-                        lsum += g_block_sum(lpart, red) / (float)B;
-                        __syncthreads();
-                        t_net_backward(nc, cth, w.g_c, w.X, XI, w.A1, w.D, B, nullptr, 0, sm);
-                        t_adam(cth, which ? w.m_c2 : w.m_c1, which ? w.v_c2 : w.v_c1, w.g_c, nc.P, ls, b1pow_c, b2pow_c);
-                    }
-                    loss = lsum;
-                    if (total_it % G.tc.policy_delay == 0) {
-                        // actor loss = -mean(critic_1(s, actor(s))) through the (updated) critic and the straight-through Gumbel-softmax
-                        g_net_forward(na, w.actor, w.X, XI, B, w.Aa, sm);
-                        for (int b = tid; b < B; b += kGThreads) {
-                            float logits[AD], expo[AD], y[AD], ret[AD];
-#pragma unroll
-                            for (int k = 0; k < AD; ++k) {
-                                logits[k] = __ldcg(w.Aa + (int64_t)b * Sa + yo_a + k) * max_action;
-                                expo[k] = td3_expo(k0, k1, 3u, (uint32_t)learn_iters, 0u, b * AD + k);
-                            }
-                            gumbel_softmax_row<AD>(logits, expo, temp, hard, y, ret);
-#pragma unroll
-                            for (int i = 0; i < SD; ++i) w.Xpi[b * XI + i] = w.X[b * XI + i];
-#pragma unroll
-                            for (int k = 0; k < AD; ++k) { w.Xpi[b * XI + SD + k] = ret[k]; w.Y[4 * b + k] = y[k]; }
-                        }
-                        __syncthreads();
-                        g_net_forward(nc, w.c1, w.Xpi, XI, B, w.A1, sm);
-                        for (int b = tid; b < B; b += kGThreads) __stcg(w.D + (int64_t)b * Sc + yo_c, -1.f / (float)B);
-                        __syncthreads();
-                        t_net_backward(nc, w.c1, w.g_c, w.Xpi, XI, w.A1, w.D, B, w.DX, XI, sm);     // only dL/d(action) is used
-                        for (int b = tid; b < B; b += kGThreads) {
-                            float dot = 0.f;
-#pragma unroll
-                            for (int k = 0; k < AD; ++k) dot += w.Y[4 * b + k] * __ldcg(w.DX + (int64_t)b * XI + SD + k);
-#pragma unroll
-                            for (int k = 0; k < AD; ++k)
-                                __stcg(w.D + (int64_t)b * Sa + yo_a + k,
-                                       __fdiv_rn(w.Y[4 * b + k] * (__ldcg(w.DX + (int64_t)b * XI + SD + k) - dot), temp) * max_action);
-                        }
-                        __syncthreads();
-                        t_net_backward(na, w.actor, w.g_a, w.X, XI, w.Aa, w.D, B, nullptr, 0, sm);
-                        b1pow_a *= ls.beta1; b2pow_a *= ls.beta2d;
-                        t_adam(w.actor, w.m_a, w.v_a, w.g_a, na.P, ls, b1pow_a, b2pow_a);
-                        t_polyak(w.c1, w.c1T, nc.P, ls);
-                        t_polyak(w.c2, w.c2T, nc.P, ls);
-                        t_polyak(w.actor, w.actorT, na.P, ls);
-                    }
-                    learn_iters += 1;
-                }
-                if (tracing && train_steps < P.trace.cap && tid == 0) {
-                    const int64_t i = train_steps;
-                    P.trace.action[i] = action; P.trace.explore[i] = episode < c.init_episodes ? 1 : 0;
-                    P.trace.reward[i] = r; P.trace.done[i] = d; P.trace.loss[i] = loss;
-#pragma unroll
-                    for (int k = 0; k < SD; ++k) P.trace.next_state[i * SD + k] = ns[k];
-                }
-                train_steps += 1;
-                if (d > 0.5f) break;
-            }
-            double ep_value;
-            if (c.use_test_env) ep_value = run_test(test_calls++, nullptr, test_steps);
-            else ep_value = (double)ep_rew;
             __syncthreads();
-            if (tid == 0) { lengths[n_ep] = ep_len; rewards[n_ep] = ep_value; __threadfence_block(); }
-            n_ep += 1;
+            g_net_forward(nc, w.c1, w.Xpi, XI, B, w.A1, sm);
+            for (int b = tid; b < B; b += kGThreads) __stcg(w.D + (int64_t)b * Sc + yo_c, -1.f / (float)B);
             __syncthreads();
-            if (episode >= c.init_episodes) {
-                const double avg = mean_window(rewards, n_ep, c.early_out_num, 0);
-                bool solved;
-                if (rule_virtual) {
-                    const double avg_last = mean_window(rewards, n_ep, c.early_out_num, c.early_out_num);
-                    solved = (fabs(avg - avg_last) / (fabs(avg_last) + 1e-9) < c.early_out_virtual_diff) &&
-                             (episode >= c.init_episodes + c.early_out_num);
-                } else solved = avg >= c.solved_reward;
-                if (solved) break;
+            t_net_backward(nc, w.c1, w.g_c, w.Xpi, XI, w.A1, w.D, B, w.DX, XI, sm);     // only dL/d(action) is used
+            for (int b = tid; b < B; b += kGThreads) {
+                float dot = 0.f;
+#pragma unroll
+                for (int k = 0; k < AD; ++k) dot += w.Y[4 * b + k] * __ldcg(w.DX + (int64_t)b * XI + SD + k);
+#pragma unroll
+                for (int k = 0; k < AD; ++k)
+                    __stcg(w.D + (int64_t)b * Sa + yo_a + k,
+                           __fdiv_rn(w.Y[4 * b + k] * (__ldcg(w.DX + (int64_t)b * XI + SD + k) - dot), temp) * max_action);
             }
+            __syncthreads();
+            t_net_backward(na, w.actor, w.g_a, w.X, XI, w.Aa, w.D, B, nullptr, 0, sm);
+            b1pow_a *= ls.beta1; b2pow_a *= ls.beta2d;
+            g_adam(w.actor, nullptr, w.m_a, w.v_a, w.g_a, na.P, ls, b1pow_a, b2pow_a);
+            // Polyak on the three targets, after all three updates
+            for (int p = tid; p < nc.P; p += kGThreads) {
+                __stcg(w.c1T + p, ls.tau * __ldcg(w.c1 + p) + ls.one_minus_tau * __ldcg(w.c1T + p));
+                __stcg(w.c2T + p, ls.tau * __ldcg(w.c2 + p) + ls.one_minus_tau * __ldcg(w.c2T + p));
+            }
+            for (int p = tid; p < na.P; p += kGThreads) __stcg(w.actorT + p, ls.tau * __ldcg(w.actor + p) + ls.one_minus_tau * __ldcg(w.actorT + p));
+            __syncthreads();
         }
-        double score = 0.0;
-        if (c.final_test) score = run_test(test_calls++, test_rewards, test_steps);
-        __syncthreads();
-        if (G.actor_final) for (int p = tid; p < na.P; p += kGThreads) G.actor_final[(int64_t)lane_id * na.P + p] = w.actor[p];
-        if (tid == 0) {
-            le_lane_out o;
-            o.n_episodes = n_ep; o.timed_out = timed_out; o.train_steps = train_steps; o.learn_iters = learn_iters;
-            o.test_steps = test_steps; o.score = score;
-            P.out[lane_id] = o;
-        }
+        return lsum;
     }
+
+    __device__ __forceinline__ float* test_obs() { return w.obs; }
+
+    // select_test_action (:163-166) of test row threadIdx.x: actor + Gumbel-softmax + noise on the P_TD3 phase-1 draws
+    __device__ __forceinline__ int test_action(int M, int test_call, int step, int ep0, bool running) {
+        float av[AD];
+        return act_rows(w.obs, SD, M, 1u, ((uint32_t)test_call << 16) | (uint32_t)step, (uint32_t)(ep0 + threadIdx.x), running, av);
+    }
+
+    __device__ __forceinline__ void end_lane(int lane_id) {
+        if (G.actor_final) for (int p = threadIdx.x; p < G.na.P; p += kGThreads) G.actor_final[(int64_t)lane_id * G.na.P + p] = w.actor[p];
+    }
+};
+
+template <int SD, int AD>
+__global__ void __launch_bounds__(kGThreads, 2) td3_loop_kernel(const TRunParams G) {
+    static_assert(AD <= 4, "action vectors are handled as register arrays");
+    __shared__ __align__(16) float sm[kGSmemFloats];
+    __shared__ float red[32];
+    Td3Agent<SD, AD> ag{G, tslot_view(G.slots + (int64_t)blockIdx.x * G.slot_stride, G.na, G.nc, SD, AD, G.rp.ring_cap, G.rowf, G.bmax), sm, red};
+    cta_lane_loop<SD, AD>(G.rp, ag);
 }
 
 // ---- host side ---------------------------------------------------------------------------------------------------

@@ -245,6 +245,37 @@ typedef struct le_td3_cfg {
  * [n_init][P_critic] with n_init = 1 (shared by all lanes) or n_lanes; parameter vectors in torch state_dict order.
  * Training env: LE_ENV_SE or LE_ENV_REAL.  trace_host (may be NULL): HOST arrays recording lane `trace_lane`.           */
 int le_td3_param_counts(const le_td3_cfg* cfg, int* p_actor, int* p_critic);
+
+/* Bytes of device workspace for le_td3_run: the packed SE weights, the lane queue counter and one slot (replay ring, the six
+ * nets, Adam state, minibatch activations) per RESIDENT lane, every slot sized for cfg_host0 (the maxima of the launch).
+ * When the slots of all resident lanes do not fit 90 % of the free device memory, the size asks for fewer slots (at least
+ * one); le_td3_run then keeps fewer lanes resident and queues the rest.  Returns a negative LE_E* code on error. */
+int64_t le_td3_workspace_bytes(const le_td3_cfg* cfg_host0, int n_lanes, int n_env);
+
+/*
+ * The TD3 counterpart of le_inner_loop_run: n_lanes TD3_discrete_vary agents, one 256-thread CTA per lane, DEVICE buffers,
+ * asynchronous on `stream`.  vary_hp batches of transfer evaluations run here in one launch.
+ *   cfg_dev        [n_cfg] configurations (DEVICE); lane i uses cfg_dev[n_cfg == 1 ? 0 : i] with its own q_hidden, q_layers,
+ *                  batch_size, lr, ...; cfg_host0 = HOST copy of the maxima (q_hidden, q_layers, batch_size) that sizes the
+ *                  slots, and the configuration whose env / loop fields fix the ring capacity and the result strides
+ *   env_theta_dev  [n_env][P_se]; lane i uses row env_index_dev[i] (NULL: row 0); NULL for LE_ENV_REAL
+ *   keys_dev       [n_lanes][2] Philox lane keys
+ *   actor_init_dev / critic1_init_dev / critic2_init_dev   all NULL: every lane initialises its three nets on the device
+ *                  (torch default nn.Linear init from the P_TD3_INIT stream, restated in tests/td3_init_stream.py); else [n_init][P] with
+ *                  n_init = 1 (shared) or n_lanes, row stride = the parameter counts of cfg_host0 (le_td3_param_counts)
+ *   actor_final_dev NULL or [n_lanes][P_actor of cfg_host0]: trained actors (the first P_actor of lane i's own shape)
+ *   out_dev, rewards_dev, lengths_dev, test_rewards_dev   as for le_inner_loop_run
+ *   workspace_dev  le_td3_workspace_bytes() bytes (a smaller workspace that holds at least one slot runs fewer lanes at once)
+ *   trace_host     NULL or one le_trace (DEVICE pointers inside) that records lane `trace_lane`
+ * Training env: LE_ENV_SE or LE_ENV_REAL (LE_ENV_RN: LE_EUNSUPPORTED).
+ */
+int le_td3_run(const le_td3_cfg* cfg_dev, int n_cfg, const le_td3_cfg* cfg_host0, const float* env_theta_dev, int n_env,
+               const int32_t* env_index_dev, const uint32_t* keys_dev, const float* actor_init_dev, const float* critic1_init_dev,
+               const float* critic2_init_dev, int n_init, float* actor_final_dev, int n_lanes, le_lane_out* out_dev, double* rewards_dev,
+               int32_t* lengths_dev, double* test_rewards_dev, void* workspace_dev, int64_t workspace_bytes, const le_trace* trace_host,
+               int trace_lane, void* stream);
+
+/* Host-buffer wrapper of le_td3_run with one configuration for all lanes (arrays as above, HOST pointers). */
 int le_td3_run_host(const le_td3_cfg* cfg, const float* env_theta, int n_env, const int32_t* env_index, const uint32_t* keys,
                     const float* actor_init, const float* critic1_init, const float* critic2_init, int n_init, float* actor_final,
                     int n_lanes, le_lane_out* out, double* rewards, int32_t* lengths, double* test_rewards,

@@ -93,6 +93,18 @@ class Td3Cfg(C.Structure):
     _fields_ = [("base", LaneCfg), ("policy_delay", C.c_int32), ("gumbel_hard", C.c_int32), ("action_std", C.c_double),
                 ("policy_std", C.c_double), ("policy_std_clip", C.c_double), ("gumbel_temp", C.c_double), ("max_action", C.c_double)]
 
+    def copy(self):
+        o = Td3Cfg()
+        C.memmove(C.byref(o), C.byref(self), C.sizeof(Td3Cfg))
+        return o
+
+    def param_counts(self):
+        """(P_actor, P_critic) as le_td3_param_counts: actor sd -> H (x L) -> ad, critics sd+ad -> H (x L) -> 1."""
+        b = self.base
+        L, H = max(int(b.q_layers), 1), b.q_hidden
+        hidden = (L - 1) * (H * H + H)
+        return b.sd * H + H + hidden + H * b.ad + b.ad, (b.sd + b.ad) * H + H + hidden + H + 1
+
 
 class LaneOut(C.Structure):
     """struct le_lane_out."""
@@ -128,6 +140,7 @@ def load_library():
     lib.le_last_error.restype = C.c_char_p
     lib.le_version.restype = C.c_int
     lib.le_inner_loop_workspace_bytes.restype = C.c_int64
+    lib.le_td3_workspace_bytes.restype = C.c_int64
     _lib = lib
     return lib
 
@@ -137,7 +150,7 @@ EXPORTED_SYMBOLS = [
     "le_se_forward", "le_rn_reward", "le_qnet_forward", "le_real_env_step", "le_td_update", "le_tc_gemm",
     "le_inner_loop_workspace_bytes", "le_inner_loop_plan", "le_inner_loop_run", "le_inner_loop_run_host",
     "le_nes_perturb", "le_nes_noise", "le_nes_update", "le_nes_partial_update",
-    "le_td3_param_counts", "le_td3_run_host",
+    "le_td3_param_counts", "le_td3_workspace_bytes", "le_td3_run", "le_td3_run_host",
 ]
 
 

@@ -77,5 +77,19 @@ def lane_cfg(config, agent_name="ddqn", env_kind=ENV_SE, use_test_env=True, fina
     return c
 
 
+def td3_lane_cfg(config, env_kind=ENV_SE, use_test_env=True, final_test=True, max_action=1.0):
+    """le_td3_cfg of the config's td3_discrete_vary section (agents/TD3_discrete_vary.py:20-59); max_action of the discrete
+    envs is 1 (envs/env_wrapper.py:106-110).  The eps_* fields of the base configuration are unused by TD3 lanes."""
+    from ._abi import Td3Cfg
+    a = config["agents"]["td3_discrete_vary"]
+    cfg = dict(config, agents=dict(config["agents"], td3_discrete_vary=dict(a, eps_init=0.0, eps_min=0.0, eps_decay=0.0)))
+    t = Td3Cfg()
+    t.base = lane_cfg(cfg, "td3_discrete_vary", env_kind, use_test_env, final_test)
+    t.policy_delay, t.gumbel_hard = int(a["policy_delay"]), int(bool(a["gumbel_softmax_hard"]))
+    t.action_std, t.policy_std, t.policy_std_clip = float(a["action_std"]), float(a["policy_std"]), float(a["policy_std_clip"])
+    t.gumbel_temp, t.max_action = float(a["gumbel_softmax_temp"]), float(max_action)
+    return t
+
+
 def clone_config(config):
     return copy.deepcopy(config)

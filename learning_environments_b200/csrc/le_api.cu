@@ -674,6 +674,105 @@ int le_td3_param_counts(const le_td3_cfg* cfg, int* p_actor, int* p_critic) {
     return LE_OK;
 }
 
+// the checks shared by the TD3 entry points, on the (maxima) configuration; no CUDA call
+static int td3_check(const le_td3_cfg* cfg, const char* who) {
+    const le_lane_cfg* c = &cfg->base;
+    const int rc = check_env_cfg(c);
+    if (rc != LE_OK) return rc;
+    if (c->env_kind == LE_ENV_RN) { le_set_error("%s: reward-network training envs are not built for TD3 lanes", who); return LE_EUNSUPPORTED; }
+    if (qact_of(c) < 0 || c->q_hidden < 1 || c->q_layers > 3 || cfg->policy_delay < 1 || !(cfg->gumbel_temp > 0.0) || c->ad > 4 ||
+        c->batch_size < 1 || c->train_episodes < 0 || c->test_episodes < 1 || c->max_steps < 1) {
+        le_set_error("%s: configuration outside the compiled kernel set", who);
+        return LE_EUNSUPPORTED;
+    }
+    if (!le_find_instance(c->sd, c->ad, 1, QACT_TANH)) { le_set_error("no compiled kernel set for state_dim=%d action_dim=%d", c->sd, c->ad); return LE_EUNSUPPORTED; }
+    return LE_OK;
+}
+
+// workspace layout of the TD3 entry points: [SE pack | lane queue counter | resident lane slots]
+struct Td3Layout {
+    Td3Plan tp;
+    const InstanceOps* ops;
+    int ring_cap;
+    int64_t pack_stride_f, off_counter, off_slots, slot_bytes;
+};
+
+static int td3_layout(const le_td3_cfg* cfg, int n_lanes, int n_env, const char* who, Td3Layout* L) {
+    const le_lane_cfg* c = &cfg->base;
+    int rc = td3_check(cfg, who);
+    if (rc != LE_OK) return rc;
+    L->ops = le_find_instance(c->sd, c->ad, 1, QACT_TANH);
+    int dev = 0, sms = 0;
+    LE_CUDA_CHECK(cudaGetDevice(&dev));
+    LE_CUDA_CHECK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
+    L->ring_cap = ring_capacity(c);
+    rc = td3_plan(cfg, n_lanes, L->ring_cap, sms, &L->tp);
+    if (rc != LE_OK) return rc;
+    L->pack_stride_f = (c->env_kind == LE_ENV_SE ? L->ops->se_pack_vec4(c->env_hidden) : 1) * 4;
+    L->off_counter = ((int64_t)(n_env > 0 ? n_env : 1) * L->pack_stride_f * 4 + 255) / 256 * 256;
+    L->off_slots = L->off_counter + 256;
+    L->slot_bytes = L->tp.slot_floats * (int64_t)sizeof(float);
+    return LE_OK;
+}
+
+int64_t le_td3_workspace_bytes(const le_td3_cfg* cfg_host0, int n_lanes, int n_env) {
+    if (!cfg_host0 || n_lanes < 1) { le_set_error("le_td3_workspace_bytes: bad arguments"); return LE_EINVAL; }
+    Td3Layout L;
+    const int rc = td3_layout(cfg_host0, n_lanes, n_env, "le_td3_workspace_bytes", &L);
+    if (rc != LE_OK) return rc;
+    // a slot of the widest vary_hp shapes (hidden 1530 x 3 layers) is ~0.3 GB: when every resident lane's slot does not fit
+    // 90 % of the free device memory, ask for fewer slots (the lane queue runs the rest on them)
+    size_t free_b = 0, total_b = 0;
+    LE_CUDA_CHECK(cudaMemGetInfo(&free_b, &total_b));
+    const int64_t room = (int64_t)(0.9 * (double)free_b) - L.off_slots;
+    int64_t slots = L.tp.grid;
+    if (slots * L.slot_bytes > room) slots = room / L.slot_bytes > 1 ? room / L.slot_bytes : 1;
+    return L.off_slots + slots * L.slot_bytes;
+}
+
+int le_td3_run(const le_td3_cfg* cfg_dev, int n_cfg, const le_td3_cfg* cfg_host0, const float* env_theta_dev, int n_env,
+               const int32_t* env_index_dev, const uint32_t* keys_dev, const float* actor_init_dev, const float* critic1_init_dev,
+               const float* critic2_init_dev, int n_init, float* actor_final_dev, int n_lanes, le_lane_out* out_dev, double* rewards_dev,
+               int32_t* lengths_dev, double* test_rewards_dev, void* workspace_dev, int64_t workspace_bytes, const le_trace* trace_host,
+               int trace_lane, void* stream) {
+    const bool any_init = actor_init_dev || critic1_init_dev || critic2_init_dev;
+    const bool all_init = actor_init_dev && critic1_init_dev && critic2_init_dev;
+    if (!cfg_dev || !cfg_host0 || !keys_dev || !out_dev || !rewards_dev || !lengths_dev || !test_rewards_dev || !workspace_dev || n_lanes < 1 ||
+        (n_cfg != 1 && n_cfg != n_lanes) || any_init != all_init || (all_init && n_init != 1 && n_init != n_lanes)) {
+        le_set_error("le_td3_run: bad arguments (n_cfg and n_init must be 1 or n_lanes; all three init arrays or none; no NULL outputs)");
+        return LE_EINVAL;
+    }
+    Td3Layout L;
+    int rc = td3_layout(cfg_host0, n_lanes, n_env, "le_td3_run", &L);
+    if (rc != LE_OK) return rc;
+    const le_lane_cfg* c = &cfg_host0->base;
+    if (c->env_kind == LE_ENV_SE && (!env_theta_dev || n_env < 1)) { le_set_error("le_td3_run: env_theta is required for SE lanes"); return LE_EINVAL; }
+    // resident lanes: as many slots as the workspace holds, up to the occupancy-bound grid
+    const int64_t fit = workspace_bytes > L.off_slots ? (workspace_bytes - L.off_slots) / L.slot_bytes : 0;
+    if (fit < 1) {
+        le_set_error("le_td3_run: workspace too small (%lld < %lld bytes)", (long long)workspace_bytes, (long long)(L.off_slots + L.slot_bytes));
+        return LE_EINVAL;
+    }
+    if (fit < L.tp.grid) L.tp.grid = (int)fit;
+    cudaStream_t st = (cudaStream_t)stream;
+    char* ws = (char*)workspace_dev;
+    LE_CUDA_CHECK(cudaMemsetAsync(ws + L.off_counter, 0, 256, st));
+    LE_CUDA_CHECK(pack_env(L.ops, c, env_theta_dev, n_env, (float*)ws, L.pack_stride_f, st));
+    RunParams P;
+    memset(&P, 0, sizeof(P));
+    P.env_pack = (const float4*)ws; P.env_pack_stride = L.pack_stride_f / 4;
+    P.env_index = env_index_dev; P.keys = keys_dev;
+    P.n_lanes = n_lanes; P.out = out_dev; P.rewards = rewards_dev; P.lengths = lengths_dev; P.test_rewards = test_rewards_dev;
+    P.rew_stride = c->train_episodes > 0 ? c->train_episodes : 1; P.test_stride = c->test_episodes;
+    P.ring_cap = L.ring_cap;
+    P.work_counter = (int*)(ws + L.off_counter);
+    if (trace_host && trace_host->cap > 0) { P.trace = *trace_host; P.trace_lane = trace_lane; }
+    cudaError_t le = td3_launch(cfg_dev, n_cfg, cfg_host0, P, (float*)(ws + L.off_slots), L.tp, actor_init_dev, critic1_init_dev, critic2_init_dev,
+                                all_init && n_init == n_lanes && n_lanes > 1, actor_final_dev, st);
+    if (le != cudaSuccess) { le_set_error("td3 launch failed: %s", cudaGetErrorString(le)); return LE_ECUDA; }
+    return LE_OK;
+}
+
 int le_td3_run_host(const le_td3_cfg* cfg, const float* env_theta, int n_env, const int32_t* env_index, const uint32_t* keys,
                     const float* actor_init, const float* critic1_init, const float* critic2_init, int n_init, float* actor_final,
                     int n_lanes, le_lane_out* out, double* rewards, int32_t* lengths, double* test_rewards, const le_trace* trace_host,
@@ -684,35 +783,26 @@ int le_td3_run_host(const le_td3_cfg* cfg, const float* env_theta, int n_env, co
         return LE_EINVAL;
     }
     const le_lane_cfg* c = &cfg->base;
-    int rc = check_env_cfg(c);
+    int rc = td3_check(cfg, "le_td3_run_host");
     if (rc != LE_OK) return rc;
-    if (c->env_kind == LE_ENV_RN) { le_set_error("le_td3_run_host: reward-network training envs are not built for TD3 lanes"); return LE_EUNSUPPORTED; }
-    if (qact_of(c) < 0 || c->q_hidden < 1 || c->q_layers > 3 || cfg->policy_delay < 1 || !(cfg->gumbel_temp > 0.0) || c->ad > 4 ||
-        c->batch_size < 1 || c->train_episodes < 0 || c->test_episodes < 1 || c->max_steps < 1) {
-        le_set_error("le_td3_run_host: configuration outside the compiled kernel set");
-        return LE_EUNSUPPORTED;
-    }
-    const InstanceOps* ops = le_find_instance(c->sd, c->ad, 1, QACT_TANH);
-    if (!ops) { le_set_error("no compiled kernel set for state_dim=%d action_dim=%d", c->sd, c->ad); return LE_EUNSUPPORTED; }
     LE_CUDA_CHECK(cudaSetDevice(device));
-    int sms = 0;
-    LE_CUDA_CHECK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device));
-    const int ring_cap = ring_capacity(c);
-    Td3Plan tp;
-    rc = td3_plan(cfg, n_lanes, ring_cap, sms, &tp);
+    Td3Layout L;
+    rc = td3_layout(cfg, n_lanes, n_env, "le_td3_run_host", &L);
     if (rc != LE_OK) return rc;
     if (c->env_kind == LE_ENV_SE && (!env_theta || n_env < 1)) { le_set_error("le_td3_run_host: env_theta is required for SE lanes"); return LE_EINVAL; }
-    const int64_t pack_stride_f = (c->env_kind == LE_ENV_SE ? ops->se_pack_vec4(c->env_hidden) : 1) * 4;
+    const int64_t ws_bytes = le_td3_workspace_bytes(cfg, n_lanes, n_env);
+    if (ws_bytes < 0) return (int)ws_bytes;
     const int rs = c->train_episodes > 0 ? c->train_episodes : 1;
     const int tcap = trace_host ? trace_host->cap : 0;
     HostCall hc;
+    const size_t i_cfg = hc.add(cfg, nullptr, sizeof(le_td3_cfg));
     const size_t i_th = hc.add(env_theta, nullptr, sizeof(float) * (size_t)env_param_count(c) * n_env);
     const size_t i_ei = hc.add(env_index, nullptr, env_index ? sizeof(int32_t) * n_lanes : 0);
     const size_t i_key = hc.add(keys, nullptr, sizeof(uint32_t) * 2 * n_lanes);
-    const size_t i_a = hc.add(actor_init, nullptr, sizeof(float) * (size_t)tp.p_actor * n_init);
-    const size_t i_c1 = hc.add(critic1_init, nullptr, sizeof(float) * (size_t)tp.p_critic * n_init);
-    const size_t i_c2 = hc.add(critic2_init, nullptr, sizeof(float) * (size_t)tp.p_critic * n_init);
-    const size_t i_af = hc.add(nullptr, actor_final, actor_final ? sizeof(float) * (size_t)tp.p_actor * n_lanes : 0);
+    const size_t i_a = hc.add(actor_init, nullptr, sizeof(float) * (size_t)L.tp.p_actor * n_init);
+    const size_t i_c1 = hc.add(critic1_init, nullptr, sizeof(float) * (size_t)L.tp.p_critic * n_init);
+    const size_t i_c2 = hc.add(critic2_init, nullptr, sizeof(float) * (size_t)L.tp.p_critic * n_init);
+    const size_t i_af = hc.add(nullptr, actor_final, actor_final ? sizeof(float) * (size_t)L.tp.p_actor * n_lanes : 0);
     const size_t i_out = hc.add(nullptr, out, sizeof(le_lane_out) * n_lanes);
     const size_t i_rw = hc.add(nullptr, rewards, sizeof(double) * (size_t)rs * n_lanes);
     const size_t i_ln = hc.add(nullptr, lengths, sizeof(int32_t) * (size_t)rs * n_lanes);
@@ -723,33 +813,22 @@ int le_td3_run_host(const le_td3_cfg* cfg, const float* env_theta, int n_env, co
     const size_t i_trw = hc.add(nullptr, tcap ? trace_host->reward : nullptr, sizeof(float) * (size_t)tcap);
     const size_t i_td = hc.add(nullptr, tcap ? trace_host->done : nullptr, sizeof(float) * (size_t)tcap);
     const size_t i_tl = hc.add(nullptr, tcap ? trace_host->loss : nullptr, sizeof(float) * (size_t)tcap);
-    const size_t off_pack = hc.reserve(((size_t)(n_env > 0 ? n_env : 1) * pack_stride_f * 4 + 255) / 256 * 256);
-    const size_t off_counter = hc.reserve(256);
-    const size_t off_slots = hc.reserve((size_t)tp.grid * tp.slot_floats * sizeof(float));
+    const size_t off_ws = hc.reserve((size_t)ws_bytes);
     rc = hc.stage_in();
     if (rc != LE_OK) return rc;
     char* arena = hc.arena;
     LE_CUDA_CHECK(cudaMemsetAsync(arena + hc.segs[i_rw].off, 0, hc.segs[i_rw].bytes + hc.segs[i_ln].bytes, hc.st));
-    if (tcap) LE_CUDA_CHECK(cudaMemsetAsync(arena + hc.segs[i_ta].off, 0xff, off_pack - hc.segs[i_ta].off, hc.st));   /* untouched trace slots: -1 / NaN */
-    LE_CUDA_CHECK(cudaMemsetAsync(arena + off_counter, 0, 256, hc.st));
-    LE_CUDA_CHECK(pack_env(ops, c, (const float*)hc.dp(i_th), n_env, (float*)(arena + off_pack), pack_stride_f, hc.st));
-    RunParams P;
-    memset(&P, 0, sizeof(P));
-    P.env_pack = (const float4*)(arena + off_pack); P.env_pack_stride = pack_stride_f / 4;
-    P.env_index = (const int32_t*)hc.dp(i_ei); P.keys = (const uint32_t*)hc.dp(i_key);
-    P.n_lanes = n_lanes; P.out = (le_lane_out*)hc.dp(i_out); P.rewards = (double*)hc.dp(i_rw); P.lengths = (int32_t*)hc.dp(i_ln);
-    P.test_rewards = (double*)hc.dp(i_tr);
-    P.rew_stride = rs; P.test_stride = c->test_episodes;
-    P.ring_cap = ring_cap;
-    P.work_counter = (int*)(arena + off_counter);
+    le_trace tr;
+    memset(&tr, 0, sizeof(tr));
     if (tcap) {
-        P.trace.cap = tcap; P.trace.action = (int32_t*)hc.dp(i_ta); P.trace.explore = (int32_t*)hc.dp(i_te); P.trace.next_state = (float*)hc.dp(i_tn);
-        P.trace.reward = (float*)hc.dp(i_trw); P.trace.done = (float*)hc.dp(i_td); P.trace.loss = (float*)hc.dp(i_tl);
-        P.trace_lane = trace_lane;
+        LE_CUDA_CHECK(cudaMemsetAsync(arena + hc.segs[i_ta].off, 0xff, off_ws - hc.segs[i_ta].off, hc.st));   /* untouched trace slots: -1 / NaN */
+        tr.cap = tcap; tr.action = (int32_t*)hc.dp(i_ta); tr.explore = (int32_t*)hc.dp(i_te); tr.next_state = (float*)hc.dp(i_tn);
+        tr.reward = (float*)hc.dp(i_trw); tr.done = (float*)hc.dp(i_td); tr.loss = (float*)hc.dp(i_tl);
     }
-    cudaError_t le = td3_launch(cfg, P, (float*)(arena + off_slots), tp, (const float*)hc.dp(i_a), (const float*)hc.dp(i_c1),
-                                (const float*)hc.dp(i_c2), n_init == n_lanes && n_lanes > 1, (float*)hc.dp(i_af), hc.st);
-    if (le != cudaSuccess) { le_set_error("td3 launch failed: %s", cudaGetErrorString(le)); rc = LE_ECUDA; }
+    rc = le_td3_run((const le_td3_cfg*)hc.dp(i_cfg), 1, cfg, (const float*)hc.dp(i_th), n_env, (const int32_t*)hc.dp(i_ei),
+                    (const uint32_t*)hc.dp(i_key), (const float*)hc.dp(i_a), (const float*)hc.dp(i_c1), (const float*)hc.dp(i_c2), n_init,
+                    (float*)hc.dp(i_af), n_lanes, (le_lane_out*)hc.dp(i_out), (double*)hc.dp(i_rw), (int32_t*)hc.dp(i_ln), (double*)hc.dp(i_tr),
+                    arena + off_ws, ws_bytes, tcap ? &tr : nullptr, trace_lane, hc.st);
     return hc.stage_out(rc, "le_td3_run_host");   // ~HostCall frees the arena and destroys the stream
 }
 

@@ -7,13 +7,16 @@
 //       the environment receives argmax (agents/base_agent.py:111-114), the replay ring the action VECTOR;
 //   learn (:62-119): target policy smoothing, twin target critics (min), two Adam optimizers, delayed policy update through
 //       critic_1 with the straight-through Gumbel-softmax gradient, Polyak on the three targets.
-// Random draws: Philox streams P_TD3_EXPO / P_TD3_NORMAL (documented with the CPU restatement's stream table).
+// Every lane copies its own le_td3_cfg into shared memory and builds its actor / critic GNets there (vary_hp: per-lane
+// q_hidden, q_layers, batch_size, lr, ...); the slot workspace is sized for the maxima configuration of the launch.
+// Random draws: Philox streams P_TD3_EXPO / P_TD3_NORMAL (documented with the CPU restatement's stream table) and P_TD3_INIT
+// (device init of the nets; restated in numpy by tests/td3_init_stream.py).
 #include "le_general.cuh"
 #include "le_td3_api.h"
 
 namespace le {
 
-constexpr uint32_t LE_P_TD3_EXPO = 8u, LE_P_TD3_NORMAL = 9u;
+constexpr uint32_t LE_P_TD3_EXPO = 8u, LE_P_TD3_NORMAL = 9u, LE_P_TD3_INIT = 10u;
 
 // Exp(1) draw i of (phase, c0, sub): -ln((w + 0.5) * 2^-32) in fp64, rounded to fp32
 __device__ __forceinline__ float td3_expo(uint32_t k0, uint32_t k1, uint32_t phase, uint32_t c0, uint32_t sub, int i) {
@@ -59,6 +62,19 @@ __host__ __device__ inline void tnet_build(GNet* n, int in, int H, int L, int ou
     n->P = p; n->sum_out = y;
 }
 
+// torch's default nn.Linear init, U(-1/sqrt(fan_in), +1/sqrt(fan_in)) for W and b (as g_init_layer), of TD3 net `net_id`
+// (0 actor, 1 critic 1, 2 critic 2) from the P_TD3_INIT stream: parameter p takes word p & 3 of counter (p >> 2, net_id, P_TD3_INIT, 0)
+static __device__ void td3_init_net(const GNet& n, float* th, uint32_t net_id, uint32_t k0, uint32_t k1) {
+    for (int i = 0; i < n.nfeat; ++i) {
+        const GLayer& l = n.feat[i];
+        const double bnd = 1.0 / sqrt((double)l.in);
+        for (int p = l.w_off + threadIdx.x; p < l.b_off + l.out; p += kGThreads) {
+            const u32x4 w = philox4x32_10((uint32_t)(p >> 2), net_id, LE_P_TD3_INIT, 0u, k0, k1);
+            th[p] = (float)((2.0 * (((double)pick(w, p & 3) + 0.5) * (1.0 / 4294967296.0)) - 1.0) * bnd);
+        }
+    }
+}
+
 // backward of all layers for B rows: dact holds dL/d(output layer) at its y_off (everything else is overwritten);
 // grad <- parameter gradients; dX (may be null) <- dL/d(input rows), row stride dxs
 static __device__ void t_net_backward(const GNet& n, const float* th, float* grad, const float* X, int xs, const float* acts, float* dact, int B,
@@ -78,13 +94,13 @@ struct TSlot {
 
 struct TRunParams {
     RunParams rp;
-    le_td3_cfg tc;
-    GNet na, nc;
+    const le_td3_cfg* cfg; int n_cfg;   // lane i runs cfg[n_cfg == 1 ? 0 : i] (device memory)
+    GNet na_max, nc_max;                // nets of the maxima configuration: they fix the slot layout
     float* slots; int64_t slot_stride;
     int bmax, rowf;
-    const float *actor_init, *c1_init, *c2_init;   // [n_lanes][P] or the same for all lanes when init_stride == 0
+    const float *actor_init, *c1_init, *c2_init;   // null: device init; else row lane_id * init_stride (stride 0: one row for all lanes)
     int init_stride_a, init_stride_c;
-    float* actor_final;
+    float* actor_final; int final_stride;
 };
 
 __host__ __device__ inline int64_t tslot_floats(const GNet& na, const GNet& nc, int sd, int ad, int ring_cap, int rowf, int bmax, int64_t* offs /* [26] */) {
@@ -122,7 +138,10 @@ template <int SD, int AD>
 struct Td3Agent {
     static constexpr int XI = SD + AD;
     const TRunParams& G;
-    const TSlot w;
+    const TSlot w;     // sized for the maxima
+    le_td3_cfg& tc;    // this lane's configuration and nets, in shared memory
+    GNet& na;
+    GNet& nc;
     float* sm;
     float* red;
     uint32_t k0, k1;
@@ -135,22 +154,42 @@ struct Td3Agent {
     __device__ __forceinline__ const le_lane_cfg& begin_lane(int lane_id, uint32_t key0, uint32_t key1) {
         const int tid = threadIdx.x;
         k0 = key0; k1 = key1;
-        // targets = copies, Adam state zero (agents/TD3_discrete_vary.py:41-52)
-        for (int p = tid; p < G.na.P; p += kGThreads) {
-            const float v0 = G.actor_init[(int64_t)lane_id * G.init_stride_a + p];
-            w.actor[p] = v0; w.actorT[p] = v0; w.m_a[p] = 0.f; w.v_a[p] = 0.f;
-        }
-        for (int p = tid; p < G.nc.P; p += kGThreads) {
-            const float a1 = G.c1_init[(int64_t)lane_id * G.init_stride_c + p], a2 = G.c2_init[(int64_t)lane_id * G.init_stride_c + p];
-            w.c1[p] = a1; w.c1T[p] = a1; w.m_c1[p] = 0.f; w.v_c1[p] = 0.f;
-            w.c2[p] = a2; w.c2T[p] = a2; w.m_c2[p] = 0.f; w.v_c2[p] = 0.f;
+        {
+            const uint32_t* src = reinterpret_cast<const uint32_t*>(G.cfg + (G.n_cfg == 1 ? 0 : lane_id));
+            uint32_t* dst = reinterpret_cast<uint32_t*>(&tc);
+            for (int i = tid; i < (int)(sizeof(le_td3_cfg) / 4); i += kGThreads) dst[i] = src[i];
         }
         __syncthreads();
-        fill_learn_scalars(ls, G.tc.base);
+        if (tid == 0) {
+            const le_lane_cfg& c = tc.base;
+            tnet_build(&na, c.sd, c.q_hidden, c.q_layers, c.ad, c.q_act);
+            tnet_build(&nc, c.sd + c.ad, c.q_hidden, c.q_layers, 1, c.q_act);
+        }
+        __syncthreads();
+        if (G.actor_init) {
+            for (int p = tid; p < na.P; p += kGThreads) w.actor[p] = G.actor_init[(int64_t)lane_id * G.init_stride_a + p];
+            for (int p = tid; p < nc.P; p += kGThreads) {
+                w.c1[p] = G.c1_init[(int64_t)lane_id * G.init_stride_c + p];
+                w.c2[p] = G.c2_init[(int64_t)lane_id * G.init_stride_c + p];
+            }
+        } else {
+            td3_init_net(na, w.actor, 0u, k0, k1);
+            td3_init_net(nc, w.c1, 1u, k0, k1);
+            td3_init_net(nc, w.c2, 2u, k0, k1);
+        }
+        __syncthreads();
+        // targets = copies, Adam state zero (agents/TD3_discrete_vary.py:41-52)
+        for (int p = tid; p < na.P; p += kGThreads) { w.actorT[p] = w.actor[p]; w.m_a[p] = 0.f; w.v_a[p] = 0.f; }
+        for (int p = tid; p < nc.P; p += kGThreads) {
+            w.c1T[p] = w.c1[p]; w.m_c1[p] = 0.f; w.v_c1[p] = 0.f;
+            w.c2T[p] = w.c2[p]; w.m_c2[p] = 0.f; w.v_c2[p] = 0.f;
+        }
+        __syncthreads();
+        fill_learn_scalars(ls, tc.base);
         b1pow_a = 1.0; b2pow_a = 1.0; b1pow_c = 1.0; b2pow_c = 1.0;
-        temp = (float)G.tc.gumbel_temp;
+        temp = (float)tc.gumbel_temp;
         total_it = 0;
-        return G.tc.base;
+        return tc.base;
     }
 
     __device__ __forceinline__ void begin_episode(int) {}
@@ -159,20 +198,20 @@ struct Td3Agent {
     // Returns this thread's argmax; av <- the action vector.
     __device__ __forceinline__ int act_rows(const float* Xrows, int xs, int M, uint32_t phase, uint32_t c0, uint32_t sub_of_thread, bool active,
                                             float (&av)[AD]) {
-        const int Sa = G.na.sum_out, yo_a = G.na.feat[G.na.nfeat - 1].y_off;
-        g_net_forward(G.na, w.actor, Xrows, xs, M, w.Aa, sm);
+        const int Sa = na.sum_out, yo_a = na.feat[na.nfeat - 1].y_off;
+        g_net_forward(na, w.actor, Xrows, xs, M, w.Aa, sm);
         int best = 0;
         if (active) {
             float logits[AD], expo[AD], y[AD], ret[AD];
 #pragma unroll
             for (int k = 0; k < AD; ++k) {
-                logits[k] = __ldcg(w.Aa + (int64_t)threadIdx.x * Sa + yo_a + k) * (float)G.tc.max_action;
+                logits[k] = __ldcg(w.Aa + (int64_t)threadIdx.x * Sa + yo_a + k) * (float)tc.max_action;
                 expo[k] = td3_expo(k0, k1, phase, c0, sub_of_thread, k);
             }
-            gumbel_softmax_row<AD>(logits, expo, temp, G.tc.gumbel_hard, y, ret);
+            gumbel_softmax_row<AD>(logits, expo, temp, tc.gumbel_hard, y, ret);
 #pragma unroll
             for (int k = 0; k < AD; ++k) {
-                av[k] = ret[k] + td3_normal(k0, k1, phase, c0, sub_of_thread, k) * (float)G.tc.action_std;
+                av[k] = ret[k] + td3_normal(k0, k1, phase, c0, sub_of_thread, k) * (float)tc.action_std;
                 if (av[k] > av[best]) best = k;
             }
         }
@@ -180,9 +219,9 @@ struct Td3Agent {
     }
 
     // select_train_action (:155-162): random before init_episodes, then the actor on row 0; `box` broadcasts the action vector
-    __device__ __forceinline__ int train_action(const float (&state)[SD], int episode, int64_t train_steps, bool, bool& explore, float&,
-                                                float* box) {
-        explore = episode < G.tc.base.init_episodes;
+    __device__ __forceinline__ int train_action(const float (&state)[SD], int episode, int64_t train_steps, bool tracing, bool& explore,
+                                                float& qgap, float* box) {
+        explore = episode < tc.base.init_episodes;
         if (explore) {
             const u32x4 wa = philox4x32_10((uint32_t)train_steps, 0u, LE_P_ACT, 0u, k0, k1);
             const int action = (int)__umulhi(wa.y, (uint32_t)AD);
@@ -204,6 +243,7 @@ struct Td3Agent {
         int action = 0;
 #pragma unroll
         for (int k = 0; k < AD; ++k) { avec[k] = box[k]; if (avec[k] > avec[action]) action = k; }
+        if (tracing) qgap = relative_q_gap<AD>(avec, action);   // near-tie marker of the noisy action vector's argmax
         __syncthreads();
         return action;
     }
@@ -223,13 +263,11 @@ struct Td3Agent {
 
     // learn (:62-119)
     __device__ __forceinline__ float learn(int64_t learn_iters, int rb_size) {
-        const GNet& na = G.na;
-        const GNet& nc = G.nc;
         const int tid = threadIdx.x;
         const int Sa = na.sum_out, Sc = nc.sum_out, yo_a = na.feat[na.nfeat - 1].y_off, yo_c = nc.feat[nc.nfeat - 1].y_off;
-        const float max_action = (float)G.tc.max_action, policy_std = (float)G.tc.policy_std, policy_clip = (float)G.tc.policy_std_clip;
-        const int hard = G.tc.gumbel_hard;
-        const double T0 = G.tc.gumbel_temp, Tstep = (T0 / 20.0 - T0) / 1999.0;      // np.linspace(T0, T0/20, 2000)
+        const float max_action = (float)tc.max_action, policy_std = (float)tc.policy_std, policy_clip = (float)tc.policy_std_clip;
+        const int hard = tc.gumbel_hard;
+        const double T0 = tc.gumbel_temp, Tstep = (T0 / 20.0 - T0) / 1999.0;      // np.linspace(T0, T0/20, 2000)
         __syncthreads();
         temp = (float)(total_it >= 1999 ? T0 / 20.0 : (double)total_it * Tstep + T0);
         total_it += 1;
@@ -292,7 +330,7 @@ struct Td3Agent {
             t_net_backward(nc, cth, w.g_c, w.X, XI, w.A1, w.D, B, nullptr, 0, sm);
             g_adam(cth, nullptr, which ? w.m_c2 : w.m_c1, which ? w.v_c2 : w.v_c1, w.g_c, nc.P, ls, b1pow_c, b2pow_c);
         }
-        if (total_it % G.tc.policy_delay == 0) {
+        if (total_it % tc.policy_delay == 0) {
             // actor loss = -mean(critic_1(s, actor(s))) through the (updated) critic and the straight-through Gumbel-softmax
             g_net_forward(na, w.actor, w.X, XI, B, w.Aa, sm);
             for (int b = tid; b < B; b += kGThreads) {
@@ -346,7 +384,7 @@ struct Td3Agent {
     }
 
     __device__ __forceinline__ void end_lane(int lane_id) {
-        if (G.actor_final) for (int p = threadIdx.x; p < G.na.P; p += kGThreads) G.actor_final[(int64_t)lane_id * G.na.P + p] = w.actor[p];
+        if (G.actor_final) for (int p = threadIdx.x; p < na.P; p += kGThreads) G.actor_final[(int64_t)lane_id * G.final_stride + p] = w.actor[p];
     }
 };
 
@@ -355,7 +393,10 @@ __global__ void __launch_bounds__(kGThreads, 2) td3_loop_kernel(const TRunParams
     static_assert(AD <= 4, "action vectors are handled as register arrays");
     __shared__ __align__(16) float sm[kGSmemFloats];
     __shared__ float red[32];
-    Td3Agent<SD, AD> ag{G, tslot_view(G.slots + (int64_t)blockIdx.x * G.slot_stride, G.na, G.nc, SD, AD, G.rp.ring_cap, G.rowf, G.bmax), sm, red};
+    __shared__ le_td3_cfg cfg_sm;
+    __shared__ GNet na_sm, nc_sm;
+    Td3Agent<SD, AD> ag{G, tslot_view(G.slots + (int64_t)blockIdx.x * G.slot_stride, G.na_max, G.nc_max, SD, AD, G.rp.ring_cap, G.rowf, G.bmax),
+                        cfg_sm, na_sm, nc_sm, sm, red};
     cta_lane_loop<SD, AD>(G.rp, ag);
 }
 
@@ -379,19 +420,19 @@ int td3_plan(const le_td3_cfg* tc, int n_lanes, int ring_cap, int sms, Td3Plan* 
     return LE_OK;
 }
 
-cudaError_t td3_launch(const le_td3_cfg* tc, const RunParams& rp, float* slots, const Td3Plan& tp, const float* actor_init, const float* c1_init,
-                       const float* c2_init, int per_lane_init, float* actor_final, cudaStream_t st) {
+cudaError_t td3_launch(const le_td3_cfg* cfg_dev, int n_cfg, const le_td3_cfg* cfg_host0, const RunParams& rp, float* slots, const Td3Plan& tp,
+                       const float* actor_init, const float* c1_init, const float* c2_init, int per_lane_init, float* actor_final, cudaStream_t st) {
     TRunParams G;
     G.rp = rp;
-    G.tc = *tc;
-    const le_lane_cfg* c = &tc->base;
-    tnet_build(&G.na, c->sd, c->q_hidden, c->q_layers, c->ad, c->q_act);
-    tnet_build(&G.nc, c->sd + c->ad, c->q_hidden, c->q_layers, 1, c->q_act);
+    G.cfg = cfg_dev; G.n_cfg = n_cfg;
+    const le_lane_cfg* c = &cfg_host0->base;
+    tnet_build(&G.na_max, c->sd, c->q_hidden, c->q_layers, c->ad, c->q_act);
+    tnet_build(&G.nc_max, c->sd + c->ad, c->q_hidden, c->q_layers, 1, c->q_act);
     G.slots = slots; G.slot_stride = tp.slot_floats; G.bmax = tp.bmax; G.rowf = tp.rowf;
     G.actor_init = actor_init; G.c1_init = c1_init; G.c2_init = c2_init;
     G.init_stride_a = per_lane_init ? tp.p_actor : 0;
     G.init_stride_c = per_lane_init ? tp.p_critic : 0;
-    G.actor_final = actor_final;
+    G.actor_final = actor_final; G.final_stride = tp.p_actor;
     if (c->sd == 4) td3_loop_kernel<4, 2><<<tp.grid, kGThreads, 0, st>>>(G);
     else td3_loop_kernel<6, 3><<<tp.grid, kGThreads, 0, st>>>(G);
     return cudaGetLastError();

@@ -310,6 +310,84 @@ def td3_param_counts(tcfg):
     return a.value, c.value
 
 
+class Td3Buffers(object):
+    """Device buffers of one le_td3_run call, sized for `tcfg0` (the maxima configuration of the launch); the counterpart of
+    InnerLoopBuffers for TD3_discrete_vary lanes."""
+
+    def __init__(self, tcfg0, n_lanes, n_env, device, n_cfg=1, trace_cap=0, want_actor_final=False):
+        assert isinstance(tcfg0, Td3Cfg)
+        self.cfg, self.n_lanes, self.n_env, self.device = tcfg0, n_lanes, n_env, device
+        c = tcfg0.base
+        ws = _lib().le_td3_workspace_bytes(C.byref(tcfg0), C.c_int(n_lanes), C.c_int(n_env))
+        if ws < 0:
+            check(int(ws), "le_td3_workspace_bytes")
+        self.workspace = torch.empty(int(ws), dtype=torch.uint8, device=device)
+        self.p_actor, self.p_critic = td3_param_counts(tcfg0)
+        rs = max(c.train_episodes, 1)
+        self.out = torch.zeros((n_lanes, C.sizeof(LaneOut)), dtype=torch.uint8, device=device)
+        self.rewards = torch.zeros((n_lanes, rs), dtype=_F64, device=device)
+        self.lengths = torch.zeros((n_lanes, rs), dtype=_I32, device=device)
+        self.test_rewards = torch.zeros((n_lanes, c.test_episodes), dtype=_F64, device=device)
+        self.actor_final = torch.zeros((n_lanes, self.p_actor), dtype=_F32, device=device) if want_actor_final else None
+        self.cfg_dev = torch.zeros((n_cfg, C.sizeof(Td3Cfg)), dtype=torch.uint8, device=device)
+        self.trace = None
+        if trace_cap > 0:
+            self.trace = dict(cap=trace_cap,
+                              action=torch.full((trace_cap,), -1, dtype=_I32, device=device),
+                              explore=torch.zeros(trace_cap, dtype=_I32, device=device),
+                              next_state=torch.zeros((trace_cap, c.sd), dtype=_F32, device=device),
+                              reward=torch.zeros(trace_cap, dtype=_F32, device=device),
+                              done=torch.zeros(trace_cap, dtype=_F32, device=device),
+                              loss=torch.full((trace_cap,), float("nan"), dtype=_F32, device=device),
+                              qgap=torch.full((trace_cap,), float("nan"), dtype=_F32, device=device))
+
+    def results(self):
+        return np.frombuffer(self.out.cpu().numpy().tobytes(), dtype=lane_out_dtype())
+
+
+def td3_run(bufs, tcfgs, env_theta, env_index, keys, inits=None, trace_lane=0):
+    """le_td3_run on the current stream: n_lanes TD3_discrete_vary lanes, lane i with tcfgs[i] (or one Td3Cfg for all).
+
+    Every configuration must fit the maxima `bufs.cfg` (q_hidden, q_layers, batch_size).  env_theta [n_env, P_se] CUDA f32 (None
+    for ENV_REAL); env_index [n_lanes] int32 or None; keys [n_lanes, 2] int32 CUDA (keys_tensor).  inits: None (device init from
+    the P_TD3_INIT stream) or (actor, critic_1, critic_2) CUDA f32 [1 or n_lanes, P of bufs.cfg] with each lane's own vector first
+    in its row."""
+    if isinstance(tcfgs, Td3Cfg):
+        tcfgs = [tcfgs]
+    n_cfg = len(tcfgs)
+    assert n_cfg in (1, bufs.n_lanes) and bufs.cfg_dev.shape[0] == n_cfg
+    m = bufs.cfg.base
+    for t in tcfgs:
+        if t.base.q_hidden > m.q_hidden or t.base.q_layers > m.q_layers or t.base.batch_size > m.batch_size:
+            raise ValueError("a lane configuration exceeds the maxima the buffers were sized for")
+    raw = b"".join(bytes(t) for t in tcfgs)
+    if getattr(bufs, "_cfg_raw", None) != raw:
+        bufs.cfg_dev.copy_(torch.frombuffer(bytearray(raw), dtype=torch.uint8).reshape(n_cfg, -1), non_blocking=False)
+        bufs._cfg_raw = raw
+    keys = _dev(keys, _I32)
+    assert keys.numel() == 2 * bufs.n_lanes
+    a0 = q1 = q2 = None
+    n_init = 0
+    if inits is not None:
+        a0, q1, q2 = inits
+        n_init = a0.shape[0]
+        assert a0.shape == (n_init, bufs.p_actor) and q1.shape == q2.shape == (n_init, bufs.p_critic) and n_init in (1, bufs.n_lanes)
+        a0, q1, q2 = (_dev(x, _F32) for x in (a0, q1, q2))
+    tr = None
+    if bufs.trace is not None:
+        tr = Trace()
+        tr.cap = bufs.trace["cap"]
+        for n in ("action", "explore", "next_state", "reward", "done", "loss", "qgap"):
+            setattr(tr, n, bufs.trace[n].data_ptr())
+    n_env = 0 if env_theta is None else env_theta.reshape(-1, max(m.env_params(), 1)).shape[0]
+    with _on(bufs.workspace) as stream:
+        check(_lib().le_td3_run(
+            _ptr(bufs.cfg_dev), C.c_int(n_cfg), C.byref(bufs.cfg), _ptr(env_theta), C.c_int(n_env), _ptr(env_index), _ptr(keys),
+            _ptr(a0), _ptr(q1), _ptr(q2), C.c_int(n_init), _ptr(bufs.actor_final), C.c_int(bufs.n_lanes), _ptr(bufs.out),
+            _ptr(bufs.rewards), _ptr(bufs.lengths), _ptr(bufs.test_rewards), _ptr(bufs.workspace), C.c_int64(bufs.workspace.numel()),
+            C.byref(tr) if tr is not None else None, C.c_int(trace_lane), stream), "le_td3_run")
+
+
 def td3_run_host(tcfg, env_theta, env_index, keys, actor_init, critic1_init, critic2_init, trace_cap=0, trace_lane=0, device=0):
     """le_td3_run_host: n TD3_discrete_vary lanes (train with per-episode test + final test), HOST numpy buffers in and out.
     actor_init [1 or n, P_actor], critic*_init [1 or n, P_critic].  Returns a dict of arrays (+ 'trace' when trace_cap > 0)."""

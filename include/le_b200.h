@@ -275,6 +275,27 @@ int le_td3_run(const le_td3_cfg* cfg_dev, int n_cfg, const le_td3_cfg* cfg_host0
                int32_t* lengths_dev, double* test_rewards_dev, void* workspace_dev, int64_t workspace_bytes, const le_trace* trace_host,
                int trace_lane, void* stream);
 
+/* TD3_discrete_vary.learn (agents/TD3_discrete_vary.py:62-119) on explicit minibatches and explicit random draws, for n lanes
+ * of one configuration (batch_size = B; the env / loop fields are not read).  The lane kernel runs the same device step after
+ * its replay_buffer.sample.  DEVICE pointers, asynchronous on `stream`; P_actor / P_critic as le_td3_param_counts:
+ *   actor, actor_target                 [n][P_actor]    updated in place
+ *   critic1/2, critic1/2_target         [n][P_critic]   updated in place
+ *   adam_m/v_actor, adam_m/v_critic1/2  Adam moments of the two optimizers (one over both critics), updated in place
+ *   counters_dev  [n][3] int32: actor Adam steps, critic Adam steps, self.total_it BEFORE the call; all three advanced.
+ *                 The Gumbel temperature is np.linspace(T0, T0/20, 2000)[min(total_it, 1999)], T0 = gumbel_temp; the policy is
+ *                 updated when (total_it + 1) % policy_delay == 0
+ *   rows_dev      [n][B][2sd+ad+2] = [s | action vector | s' | r | d]
+ *   policy_noise_dev, expo_target_dev, expo_actor_dev   [n][B][ad]: randn_like of the target policy noise and the Exp(1) draws of
+ *                 the target / actor gumbel_softmax (expo_actor is read only on policy-update calls)
+ *   critic_loss_dev [n] out
+ * LE_EINVAL: NULL pointers, n < 1, batch_size < 1.  LE_EUNSUPPORTED: ad > 4, hidden_layer > 3, policy_delay < 1, gumbel_temp <= 0,
+ * an unknown activation or no compiled kernel for (sd, ad). */
+int le_td3_learn(const le_td3_cfg* cfg, float* actor_dev, float* actor_target_dev, float* critic1_dev, float* critic1_target_dev,
+                 float* critic2_dev, float* critic2_target_dev, float* adam_m_actor_dev, float* adam_v_actor_dev, float* adam_m_critic1_dev,
+                 float* adam_v_critic1_dev, float* adam_m_critic2_dev, float* adam_v_critic2_dev, int32_t* counters_dev, int n,
+                 const float* rows_dev, const float* policy_noise_dev, const float* expo_target_dev, const float* expo_actor_dev,
+                 float* critic_loss_dev, void* stream);
+
 /* Host-buffer wrapper of le_td3_run with one configuration for all lanes (arrays as above, HOST pointers). */
 int le_td3_run_host(const le_td3_cfg* cfg, const float* env_theta, int n_env, const int32_t* env_index, const uint32_t* keys,
                     const float* actor_init, const float* critic1_init, const float* critic2_init, int n_init, float* actor_final,

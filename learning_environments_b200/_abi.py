@@ -141,6 +141,8 @@ def load_library():
     lib.le_version.restype = C.c_int
     lib.le_inner_loop_workspace_bytes.restype = C.c_int64
     lib.le_td3_workspace_bytes.restype = C.c_int64
+    lib.le_td3_learn.argtypes = [C.c_void_p] + [C.c_void_p] * 13 + [C.c_int] + [C.c_void_p] * 6
+    lib.le_td3_learn.restype = C.c_int
     _lib = lib
     return lib
 
@@ -150,7 +152,7 @@ EXPORTED_SYMBOLS = [
     "le_se_forward", "le_rn_reward", "le_qnet_forward", "le_real_env_step", "le_td_update", "le_tc_gemm",
     "le_inner_loop_workspace_bytes", "le_inner_loop_plan", "le_inner_loop_run", "le_inner_loop_run_host",
     "le_nes_perturb", "le_nes_noise", "le_nes_update", "le_nes_partial_update",
-    "le_td3_param_counts", "le_td3_workspace_bytes", "le_td3_run", "le_td3_run_host",
+    "le_td3_param_counts", "le_td3_workspace_bytes", "le_td3_run", "le_td3_run_host", "le_td3_learn",
 ]
 
 

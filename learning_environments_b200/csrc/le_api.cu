@@ -674,19 +674,45 @@ int le_td3_param_counts(const le_td3_cfg* cfg, int* p_actor, int* p_critic) {
     return LE_OK;
 }
 
-// the checks shared by the TD3 entry points, on the (maxima) configuration; no CUDA call
-static int td3_check(const le_td3_cfg* cfg, const char* who) {
+// the checks of the fields a learn() step reads (nets, minibatch, TD3 hyper-parameters); no CUDA call
+static int td3_learn_check(const le_td3_cfg* cfg, const char* who) {
     const le_lane_cfg* c = &cfg->base;
-    const int rc = check_env_cfg(c);
-    if (rc != LE_OK) return rc;
-    if (c->env_kind == LE_ENV_RN) { le_set_error("%s: reward-network training envs are not built for TD3 lanes", who); return LE_EUNSUPPORTED; }
     if (qact_of(c) < 0 || c->q_hidden < 1 || c->q_layers > 3 || cfg->policy_delay < 1 || !(cfg->gumbel_temp > 0.0) || c->ad > 4 ||
-        c->batch_size < 1 || c->train_episodes < 0 || c->test_episodes < 1 || c->max_steps < 1) {
+        c->batch_size < 1) {
         le_set_error("%s: configuration outside the compiled kernel set", who);
         return LE_EUNSUPPORTED;
     }
     if (!le_find_instance(c->sd, c->ad, 1, QACT_TANH)) { le_set_error("no compiled kernel set for state_dim=%d action_dim=%d", c->sd, c->ad); return LE_EUNSUPPORTED; }
     return LE_OK;
+}
+
+// the checks shared by the TD3 lane entry points, on the (maxima) configuration; no CUDA call
+static int td3_check(const le_td3_cfg* cfg, const char* who) {
+    const le_lane_cfg* c = &cfg->base;
+    int rc = check_env_cfg(c);
+    if (rc != LE_OK) return rc;
+    if (c->env_kind == LE_ENV_RN) { le_set_error("%s: reward-network training envs are not built for TD3 lanes", who); return LE_EUNSUPPORTED; }
+    if (c->train_episodes < 0 || c->test_episodes < 1 || c->max_steps < 1) {
+        le_set_error("%s: configuration outside the compiled kernel set", who);
+        return LE_EUNSUPPORTED;
+    }
+    return td3_learn_check(cfg, who);
+}
+
+int le_td3_learn(const le_td3_cfg* cfg, float* actor_dev, float* actor_target_dev, float* critic1_dev, float* critic1_target_dev,
+                 float* critic2_dev, float* critic2_target_dev, float* adam_m_actor_dev, float* adam_v_actor_dev, float* adam_m_critic1_dev,
+                 float* adam_v_critic1_dev, float* adam_m_critic2_dev, float* adam_v_critic2_dev, int32_t* counters_dev, int n,
+                 const float* rows_dev, const float* policy_noise_dev, const float* expo_target_dev, const float* expo_actor_dev,
+                 float* critic_loss_dev, void* stream) {
+    float* const nets[6] = {actor_dev, actor_target_dev, critic1_dev, critic1_target_dev, critic2_dev, critic2_target_dev};
+    float* const adam[6] = {adam_m_actor_dev, adam_v_actor_dev, adam_m_critic1_dev, adam_v_critic1_dev, adam_m_critic2_dev, adam_v_critic2_dev};
+    bool any_null = !cfg || !counters_dev || !rows_dev || !policy_noise_dev || !expo_target_dev || !expo_actor_dev || !critic_loss_dev;
+    for (int i = 0; i < 6; ++i) any_null = any_null || !nets[i] || !adam[i];
+    if (any_null || n < 1 || cfg->base.batch_size < 1) { le_set_error("le_td3_learn: bad arguments"); return LE_EINVAL; }
+    const int rc = td3_learn_check(cfg, "le_td3_learn");
+    if (rc != LE_OK) return rc;
+    return td3_learn(cfg, nets, adam, counters_dev, n, rows_dev, policy_noise_dev, expo_target_dev, expo_actor_dev, critic_loss_dev,
+                     (cudaStream_t)stream);
 }
 
 // workspace layout of the TD3 entry points: [SE pack | lane queue counter | resident lane slots]

@@ -6,7 +6,8 @@
 //   select_train_action / select_test_action (:155-166): actor -> * max_action -> F.gumbel_softmax(tau, hard) + N(0,1)*action_std,
 //       the environment receives argmax (agents/base_agent.py:111-114), the replay ring the action VECTOR;
 //   learn (:62-119): target policy smoothing, twin target critics (min), two Adam optimizers, delayed policy update through
-//       critic_1 with the straight-through Gumbel-softmax gradient, Polyak on the three targets.
+//       critic_1 with the straight-through Gumbel-softmax gradient, Polyak on the three targets — td3_learn_step, which
+//       td3_learn_kernel (le_td3_learn: explicit minibatches and draws) runs as well.
 // Every lane copies its own le_td3_cfg into shared memory and builds its actor / critic GNets there (vary_hp: per-lane
 // q_hidden, q_layers, batch_size, lr, ...); the slot workspace is sized for the maxima configuration of the launch.
 // Random draws: Philox streams P_TD3_EXPO / P_TD3_NORMAL (documented with the CPU restatement's stream table) and P_TD3_INIT
@@ -102,6 +103,139 @@ struct TRunParams {
     int init_stride_a, init_stride_c;
     float* actor_final; int final_stride;
 };
+
+// self.gumbel_temp_annealed of the learn() call that starts at self.total_it = total_it: np.linspace(T0, T0/20, 2000)[total_it],
+// clamped at the last entry
+__device__ __forceinline__ float td3_anneal_temp(double T0, int total_it) {
+    const double Tstep = (T0 / 20.0 - T0) / 1999.0;
+    return (float)(total_it >= 1999 ? T0 / 20.0 : (double)total_it * Tstep + T0);
+}
+
+// The three families of random draws of one learn() call, draw k of minibatch row b: the Exp(1) samples of the target
+// policy's gumbel_softmax, the randn_like policy noise, the Exp(1) samples of the actor's gumbel_softmax.
+// Lanes: the P_TD3_EXPO / P_TD3_NORMAL streams at phase 2 (target) / 3 (actor), counter learn_iters.
+template <int AD>
+struct Td3PhiloxDraws {
+    uint32_t k0, k1, c0;
+    __device__ __forceinline__ float expo_target(int b, int k) const { return td3_expo(k0, k1, 2u, c0, 0u, b * AD + k); }
+    __device__ __forceinline__ float policy_noise(int b, int k) const { return td3_normal(k0, k1, 2u, c0, 0u, b * AD + k); }
+    __device__ __forceinline__ float expo_actor(int b, int k) const { return td3_expo(k0, k1, 3u, c0, 0u, b * AD + k); }
+};
+// td3_learn_kernel: caller-given [B][AD] arrays
+template <int AD>
+struct Td3ArrayDraws {
+    const float *expo_t, *noise, *expo_a;
+    __device__ __forceinline__ float expo_target(int b, int k) const { return expo_t[b * AD + k]; }
+    __device__ __forceinline__ float policy_noise(int b, int k) const { return noise[b * AD + k]; }
+    __device__ __forceinline__ float expo_actor(int b, int k) const { return expo_a[b * AD + k]; }
+};
+
+// learn (agents/TD3_discrete_vary.py:62-119) after replay_buffer.sample, on the B rows staged in w.X ([s | action vector]),
+// w.S2 (s') and w.misc ([r, d, -, -]): target policy smoothing, twin target critics (min), the critic loss and the one Adam step
+// of both critics, the delayed policy update through critic_1 with the straight-through Gumbel-softmax gradient (when
+// total_it, self.total_it after its increment, is a multiple of policy_delay), Polyak on the three targets.  b1pow_* / b2pow_*: beta^t of the two optimizers, advanced here.  Returns the
+// critic loss.  The lane kernel and td3_learn_kernel both run this function.
+template <int SD, int AD, typename Draws>
+__device__ __forceinline__ float td3_learn_step(const GNet& na, const GNet& nc, const TSlot& w, const le_td3_cfg& tc, const LearnScalars& ls,
+                                                float temp, int total_it, const Draws& dr, double& b1pow_a, double& b2pow_a,
+                                                double& b1pow_c, double& b2pow_c, float* sm, float* red) {
+    constexpr int XI = SD + AD;
+    const int tid = threadIdx.x;
+    const int Sa = na.sum_out, Sc = nc.sum_out, yo_a = na.feat[na.nfeat - 1].y_off, yo_c = nc.feat[nc.nfeat - 1].y_off;
+    const float max_action = (float)tc.max_action, policy_std = (float)tc.policy_std, policy_clip = (float)tc.policy_std_clip;
+    const int hard = tc.gumbel_hard;
+    const int B = ls.batch;
+    // target policy smoothing: a' = gumbel_softmax(actor_target(s')) + clip(N * policy_std)
+    g_net_forward(na, w.actorT, w.S2, SD, B, w.Aa, sm);
+    for (int b = tid; b < B; b += kGThreads) {
+        float logits[AD], expo[AD], y[AD], ret[AD];
+#pragma unroll
+        for (int k = 0; k < AD; ++k) {
+            logits[k] = __ldcg(w.Aa + (int64_t)b * Sa + yo_a + k) * max_action;
+            expo[k] = dr.expo_target(b, k);
+        }
+        gumbel_softmax_row<AD>(logits, expo, temp, hard, y, ret);
+#pragma unroll
+        for (int i = 0; i < SD; ++i) w.X2[b * XI + i] = w.S2[b * SD + i];
+#pragma unroll
+        for (int k = 0; k < AD; ++k) {
+            float nz = dr.policy_noise(b, k) * policy_std;
+            nz = nz < -policy_clip ? -policy_clip : (nz > policy_clip ? policy_clip : nz);
+            w.X2[b * XI + SD + k] = ret[k] + nz;
+        }
+    }
+    __syncthreads();
+    // target_Q = r + (1 - d) * gamma * min(Q1', Q2')
+    g_net_forward(nc, w.c1T, w.X2, XI, B, w.A1, sm);
+    for (int b = tid; b < B; b += kGThreads) w.misc[4 * b + 2] = __ldcg(w.A1 + (int64_t)b * Sc + yo_c);
+    __syncthreads();
+    g_net_forward(nc, w.c2T, w.X2, XI, B, w.A1, sm);
+    for (int b = tid; b < B; b += kGThreads) {
+        const float q1 = w.misc[4 * b + 2], q2 = __ldcg(w.A1 + (int64_t)b * Sc + yo_c);
+        w.misc[4 * b + 2] = w.misc[4 * b] + ((1.f - w.misc[4 * b + 1]) * ls.gamma) * fminf(q1, q2);
+    }
+    __syncthreads();
+    // critic loss and the two critic steps (one optimizer: shared step count)
+    b1pow_c *= ls.beta1; b2pow_c *= ls.beta2d;
+    float lsum = 0.f;
+    for (int which = 0; which < 2; ++which) {
+        float* cth = which ? w.c2 : w.c1;
+        g_net_forward(nc, cth, w.X, XI, B, w.A1, sm);
+        float lpart = 0.f;
+        for (int b = tid; b < B; b += kGThreads) {
+            const float e = __ldcg(w.A1 + (int64_t)b * Sc + yo_c) - w.misc[4 * b + 2];
+            lpart = fmaf(e, e, lpart);
+            __stcg(w.D + (int64_t)b * Sc + yo_c, ls.norm * e);
+        }
+        lsum += g_block_sum(lpart, red) / (float)B;
+        __syncthreads();
+        t_net_backward(nc, cth, w.g_c, w.X, XI, w.A1, w.D, B, nullptr, 0, sm);
+        g_adam(cth, nullptr, which ? w.m_c2 : w.m_c1, which ? w.v_c2 : w.v_c1, w.g_c, nc.P, ls, b1pow_c, b2pow_c);
+    }
+    if (total_it % tc.policy_delay == 0) {
+        // actor loss = -mean(critic_1(s, actor(s))) through the (updated) critic and the straight-through Gumbel-softmax
+        g_net_forward(na, w.actor, w.X, XI, B, w.Aa, sm);
+        for (int b = tid; b < B; b += kGThreads) {
+            float logits[AD], expo[AD], y[AD], ret[AD];
+#pragma unroll
+            for (int k = 0; k < AD; ++k) {
+                logits[k] = __ldcg(w.Aa + (int64_t)b * Sa + yo_a + k) * max_action;
+                expo[k] = dr.expo_actor(b, k);
+            }
+            gumbel_softmax_row<AD>(logits, expo, temp, hard, y, ret);
+#pragma unroll
+            for (int i = 0; i < SD; ++i) w.Xpi[b * XI + i] = w.X[b * XI + i];
+#pragma unroll
+            for (int k = 0; k < AD; ++k) { w.Xpi[b * XI + SD + k] = ret[k]; w.Y[4 * b + k] = y[k]; }
+        }
+        __syncthreads();
+        g_net_forward(nc, w.c1, w.Xpi, XI, B, w.A1, sm);
+        for (int b = tid; b < B; b += kGThreads) __stcg(w.D + (int64_t)b * Sc + yo_c, -1.f / (float)B);
+        __syncthreads();
+        t_net_backward(nc, w.c1, w.g_c, w.Xpi, XI, w.A1, w.D, B, w.DX, XI, sm);     // only dL/d(action) is used
+        for (int b = tid; b < B; b += kGThreads) {
+            float dot = 0.f;
+#pragma unroll
+            for (int k = 0; k < AD; ++k) dot += w.Y[4 * b + k] * __ldcg(w.DX + (int64_t)b * XI + SD + k);
+#pragma unroll
+            for (int k = 0; k < AD; ++k)
+                __stcg(w.D + (int64_t)b * Sa + yo_a + k,
+                       __fdiv_rn(w.Y[4 * b + k] * (__ldcg(w.DX + (int64_t)b * XI + SD + k) - dot), temp) * max_action);
+        }
+        __syncthreads();
+        t_net_backward(na, w.actor, w.g_a, w.X, XI, w.Aa, w.D, B, nullptr, 0, sm);
+        b1pow_a *= ls.beta1; b2pow_a *= ls.beta2d;
+        g_adam(w.actor, nullptr, w.m_a, w.v_a, w.g_a, na.P, ls, b1pow_a, b2pow_a);
+        // Polyak on the three targets, after all three updates
+        for (int p = tid; p < nc.P; p += kGThreads) {
+            __stcg(w.c1T + p, ls.tau * __ldcg(w.c1 + p) + ls.one_minus_tau * __ldcg(w.c1T + p));
+            __stcg(w.c2T + p, ls.tau * __ldcg(w.c2 + p) + ls.one_minus_tau * __ldcg(w.c2T + p));
+        }
+        for (int p = tid; p < na.P; p += kGThreads) __stcg(w.actorT + p, ls.tau * __ldcg(w.actor + p) + ls.one_minus_tau * __ldcg(w.actorT + p));
+        __syncthreads();
+    }
+    return lsum;
+}
 
 __host__ __device__ inline int64_t tslot_floats(const GNet& na, const GNet& nc, int sd, int ad, int ring_cap, int rowf, int bmax, int64_t* offs /* [26] */) {
     const int Pa = (na.P + 3) / 4 * 4, Pc = (nc.P + 3) / 4 * 4, XI = sd + ad;
@@ -261,15 +395,11 @@ struct Td3Agent {
         }
     }
 
-    // learn (:62-119)
+    // learn (:62-119): replay_buffer.sample, then the step shared with td3_learn_kernel
     __device__ __forceinline__ float learn(int64_t learn_iters, int rb_size) {
         const int tid = threadIdx.x;
-        const int Sa = na.sum_out, Sc = nc.sum_out, yo_a = na.feat[na.nfeat - 1].y_off, yo_c = nc.feat[nc.nfeat - 1].y_off;
-        const float max_action = (float)tc.max_action, policy_std = (float)tc.policy_std, policy_clip = (float)tc.policy_std_clip;
-        const int hard = tc.gumbel_hard;
-        const double T0 = tc.gumbel_temp, Tstep = (T0 / 20.0 - T0) / 1999.0;      // np.linspace(T0, T0/20, 2000)
         __syncthreads();
-        temp = (float)(total_it >= 1999 ? T0 / 20.0 : (double)total_it * Tstep + T0);
+        temp = td3_anneal_temp(tc.gumbel_temp, total_it);
         total_it += 1;
         const int B = ls.batch;
         for (int b = tid; b < B; b += kGThreads) {     // replay_buffer.sample on the P_SAMPLE stream
@@ -283,96 +413,8 @@ struct Td3Agent {
             w.misc[4 * b + 1] = __ldcg(src + 2 * SD + AD + 1);
         }
         __syncthreads();
-        // target policy smoothing: a' = gumbel_softmax(actor_target(s')) + clip(N * policy_std)
-        g_net_forward(na, w.actorT, w.S2, SD, B, w.Aa, sm);
-        for (int b = tid; b < B; b += kGThreads) {
-            float logits[AD], expo[AD], y[AD], ret[AD];
-#pragma unroll
-            for (int k = 0; k < AD; ++k) {
-                logits[k] = __ldcg(w.Aa + (int64_t)b * Sa + yo_a + k) * max_action;
-                expo[k] = td3_expo(k0, k1, 2u, (uint32_t)learn_iters, 0u, b * AD + k);
-            }
-            gumbel_softmax_row<AD>(logits, expo, temp, hard, y, ret);
-#pragma unroll
-            for (int i = 0; i < SD; ++i) w.X2[b * XI + i] = w.S2[b * SD + i];
-#pragma unroll
-            for (int k = 0; k < AD; ++k) {
-                float nz = td3_normal(k0, k1, 2u, (uint32_t)learn_iters, 0u, b * AD + k) * policy_std;
-                nz = nz < -policy_clip ? -policy_clip : (nz > policy_clip ? policy_clip : nz);
-                w.X2[b * XI + SD + k] = ret[k] + nz;
-            }
-        }
-        __syncthreads();
-        // target_Q = r + (1 - d) * gamma * min(Q1', Q2')
-        g_net_forward(nc, w.c1T, w.X2, XI, B, w.A1, sm);
-        for (int b = tid; b < B; b += kGThreads) w.misc[4 * b + 2] = __ldcg(w.A1 + (int64_t)b * Sc + yo_c);
-        __syncthreads();
-        g_net_forward(nc, w.c2T, w.X2, XI, B, w.A1, sm);
-        for (int b = tid; b < B; b += kGThreads) {
-            const float q1 = w.misc[4 * b + 2], q2 = __ldcg(w.A1 + (int64_t)b * Sc + yo_c);
-            w.misc[4 * b + 2] = w.misc[4 * b] + ((1.f - w.misc[4 * b + 1]) * ls.gamma) * fminf(q1, q2);
-        }
-        __syncthreads();
-        // critic loss and the two critic steps (one optimizer: shared step count)
-        b1pow_c *= ls.beta1; b2pow_c *= ls.beta2d;
-        float lsum = 0.f;
-        for (int which = 0; which < 2; ++which) {
-            float* cth = which ? w.c2 : w.c1;
-            g_net_forward(nc, cth, w.X, XI, B, w.A1, sm);
-            float lpart = 0.f;
-            for (int b = tid; b < B; b += kGThreads) {
-                const float e = __ldcg(w.A1 + (int64_t)b * Sc + yo_c) - w.misc[4 * b + 2];
-                lpart = fmaf(e, e, lpart);
-                __stcg(w.D + (int64_t)b * Sc + yo_c, ls.norm * e);
-            }
-            lsum += g_block_sum(lpart, red) / (float)B;
-            __syncthreads();
-            t_net_backward(nc, cth, w.g_c, w.X, XI, w.A1, w.D, B, nullptr, 0, sm);
-            g_adam(cth, nullptr, which ? w.m_c2 : w.m_c1, which ? w.v_c2 : w.v_c1, w.g_c, nc.P, ls, b1pow_c, b2pow_c);
-        }
-        if (total_it % tc.policy_delay == 0) {
-            // actor loss = -mean(critic_1(s, actor(s))) through the (updated) critic and the straight-through Gumbel-softmax
-            g_net_forward(na, w.actor, w.X, XI, B, w.Aa, sm);
-            for (int b = tid; b < B; b += kGThreads) {
-                float logits[AD], expo[AD], y[AD], ret[AD];
-#pragma unroll
-                for (int k = 0; k < AD; ++k) {
-                    logits[k] = __ldcg(w.Aa + (int64_t)b * Sa + yo_a + k) * max_action;
-                    expo[k] = td3_expo(k0, k1, 3u, (uint32_t)learn_iters, 0u, b * AD + k);
-                }
-                gumbel_softmax_row<AD>(logits, expo, temp, hard, y, ret);
-#pragma unroll
-                for (int i = 0; i < SD; ++i) w.Xpi[b * XI + i] = w.X[b * XI + i];
-#pragma unroll
-                for (int k = 0; k < AD; ++k) { w.Xpi[b * XI + SD + k] = ret[k]; w.Y[4 * b + k] = y[k]; }
-            }
-            __syncthreads();
-            g_net_forward(nc, w.c1, w.Xpi, XI, B, w.A1, sm);
-            for (int b = tid; b < B; b += kGThreads) __stcg(w.D + (int64_t)b * Sc + yo_c, -1.f / (float)B);
-            __syncthreads();
-            t_net_backward(nc, w.c1, w.g_c, w.Xpi, XI, w.A1, w.D, B, w.DX, XI, sm);     // only dL/d(action) is used
-            for (int b = tid; b < B; b += kGThreads) {
-                float dot = 0.f;
-#pragma unroll
-                for (int k = 0; k < AD; ++k) dot += w.Y[4 * b + k] * __ldcg(w.DX + (int64_t)b * XI + SD + k);
-#pragma unroll
-                for (int k = 0; k < AD; ++k)
-                    __stcg(w.D + (int64_t)b * Sa + yo_a + k,
-                           __fdiv_rn(w.Y[4 * b + k] * (__ldcg(w.DX + (int64_t)b * XI + SD + k) - dot), temp) * max_action);
-            }
-            __syncthreads();
-            t_net_backward(na, w.actor, w.g_a, w.X, XI, w.Aa, w.D, B, nullptr, 0, sm);
-            b1pow_a *= ls.beta1; b2pow_a *= ls.beta2d;
-            g_adam(w.actor, nullptr, w.m_a, w.v_a, w.g_a, na.P, ls, b1pow_a, b2pow_a);
-            // Polyak on the three targets, after all three updates
-            for (int p = tid; p < nc.P; p += kGThreads) {
-                __stcg(w.c1T + p, ls.tau * __ldcg(w.c1 + p) + ls.one_minus_tau * __ldcg(w.c1T + p));
-                __stcg(w.c2T + p, ls.tau * __ldcg(w.c2 + p) + ls.one_minus_tau * __ldcg(w.c2T + p));
-            }
-            for (int p = tid; p < na.P; p += kGThreads) __stcg(w.actorT + p, ls.tau * __ldcg(w.actor + p) + ls.one_minus_tau * __ldcg(w.actorT + p));
-            __syncthreads();
-        }
-        return lsum;
+        const Td3PhiloxDraws<AD> dr{k0, k1, (uint32_t)learn_iters};
+        return td3_learn_step<SD, AD>(na, nc, w, tc, ls, temp, total_it, dr, b1pow_a, b2pow_a, b1pow_c, b2pow_c, sm, red);
     }
 
     __device__ __forceinline__ float* test_obs() { return w.obs; }
@@ -398,6 +440,60 @@ __global__ void __launch_bounds__(kGThreads, 2) td3_loop_kernel(const TRunParams
     Td3Agent<SD, AD> ag{G, tslot_view(G.slots + (int64_t)blockIdx.x * G.slot_stride, G.na_max, G.nc_max, SD, AD, G.rp.ring_cap, G.rowf, G.bmax),
                         cfg_sm, na_sm, nc_sm, sm, red};
     cta_lane_loop<SD, AD>(G.rp, ag);
+}
+
+// le_td3_learn: one learn() call per CTA on caller-owned nets / Adam state (row blockIdx.x of each [n][P] array), explicit
+// minibatch rows and draws; the activations live in the CTA's scratch slot (tslot_floats with no ring)
+struct Td3LearnParams {
+    le_td3_cfg tc;
+    GNet na, nc;
+    float *actor, *actorT, *c1, *c1T, *c2, *c2T, *m_a, *v_a, *m_c1, *v_c1, *m_c2, *v_c2;
+    int32_t* counters;                                   // [n][3]: actor Adam steps, critic Adam steps, total_it
+    const float *rows, *policy_noise, *expo_target, *expo_actor;
+    float* loss;
+    float* scratch; int64_t scratch_stride;
+};
+
+template <int SD, int AD>
+__global__ void __launch_bounds__(kGThreads, 2) td3_learn_kernel(const Td3LearnParams Q) {
+    static_assert(AD <= 4, "action vectors are handled as register arrays");
+    __shared__ __align__(16) float sm[kGSmemFloats];
+    __shared__ float red[32];
+    constexpr int XI = SD + AD, ROW = 2 * SD + AD + 2;
+    const int id = blockIdx.x, tid = threadIdx.x;
+    const le_lane_cfg& c = Q.tc.base;
+    const int B = c.batch_size;
+    const int64_t pa = (int64_t)id * Q.na.P, pc = (int64_t)id * Q.nc.P;
+    TSlot w = tslot_view(Q.scratch + (int64_t)id * Q.scratch_stride, Q.na, Q.nc, SD, AD, 0, 0, B);
+    w.actor = Q.actor + pa; w.actorT = Q.actorT + pa; w.m_a = Q.m_a + pa; w.v_a = Q.v_a + pa;
+    w.c1 = Q.c1 + pc; w.c1T = Q.c1T + pc; w.m_c1 = Q.m_c1 + pc; w.v_c1 = Q.v_c1 + pc;
+    w.c2 = Q.c2 + pc; w.c2T = Q.c2T + pc; w.m_c2 = Q.m_c2 + pc; w.v_c2 = Q.v_c2 + pc;
+    const float* my_rows = Q.rows + (int64_t)id * B * ROW;
+    for (int b = tid; b < B; b += kGThreads) {      // the staging of the lane's replay_buffer.sample
+        const float* src = my_rows + (int64_t)b * ROW;
+#pragma unroll
+        for (int i = 0; i < XI; ++i) w.X[b * XI + i] = src[i];
+#pragma unroll
+        for (int i = 0; i < SD; ++i) w.S2[b * SD + i] = src[XI + i];
+        w.misc[4 * b] = src[2 * SD + AD];
+        w.misc[4 * b + 1] = src[2 * SD + AD + 1];
+    }
+    __syncthreads();
+    LearnScalars ls;
+    fill_learn_scalars(ls, c);
+    int32_t* cnt = Q.counters + 3 * id;
+    const int t_a = cnt[0], t_c = cnt[1], it = cnt[2];
+    double b1pow_a = pow(c.beta1, (double)t_a), b2pow_a = pow(c.beta2, (double)t_a);
+    double b1pow_c = pow(c.beta1, (double)t_c), b2pow_c = pow(c.beta2, (double)t_c);
+    const float temp = td3_anneal_temp(Q.tc.gumbel_temp, it);
+    const bool update_policy = (it + 1) % Q.tc.policy_delay == 0;
+    const int64_t dro = (int64_t)id * B * AD;
+    const Td3ArrayDraws<AD> dr{Q.expo_target + dro, Q.policy_noise + dro, Q.expo_actor + dro};
+    const float loss = td3_learn_step<SD, AD>(Q.na, Q.nc, w, Q.tc, ls, temp, it + 1, dr, b1pow_a, b2pow_a, b1pow_c, b2pow_c, sm, red);
+    if (tid == 0) {
+        Q.loss[id] = loss;
+        cnt[0] = t_a + (update_policy ? 1 : 0); cnt[1] = t_c + 1; cnt[2] = it + 1;
+    }
 }
 
 // ---- host side ---------------------------------------------------------------------------------------------------
@@ -436,6 +532,27 @@ cudaError_t td3_launch(const le_td3_cfg* cfg_dev, int n_cfg, const le_td3_cfg* c
     if (c->sd == 4) td3_loop_kernel<4, 2><<<tp.grid, kGThreads, 0, st>>>(G);
     else td3_loop_kernel<6, 3><<<tp.grid, kGThreads, 0, st>>>(G);
     return cudaGetLastError();
+}
+
+int td3_learn(const le_td3_cfg* tc, float* const nets[6], float* const adam[6], int32_t* counters, int n, const float* rows,
+              const float* policy_noise, const float* expo_target, const float* expo_actor, float* loss, cudaStream_t st) {
+    Td3LearnParams Q;
+    Q.tc = *tc;
+    const le_lane_cfg* c = &tc->base;
+    tnet_build(&Q.na, c->sd, c->q_hidden, c->q_layers, c->ad, c->q_act);
+    tnet_build(&Q.nc, c->sd + c->ad, c->q_hidden, c->q_layers, 1, c->q_act);
+    Q.actor = nets[0]; Q.actorT = nets[1]; Q.c1 = nets[2]; Q.c1T = nets[3]; Q.c2 = nets[4]; Q.c2T = nets[5];
+    Q.m_a = adam[0]; Q.v_a = adam[1]; Q.m_c1 = adam[2]; Q.v_c1 = adam[3]; Q.m_c2 = adam[4]; Q.v_c2 = adam[5];
+    Q.counters = counters; Q.rows = rows; Q.policy_noise = policy_noise; Q.expo_target = expo_target; Q.expo_actor = expo_actor;
+    Q.loss = loss;
+    int64_t offs[26];
+    Q.scratch_stride = tslot_floats(Q.na, Q.nc, c->sd, c->ad, 0, 0, c->batch_size, offs);
+    LE_CUDA_CHECK(cudaMallocAsync((void**)&Q.scratch, (size_t)Q.scratch_stride * 4 * n, st));
+    if (c->sd == 4) td3_learn_kernel<4, 2><<<n, kGThreads, 0, st>>>(Q);
+    else td3_learn_kernel<6, 3><<<n, kGThreads, 0, st>>>(Q);
+    LE_CUDA_CHECK(cudaGetLastError());
+    LE_CUDA_CHECK(cudaFreeAsync(Q.scratch, st));
+    return LE_OK;
 }
 
 }  // namespace le

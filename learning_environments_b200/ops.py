@@ -310,6 +310,34 @@ def td3_param_counts(tcfg):
     return a.value, c.value
 
 
+TD3_NETS = ("actor", "actor_target", "critic_1", "critic_target_1", "critic_2", "critic_target_2")
+TD3_ADAM = ("m_a", "v_a", "m_c1", "v_c1", "m_c2", "v_c2")
+
+
+def td3_learn(tcfg, nets, adam, counters, rows, policy_noise, expo_target, expo_actor):
+    """TD3_discrete_vary.learn (agents/TD3_discrete_vary.py:62-119) in place for n lanes of one Td3Cfg (le_td3_learn), on the
+    current stream.  nets: dict TD3_NETS -> CUDA f32 [n, P_actor] / [n, P_critic]; adam: dict TD3_ADAM -> the Adam moments of the
+    same shapes; counters [n, 3] int32 (actor Adam steps, critic Adam steps, total_it before the call; advanced);
+    rows [n, B, 2*sd+ad+2] = [s | action vector | s' | r | d]; policy_noise, expo_target, expo_actor [n, B, ad].
+    Returns the critic loss [n]."""
+    b = tcfg.base
+    n, B = rows.shape[0], b.batch_size
+    assert rows.shape == (n, B, 2 * b.sd + b.ad + 2) and counters.shape == (n, 3)
+    for d in (policy_noise, expo_target, expo_actor):
+        assert d.shape == (n, B, b.ad)
+    pa, pc = td3_param_counts(tcfg)
+    for k in TD3_NETS:
+        assert nets[k].shape == (n, pa if k.startswith("actor") else pc), k
+    for k in TD3_ADAM:
+        assert adam[k].shape == (n, pa if k.endswith("_a") else pc), k
+    loss = torch.empty(n, dtype=_F32, device=rows.device)
+    with _on(rows) as stream:
+        check(_lib().le_td3_learn(C.byref(tcfg), *[_ptr(_dev(nets[k], _F32)) for k in TD3_NETS], *[_ptr(_dev(adam[k], _F32)) for k in TD3_ADAM],
+                                  _ptr(_dev(counters, _I32)), n, _ptr(_dev(rows, _F32)), _ptr(_dev(policy_noise, _F32)),
+                                  _ptr(_dev(expo_target, _F32)), _ptr(_dev(expo_actor, _F32)), _ptr(loss), stream), "le_td3_learn")
+    return loss
+
+
 class Td3Buffers(object):
     """Device buffers of one le_td3_run call, sized for `tcfg0` (the maxima configuration of the launch); the counterpart of
     InnerLoopBuffers for TD3_discrete_vary lanes."""

@@ -80,3 +80,39 @@ def test_td3_entry_rejects_bad_arguments_without_gpu():
     p = lambda a: a.ctypes.data_as(C.c_void_p)
     rc = lib.le_td3_run_host(C.byref(t), p(buf), 1, None, p(keys), p(buf), p(buf), p(buf), 1, None, 1, p(buf), p(buf), p(buf), p(buf), None, 0, 0)
     assert rc == -3 and b"reward-network" in lib.le_last_error()
+
+
+def test_td3_learn_rejects_bad_arguments_without_gpu():
+    """le_td3_learn: LE_EINVAL (-1) for NULL pointers, n < 1 and batch_size < 1; LE_EUNSUPPORTED (-3) for configurations outside the
+    compiled set — every check runs before any CUDA call.  The environment fields are not checked: a learn step has none."""
+    import numpy as np
+    lib = _abi.load_library()
+    buf = np.zeros(64, np.float32)
+    p = buf.ctypes.data
+
+    def good():
+        t = _abi.Td3Cfg()
+        t.base.sd, t.base.ad, t.base.q_hidden, t.base.q_layers, t.base.batch_size = 4, 2, 8, 2, 4
+        t.base.env_kind, t.base.rn_type, t.base.test_episodes = 1, 3, 0          # would be rejected by the lane entry points
+        t.policy_delay, t.gumbel_temp = 2, 1.0
+        return t
+
+    def call(t, n=1, null_at=None):
+        ptrs = [p] * 18
+        if null_at is not None:
+            ptrs[null_at] = None
+        return lib.le_td3_learn(C.byref(t) if t is not None else None, *ptrs[:13], n, *ptrs[13:], None)
+
+    assert call(None) == -1
+    for i in range(18):
+        assert call(good(), null_at=i) == -1, "NULL argument %d accepted" % i
+        assert b"bad arguments" in lib.le_last_error()
+    assert call(good(), n=0) == -1
+    t = good()
+    t.base.batch_size = 0
+    assert call(t) == -1
+    for field, value in [("ad", 5), ("q_layers", 4), ("policy_delay", 0), ("gumbel_temp", 0.0), ("gumbel_temp", float("nan")),
+                         ("q_act", 9), ("sd", 5), ("q_hidden", 0)]:
+        t = good()
+        setattr(t if field in ("policy_delay", "gumbel_temp") else t.base, field, value)
+        assert call(t) == -3, (field, value)

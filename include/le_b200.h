@@ -179,15 +179,22 @@ int le_tc_gemm(const float* A_dev, int a_si, int a_sl, const float* B_dev, int b
 /* ------------------------------------------------------------------------------------------------ */
 /* the fused hot path                                                                               */
 
-/* Bytes of device workspace needed for n lanes sharing n_env environment parameter vectors: the packed
- * SE/RN weights, one replay ring per RESIDENT warp slot (not per lane) and the lane queue counter.
+/* The device workspace of the lane entry points (le_inner_loop_run, le_td3_run) has one layout for every lane family,
+ * each region 256-byte aligned:
+ *     [packed SE/RN weights of the n_env env parameter vectors | lane queue counter (256 B) | one slot per RESIDENT lane slot]
+ * Slots are per resident slot, not per lane: the lanes beyond them queue.  A slot is the replay ring of a warp-per-lane
+ * (multi-warp, cluster) lane, or everything a CTA-per-lane lane keeps in HBM: replay ring, nets, Adam state, minibatch
+ * activations.  With the slots last, a shorter workspace only loses slots at its end. */
+
+/* Bytes of device workspace needed for n lanes sharing n_env environment parameter vectors.
  * Returns a negative LE_E* code on error. */
 int64_t le_inner_loop_workspace_bytes(const le_lane_cfg* cfg, int n_lanes, int n_env);
 
 /* The launch plan behind the two calls above/below (diagnostics for bench.py / DESIGN.md): CTAs, resident
- * warp slots, replay ring capacity in rows, hidden units per thread of the selected kernel set. */
+ * slots, replay ring capacity in rows, hidden units per thread of the selected register kernel set (0 for the
+ * CTA-per-lane general kernel). */
 int le_inner_loop_plan(const le_lane_cfg* cfg, int n_lanes, int n_env, int* grid, int* slots, int* ring_cap, int* units,
-                       int64_t* ring_offset_bytes /* offset of warp slot 0's replay ring inside the workspace */);
+                       int64_t* ring_offset_bytes /* offset of slot 0 (a register lane's replay ring) inside the workspace */);
 
 /*
  * Runs n_lanes complete `calc_score`s (agents/GTN_worker.py:187-221) — train() with ε-greedy acting
@@ -246,8 +253,8 @@ typedef struct le_td3_cfg {
  * Training env: LE_ENV_SE or LE_ENV_REAL.  trace_host (may be NULL): HOST arrays recording lane `trace_lane`.           */
 int le_td3_param_counts(const le_td3_cfg* cfg, int* p_actor, int* p_critic);
 
-/* Bytes of device workspace for le_td3_run: the packed SE weights, the lane queue counter and one slot (replay ring, the six
- * nets, Adam state, minibatch activations) per RESIDENT lane, every slot sized for cfg_host0 (the maxima of the launch).
+/* Bytes of device workspace for le_td3_run (layout above le_inner_loop_workspace_bytes), every slot sized for cfg_host0 (the
+ * maxima of the launch).
  * When the slots of all resident lanes do not fit 90 % of the free device memory, the size asks for fewer slots (at least
  * one); le_td3_run then keeps fewer lanes resident and queues the rest.  Returns a negative LE_E* code on error. */
 int64_t le_td3_workspace_bytes(const le_td3_cfg* cfg_host0, int n_lanes, int n_env);

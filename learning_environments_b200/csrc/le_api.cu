@@ -95,6 +95,34 @@ static int check_env_cfg(const le_lane_cfg* c) {
     return LE_OK;
 }
 
+// (sd, ad) of the two compiled environment shapes, CartPole (4, 2) and Acrobot (6, 3); check_env_cfg admits only these
+static bool env_shape_compiled(int sd, int ad) { return (sd == 4 && ad == 2) || (sd == 6 && ad == 3); }
+
+// the checks of the fields a learn() step reads (nets, minibatch, TD3 hyper-parameters); no CUDA call
+static int td3_learn_check(const le_td3_cfg* cfg, const char* who) {
+    const le_lane_cfg* c = &cfg->base;
+    if (qact_of(c) < 0 || c->q_hidden < 1 || c->q_layers > 3 || cfg->policy_delay < 1 || !(cfg->gumbel_temp > 0.0) || c->ad > 4 ||
+        c->batch_size < 1) {
+        le_set_error("%s: configuration outside the compiled kernel set", who);
+        return LE_EUNSUPPORTED;
+    }
+    if (!env_shape_compiled(c->sd, c->ad)) { le_set_error("no compiled kernel set for state_dim=%d action_dim=%d", c->sd, c->ad); return LE_EUNSUPPORTED; }
+    return LE_OK;
+}
+
+// the checks shared by the TD3 lane entry points, on the (maxima) configuration; no CUDA call
+static int td3_check(const le_td3_cfg* cfg, const char* who) {
+    const le_lane_cfg* c = &cfg->base;
+    int rc = check_env_cfg(c);
+    if (rc != LE_OK) return rc;
+    if (c->env_kind == LE_ENV_RN) { le_set_error("%s: reward-network training envs are not built for TD3 lanes", who); return LE_EUNSUPPORTED; }
+    if (c->train_episodes < 0 || c->test_episodes < 1 || c->max_steps < 1) {
+        le_set_error("%s: configuration outside the compiled kernel set", who);
+        return LE_EUNSUPPORTED;
+    }
+    return td3_learn_check(cfg, who);
+}
+
 // ---- NES kernels ------------------------------------------------------------------------------------
 // Box-Muller in fp64 on Philox word pairs (oracle/philox.py normals): normal p of member `member`.
 __device__ __forceinline__ void normals4(uint32_t blk, uint32_t member, uint32_t seed, uint32_t gen, float (&z)[4]) {
@@ -243,6 +271,81 @@ __global__ void real_env_step_kernel(int real_env, int max_steps, double* __rest
     done[i] = d;
 }
 
+// parameters of one SE / RN env network (envs/virtual_env.py, envs/reward_env.py); 0 for the real envs
+static int env_param_count(const le_lane_cfg* c) {
+    const int H = c->env_hidden;
+    if (c->env_kind == LE_ENV_SE) return 3 * H * (c->sd + c->ad + 1) + H * (c->sd + 2) + c->sd + 2;
+    if (c->env_kind == LE_ENV_RN) return H * (c->sd + 2) + 1;
+    return 0;
+}
+
+// ---- environment kernels: compiled once per environment shape, dispatched on sd ---------------------------------------
+
+// floats per env of the packed SE / RN layout the lane kernels read (real envs: one float4, never read)
+static int64_t env_pack_stride_f(const le_lane_cfg* c) {
+    const int H = c->env_hidden;
+    if (c->env_kind == LE_ENV_SE) return 4 * (c->sd == 4 ? SePack<4, 2>::pack_vec4(H) : SePack<6, 3>::pack_vec4(H));
+    if (c->env_kind == LE_ENV_RN) return 4 * (c->sd == 4 ? RnPack<4>::pack_vec4(H) : RnPack<6>::pack_vec4(H));
+    return 4;
+}
+
+static int64_t ring_row_floats(int sd) { return sd == 4 ? RowLayout<4>::ROWF : RowLayout<6>::ROWF; }
+
+template <int SD, int AD>
+static cudaError_t launch_pack_env(const le_lane_cfg* c, const float* theta, int n_env, float* pack, int64_t stride_f, cudaStream_t st) {
+    const int64_t total = stride_f * n_env;
+    const int grid = (int)((total + 255) / 256 < 4096 ? (total + 255) / 256 : 4096);
+    if (c->env_kind == LE_ENV_SE)
+        pack_se_kernel<SD, AD><<<grid, 256, 0, st>>>(theta, env_param_count(c), n_env, c->env_hidden, act_slope(c->env_act, c->env_slope[0]),
+                                                     act_slope(c->env_act, c->env_slope[1]), act_slope(c->env_act, c->env_slope[2]), pack,
+                                                     stride_f);
+    else
+        pack_rn_kernel<SD><<<grid, 256, 0, st>>>(theta, env_param_count(c), n_env, c->env_hidden, act_slope(c->env_act, c->env_slope[0]),
+                                                 pack, stride_f);
+    return cudaGetLastError();
+}
+
+// n_env SE / RN parameter vectors -> the packed layout (stride_f = env_pack_stride_f floats per env); real envs: nothing
+static cudaError_t pack_env(const le_lane_cfg* c, const float* theta, int n_env, float* pack, int64_t stride_f, cudaStream_t st) {
+    if (c->env_kind == LE_ENV_REAL) return cudaSuccess;
+    return c->sd == 4 ? launch_pack_env<4, 2>(c, theta, n_env, pack, stride_f, st) : launch_pack_env<6, 3>(c, theta, n_env, pack, stride_f, st);
+}
+
+// SE / RN unit operators (one warp per row), sharing the device code of the lane kernels
+template <int SD, int AD>
+__global__ void se_forward_kernel(const float4* __restrict__ pack, int64_t pack_stride, int H, int is_tanh, int lanes_per_member,
+                                  const float* __restrict__ state, const int32_t* __restrict__ action, float* __restrict__ ns_out,
+                                  float* __restrict__ reward, float* __restrict__ done, int n) {
+    const int lane = threadIdx.x & 31;
+    const int row = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+    if (row >= n) return;
+    float s[SD], ns[SD], r, d;
+#pragma unroll
+    for (int i = 0; i < SD; ++i) s[i] = state[(int64_t)row * SD + i];
+    se_step_row<SD, AD>(pack + (int64_t)(row / lanes_per_member) * pack_stride, H, is_tanh != 0, s, action[row], lane, ns, r, d);
+    if (lane == 0) {
+#pragma unroll
+        for (int i = 0; i < SD; ++i) ns_out[(int64_t)row * SD + i] = ns[i];
+        reward[row] = r;
+        done[row] = d;
+    }
+}
+
+template <int SD>
+__global__ void rn_reward_kernel(const float4* __restrict__ pack, int64_t pack_stride, int H, int is_tanh, int rn_type, float gamma,
+                                 int lanes_per_member, const float* __restrict__ s_in, const float* __restrict__ s2_in,
+                                 const float* __restrict__ rr, float* __restrict__ out, int n) {
+    const int lane = threadIdx.x & 31;
+    const int row = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+    if (row >= n) return;
+    float s[SD], s2[SD];
+#pragma unroll
+    for (int i = 0; i < SD; ++i) { s[i] = s_in[(int64_t)row * SD + i]; s2[i] = s2_in[(int64_t)row * SD + i]; }
+    float ps = 0.f, ps2 = 0.f;
+    if (rn_type != 0) rn_phi2<SD>(pack + (int64_t)(row / lanes_per_member) * pack_stride, H, is_tanh != 0, s, s2, lane, ps, ps2);
+    if (lane == 0) out[row] = rn_combine(rn_type, gamma, rr[row], ps, ps2);
+}
+
 // FP32 FFMA peak microbenchmark: the denominator of the fused kernel's roofline (MEASURED_PEAKS.json has no
 // FP32 figure).  8 independent FMA chains per thread, 256 threads x 8 CTAs per SM.
 __global__ void __launch_bounds__(256) ffma_peak_kernel(float* out, int iters, float a, float b) {
@@ -257,16 +360,6 @@ __global__ void __launch_bounds__(256) ffma_peak_kernel(float* out, int iters, f
     const float s = ((x0 + x1) + (x2 + x3)) + ((x4 + x5) + (x6 + x7));
     if (s == 123.456f) out[0] = s;
 }
-
-struct Plan {
-    bool general;
-    GeneralPlan gp;
-    const InstanceOps* ops;
-    int grid, slots, ring_cap;
-    bool mw;   // multi-warp lanes: one lane per CTA
-    bool mwc;  // cluster lanes: one lane per cluster of two CTAs (two SMs)
-    int64_t ring_stride_f, pack_stride_f, pack_bytes, rings_bytes, total_bytes, off_rings, off_counter;
-};
 
 // Multi-warp lanes (inner_loop_mw_kernel) for small populations: a lane gets a whole CTA instead of one warp (2.7x shorter
 // generations at the yaml's population of 16, profiles/r02_mw_lanes.txt); up to two lanes per SM queue on the CTAs before the
@@ -297,78 +390,117 @@ static int ring_capacity(const le_lane_cfg* c) {
     return (int)((int64_t)c->rb_size < max_total ? c->rb_size : max_total);
 }
 
-// parameters of one SE / RN env network (envs/virtual_env.py, envs/reward_env.py); 0 for the real envs
-static int env_param_count(const le_lane_cfg* c) {
-    const int H = c->env_hidden;
-    if (c->env_kind == LE_ENV_SE) return 3 * H * (c->sd + c->ad + 1) + H * (c->sd + 2) + c->sd + 2;
-    if (c->env_kind == LE_ENV_RN) return H * (c->sd + 2) + 1;
-    return 0;
-}
+static int64_t round256(int64_t bytes) { return (bytes + 255) / 256 * 256; }
 
-// n_env SE / RN parameter vectors -> the packed layout the lane kernels read (stride_f floats per env); real envs: nothing
-static cudaError_t pack_env(const InstanceOps* ops, const le_lane_cfg* c, const float* theta, int n_env, float* pack, int64_t stride_f,
-                            cudaStream_t st) {
-    if (c->env_kind == LE_ENV_SE) {
-        float slopes[3];
-        for (int i = 0; i < 3; ++i) slopes[i] = act_slope(c->env_act, c->env_slope[i]);
-        return ops->launch_pack_se(theta, env_param_count(c), n_env, c->env_hidden, slopes, pack, stride_f, st);
-    }
-    if (c->env_kind == LE_ENV_RN)
-        return ops->launch_pack_rn(theta, env_param_count(c), n_env, c->env_hidden, act_slope(c->env_act, c->env_slope[0]), pack, stride_f, st);
-    return cudaSuccess;
-}
+// The lane families: the warp-per-lane, multi-warp (one lane per CTA) and cluster (one lane per cluster of two CTAs) kernels of
+// a register Q-net kernel set, the CTA-per-lane general DDQN kernel and the TD3 kernel.
+enum class LaneFamily { Warp, MultiWarp, Cluster, General, Td3 };
 
-static int make_plan(const le_lane_cfg* c, int n_lanes, int n_env, Plan* pl) {
-    { const int rc0 = check_env_cfg(c); if (rc0 != LE_OK) return rc0; }
+// One launch of lanes.  Every family lays out its workspace the same way, each region 256-byte aligned:
+//   [env pack: max(n_env, 1) x pack_stride_f floats | lane queue counter: 256 B | slots: `slots` x slot_bytes]
+// A slot is the replay ring of a register lane, or everything a CTA-per-lane lane keeps in HBM (ring, nets, Adam state,
+// activations).  With the slots last, a shorter workspace only cuts slots off the end: le_td3_run keeps fewer lanes resident.
+struct LanePlan {
+    LaneFamily family;
+    const InstanceOps* ops;   // register kernel set of warp / multi-warp / cluster lanes, else null
+    GeneralPlan gp;           // general lanes
+    Td3Plan tp;               // TD3 lanes
+    int grid, slots, ring_cap;
+    int64_t pack_stride_f, slot_bytes, off_counter, off_slots, total_bytes;
+};
+
+// The configuration checks of the lane entry points, before any CUDA call.  c: the lane configuration that fixes the shapes
+// (cfg 0 / the maxima); td3: its TD3 configuration for TD3 lanes, else null.  Sets pl->family (Warp for every register kernel
+// set; plan_lanes picks among its kernels) and pl->ops.
+static int check_lanes(const le_lane_cfg* c, const le_td3_cfg* td3, int n_lanes, const char* who, LanePlan* pl) {
+    pl->ops = nullptr;
+    if (td3) { pl->family = LaneFamily::Td3; return td3_check(td3, who); }
+    const int rc = check_env_cfg(c);
+    if (rc != LE_OK) return rc;
     if (c->batch_size < 1 || c->rb_size < 1 || c->train_episodes < 0 || c->test_episodes < 1 || c->max_steps < 1 || n_lanes < 1) {
         le_set_error("bad lane configuration (batch_size=%d rb_size=%d train_episodes=%d test_episodes=%d max_steps=%d n_lanes=%d)",
                      c->batch_size, c->rb_size, c->train_episodes, c->test_episodes, c->max_steps, n_lanes);
         return LE_EINVAL;
     }
-    pl->general = !is_register_resident(c);
-    pl->mw = false;
-    pl->mwc = false;
     if (c->q_layers > 3) { le_set_error("Q-network hidden_layer=%d: the compiled kernel set covers up to 3 hidden layers", c->q_layers); return LE_EUNSUPPORTED; }
-    // the env-packing / unit kernels of any kernel set with the right (sd, ad) serve the general path too
-    const InstanceOps* ops = pl->general ? le_find_instance(c->sd, c->ad, 1, QACT_TANH) : instance_for(c, c->q_hidden);
-    if (!ops) { if (pl->general) le_set_error("no compiled kernel set for state_dim=%d action_dim=%d", c->sd, c->ad); return LE_EUNSUPPORTED; }
-    if (pl->general && qact_of(c) < 0) { le_set_error("Q-net activation id %d is outside the compiled kernel set", c->q_act); return LE_EUNSUPPORTED; }
+    if (is_register_resident(c)) {
+        pl->family = LaneFamily::Warp;
+        pl->ops = instance_for(c, c->q_hidden);
+        return pl->ops ? LE_OK : LE_EUNSUPPORTED;
+    }
+    pl->family = LaneFamily::General;
+    if (qact_of(c) < 0) { le_set_error("Q-net activation id %d is outside the compiled kernel set", c->q_act); return LE_EUNSUPPORTED; }
+    return LE_OK;
+}
+
+// Sizes lanes that passed check_lanes for the current device: family, grid, resident slots and the workspace layout.
+static int plan_lanes(const le_lane_cfg* c, const le_td3_cfg* td3, int n_lanes, int n_env, LanePlan* pl) {
     int dev = 0, sms = 0;
     LE_CUDA_CHECK(cudaGetDevice(&dev));
     LE_CUDA_CHECK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
     pl->ring_cap = ring_capacity(c);
-    pl->ops = ops;
-    if (pl->general) {
+    const InstanceOps* ops = pl->ops;
+    int64_t slot_floats = (int64_t)pl->ring_cap * ring_row_floats(c->sd);   // register lanes: one replay ring
+    if (pl->family == LaneFamily::Td3) {
+        const int rc = td3_plan(td3, n_lanes, pl->ring_cap, sms, &pl->tp);
+        if (rc != LE_OK) return rc;
+        pl->grid = pl->slots = pl->tp.grid;
+        slot_floats = pl->tp.slot_floats;
+    } else if (pl->family == LaneFamily::General) {
         const int rc = general_plan(c, n_lanes, pl->ring_cap, sms, &pl->gp);
         if (rc != LE_OK) return rc;
-        pl->grid = pl->gp.grid;
-        pl->slots = pl->grid;
-        pl->ring_stride_f = pl->gp.slot_floats;   // one slot = ring + parameters + activations
+        pl->grid = pl->slots = pl->gp.grid;
+        slot_floats = pl->gp.slot_floats;
     } else if (use_mwc_lanes(ops, n_lanes, sms)) {
-        pl->mw = true; pl->mwc = true;
+        pl->family = LaneFamily::Cluster;
         pl->grid = 2 * n_lanes;      // one cluster of two CTAs per lane
         pl->slots = n_lanes;
-        pl->ring_stride_f = (int64_t)pl->ring_cap * ops->ring_row_floats();
     } else if (use_mw_lanes(ops, n_lanes, sms)) {
-        pl->mw = true;
-        pl->grid = n_lanes < sms ? n_lanes : sms;
-        pl->slots = pl->grid;
-        pl->ring_stride_f = (int64_t)pl->ring_cap * ops->ring_row_floats();
+        pl->family = LaneFamily::MultiWarp;
+        pl->grid = pl->slots = n_lanes < sms ? n_lanes : sms;
     } else {
         int per_sm = ops->inner_max_ctas_per_sm();
         if (per_sm < 1) per_sm = 1;
         const int want = (n_lanes + ops->inner_warps - 1) / ops->inner_warps;
         pl->grid = want < sms * per_sm ? want : sms * per_sm;
         pl->slots = pl->grid * ops->inner_warps;
-        pl->ring_stride_f = (int64_t)pl->ring_cap * ops->ring_row_floats();
     }
-    const int64_t pv4 = c->env_kind == LE_ENV_SE ? ops->se_pack_vec4(c->env_hidden) : (c->env_kind == LE_ENV_RN ? ops->rn_pack_vec4(c->env_hidden) : 1);
-    pl->pack_stride_f = pv4 * 4;
-    pl->pack_bytes = ((int64_t)(n_env > 0 ? n_env : 1) * pl->pack_stride_f * 4 + 255) / 256 * 256;
-    pl->rings_bytes = ((int64_t)pl->slots * pl->ring_stride_f * 4 + 255) / 256 * 256;
-    pl->off_rings = pl->pack_bytes;
-    pl->off_counter = pl->off_rings + pl->rings_bytes;
-    pl->total_bytes = pl->off_counter + 256;
+    pl->pack_stride_f = env_pack_stride_f(c);
+    pl->slot_bytes = slot_floats * (int64_t)sizeof(float);
+    pl->off_counter = round256((int64_t)(n_env > 0 ? n_env : 1) * pl->pack_stride_f * 4);
+    pl->off_slots = pl->off_counter + 256;
+    // the TD3 size is td3_workspace_bytes: a slot region without padding, and possibly fewer slots
+    pl->total_bytes = pl->off_slots + round256((int64_t)pl->slots * pl->slot_bytes);
+    return LE_OK;
+}
+
+// le_td3_workspace_bytes of a planned TD3 launch.  A slot of the widest vary_hp shapes (hidden 1530 x 3 layers) is ~0.3 GB:
+// when every resident lane's slot does not fit 90 % of the free device memory, ask for fewer slots (the lane queue runs the
+// rest on them).
+static int64_t td3_workspace_bytes(const LanePlan& pl) {
+    size_t free_b = 0, total_b = 0;
+    LE_CUDA_CHECK(cudaMemGetInfo(&free_b, &total_b));
+    const int64_t room = (int64_t)(0.9 * (double)free_b) - pl.off_slots;
+    int64_t slots = pl.slots;
+    if (slots * pl.slot_bytes > room) slots = room / pl.slot_bytes > 1 ? room / pl.slot_bytes : 1;
+    return pl.off_slots + slots * pl.slot_bytes;
+}
+
+// Packs the env into the workspace, zeroes the lane queue counter and fills the RunParams fields every lane family reads;
+// the entry points add their own.
+static int start_lanes(const LanePlan& pl, const le_lane_cfg* c, const float* env_theta, int n_env, const int32_t* env_index,
+                       const uint32_t* keys, int n_lanes, le_lane_out* out, double* rewards, int32_t* lengths, double* test_rewards,
+                       char* ws, const le_trace* trace, int trace_lane, cudaStream_t st, RunParams* P) {
+    LE_CUDA_CHECK(pack_env(c, env_theta, n_env, (float*)ws, pl.pack_stride_f, st));
+    LE_CUDA_CHECK(cudaMemsetAsync(ws + pl.off_counter, 0, sizeof(int), st));
+    memset(P, 0, sizeof(*P));
+    P->env_pack = (const float4*)ws; P->env_pack_stride = pl.pack_stride_f / 4;
+    P->env_index = env_index; P->keys = keys;
+    P->n_lanes = n_lanes; P->out = out; P->rewards = rewards; P->lengths = lengths; P->test_rewards = test_rewards;
+    P->rew_stride = c->train_episodes > 0 ? c->train_episodes : 1; P->test_stride = c->test_episodes;
+    P->ring_cap = pl.ring_cap;
+    P->work_counter = (int*)(ws + pl.off_counter);
+    if (trace && trace->cap > 0) { P->trace = *trace; P->trace_lane = trace_lane; }
     return LE_OK;
 }
 
@@ -418,6 +550,48 @@ struct HostCall {
         return rc;
     }
 };
+
+// The segments both *_run_host entries stage: the lane configurations, env parameters, env index and keys in; per-lane results,
+// reward / length histories and test rewards out; and the arrays of an optional trace.
+struct LaneSegs { size_t cfg, th, ei, key, out, rw, ln, tr, trace[6]; int tcap; };
+
+static LaneSegs add_lane_segs(HostCall& hc, const void* cfgs, size_t cfg_bytes, const le_lane_cfg* c, const float* env_theta, int n_env,
+                              const int32_t* env_index, const uint32_t* keys, int n_lanes, le_lane_out* out, double* rewards,
+                              int32_t* lengths, double* test_rewards, const le_trace* trace) {
+    const int rs = c->train_episodes > 0 ? c->train_episodes : 1;
+    LaneSegs s;
+    s.cfg = hc.add(cfgs, nullptr, cfg_bytes);
+    s.th = hc.add(env_theta, nullptr, env_theta ? sizeof(float) * (size_t)env_param_count(c) * n_env : 0);
+    s.ei = hc.add(env_index, nullptr, env_index ? sizeof(int32_t) * n_lanes : 0);
+    s.key = hc.add(keys, nullptr, sizeof(uint32_t) * 2 * n_lanes);
+    s.out = hc.add(nullptr, out, sizeof(le_lane_out) * n_lanes);
+    s.rw = hc.add(nullptr, rewards, sizeof(double) * (size_t)rs * n_lanes);
+    s.ln = hc.add(nullptr, lengths, sizeof(int32_t) * (size_t)rs * n_lanes);
+    s.tr = hc.add(nullptr, test_rewards, sizeof(double) * (size_t)c->test_episodes * n_lanes);
+    s.tcap = trace && trace->cap > 0 ? trace->cap : 0;
+    if (s.tcap) {   // 4-byte entries, one per step (next_state, k = 2: sd per step)
+        void* const dst[6] = {trace->action, trace->explore, trace->next_state, trace->reward, trace->done, trace->loss};
+        for (int k = 0; k < 6; ++k) s.trace[k] = hc.add(nullptr, dst[k], 4 * (size_t)s.tcap * (k == 2 ? c->sd : 1));
+    }
+    return s;
+}
+
+// HostCall::stage_in, then zeroes the reward / length histories and marks the trace (untouched entries read -1 / NaN);
+// *tr: the trace with device pointers (cap 0 without one)
+static int stage_lane_segs(HostCall& hc, const LaneSegs& s, le_trace* tr) {
+    const int rc = hc.stage_in();
+    if (rc != LE_OK) return rc;
+    LE_CUDA_CHECK(cudaMemsetAsync(hc.dp(s.rw), 0, hc.segs[s.rw].bytes, hc.st));
+    LE_CUDA_CHECK(cudaMemsetAsync(hc.dp(s.ln), 0, hc.segs[s.ln].bytes, hc.st));
+    memset(tr, 0, sizeof(*tr));
+    if (s.tcap) {
+        for (int k = 0; k < 6; ++k) LE_CUDA_CHECK(cudaMemsetAsync(hc.dp(s.trace[k]), 0xff, hc.segs[s.trace[k]].bytes, hc.st));
+        tr->cap = s.tcap;
+        tr->action = (int32_t*)hc.dp(s.trace[0]); tr->explore = (int32_t*)hc.dp(s.trace[1]); tr->next_state = (float*)hc.dp(s.trace[2]);
+        tr->reward = (float*)hc.dp(s.trace[3]); tr->done = (float*)hc.dp(s.trace[4]); tr->loss = (float*)hc.dp(s.trace[5]);
+    }
+    return LE_OK;
+}
 
 extern "C" {
 
@@ -472,18 +646,21 @@ int le_se_forward(const le_lane_cfg* cfg, const float* theta_dev, int pop, int l
                   const int32_t* action_dev, float* next_state_dev, float* reward_dev, float* done_dev, void* stream) {
     if (!cfg || pop < 1 || lanes_per_member < 1) { le_set_error("le_se_forward: bad arguments"); return LE_EINVAL; }
     if (check_env_cfg(cfg) != LE_OK) return LE_EINVAL;
-    const InstanceOps* ops = le_find_instance(cfg->sd, cfg->ad, 1, QACT_TANH);
-    if (!ops) { le_set_error("no compiled kernel set for state_dim=%d action_dim=%d", cfg->sd, cfg->ad); return LE_EUNSUPPORTED; }
     cudaStream_t st = (cudaStream_t)stream;
     le_lane_cfg c = *cfg;
     c.env_kind = LE_ENV_SE;
-    const int H = c.env_hidden;
-    const int64_t stride_f = ops->se_pack_vec4(H) * 4;
+    const int H = c.env_hidden, n = pop * lanes_per_member, is_tanh = c.env_act == LE_ACT_TANH;
+    const int64_t stride_f = env_pack_stride_f(&c);
     float* pack = nullptr;
     LE_CUDA_CHECK(cudaMallocAsync((void**)&pack, (size_t)pop * stride_f * 4, st));
-    LE_CUDA_CHECK(pack_env(ops, &c, theta_dev, pop, pack, stride_f, st));
-    LE_CUDA_CHECK(ops->launch_se_forward((const float4*)pack, stride_f / 4, H, cfg->env_act == LE_ACT_TANH, lanes_per_member, state_dev,
-                                         action_dev, next_state_dev, reward_dev, done_dev, pop * lanes_per_member, st));
+    LE_CUDA_CHECK(pack_env(&c, theta_dev, pop, pack, stride_f, st));
+    if (c.sd == 4)
+        se_forward_kernel<4, 2><<<(n + 3) / 4, 128, 0, st>>>((const float4*)pack, stride_f / 4, H, is_tanh, lanes_per_member, state_dev,
+                                                             action_dev, next_state_dev, reward_dev, done_dev, n);
+    else
+        se_forward_kernel<6, 3><<<(n + 3) / 4, 128, 0, st>>>((const float4*)pack, stride_f / 4, H, is_tanh, lanes_per_member, state_dev,
+                                                             action_dev, next_state_dev, reward_dev, done_dev, n);
+    LE_CUDA_CHECK(cudaGetLastError());
     LE_CUDA_CHECK(cudaFreeAsync(pack, st));
     return LE_OK;
 }
@@ -495,16 +672,19 @@ int le_rn_reward(const le_lane_cfg* cfg, const float* theta_dev, int pop, int la
     c.env_kind = LE_ENV_RN;
     int rc = check_env_cfg(&c);
     if (rc != LE_OK) return rc;
-    const InstanceOps* ops = le_find_instance(c.sd, c.ad, 1, QACT_TANH);
-    if (!ops) { le_set_error("no compiled kernel set for state_dim=%d action_dim=%d", c.sd, c.ad); return LE_EUNSUPPORTED; }
     cudaStream_t st = (cudaStream_t)stream;
-    const int H = c.env_hidden;
-    const int64_t stride_f = ops->rn_pack_vec4(H) * 4;
+    const int H = c.env_hidden, n = pop * lanes_per_member, is_tanh = c.env_act == LE_ACT_TANH;
+    const int64_t stride_f = env_pack_stride_f(&c);
     float* pack = nullptr;
     LE_CUDA_CHECK(cudaMallocAsync((void**)&pack, (size_t)pop * stride_f * 4, st));
-    LE_CUDA_CHECK(pack_env(ops, &c, theta_dev, pop, pack, stride_f, st));
-    LE_CUDA_CHECK(ops->launch_rn_reward((const float4*)pack, stride_f / 4, H, c.env_act == LE_ACT_TANH, c.rn_type, (float)c.gamma,
-                                        lanes_per_member, state_dev, next_state_dev, real_reward_dev, reward_dev, pop * lanes_per_member, st));
+    LE_CUDA_CHECK(pack_env(&c, theta_dev, pop, pack, stride_f, st));
+    if (c.sd == 4)
+        rn_reward_kernel<4><<<(n + 3) / 4, 128, 0, st>>>((const float4*)pack, stride_f / 4, H, is_tanh, c.rn_type, (float)c.gamma,
+                                                         lanes_per_member, state_dev, next_state_dev, real_reward_dev, reward_dev, n);
+    else
+        rn_reward_kernel<6><<<(n + 3) / 4, 128, 0, st>>>((const float4*)pack, stride_f / 4, H, is_tanh, c.rn_type, (float)c.gamma,
+                                                         lanes_per_member, state_dev, next_state_dev, real_reward_dev, reward_dev, n);
+    LE_CUDA_CHECK(cudaGetLastError());
     LE_CUDA_CHECK(cudaFreeAsync(pack, st));
     return LE_OK;
 }
@@ -514,7 +694,7 @@ int le_qnet_forward(const le_lane_cfg* cfg, const float* q_theta_dev, int n, con
     if (!cfg || n < 1) { le_set_error("le_qnet_forward: bad arguments"); return LE_EINVAL; }
     if (cfg->q_layers > 3) { le_set_error("le_qnet_forward: hidden_layer > 3"); return LE_EUNSUPPORTED; }
     if (!is_register_resident(cfg)) {
-        if (qact_of(cfg) < 0 || !le_find_instance(cfg->sd, cfg->ad, 1, QACT_TANH)) { le_set_error("le_qnet_forward: unsupported Q-network"); return LE_EUNSUPPORTED; }
+        if (qact_of(cfg) < 0 || !env_shape_compiled(cfg->sd, cfg->ad)) { le_set_error("le_qnet_forward: unsupported Q-network"); return LE_EUNSUPPORTED; }
         return general_qnet_forward(cfg, q_theta_dev, n, state_dev, q_out_dev, argmax_dev, (cudaStream_t)stream);
     }
     const InstanceOps* ops = instance_for(cfg, cfg->q_hidden);
@@ -539,8 +719,9 @@ int le_td_update(const le_lane_cfg* cfg, float* q_theta_dev, float* q_target_dev
     if (!cfg || n < 1 || cfg->batch_size < 1) { le_set_error("le_td_update: bad arguments"); return LE_EINVAL; }
     if (cfg->q_layers > 3) { le_set_error("le_td_update: hidden_layer > 3"); return LE_EUNSUPPORTED; }
     const bool general = !is_register_resident(cfg);
-    const InstanceOps* ops = general ? le_find_instance(cfg->sd, cfg->ad, 1, QACT_TANH) : instance_for(cfg, cfg->q_hidden);
-    if (!ops || qact_of(cfg) < 0) { if (general) le_set_error("le_td_update: unsupported Q-network"); return LE_EUNSUPPORTED; }
+    const InstanceOps* ops = general ? nullptr : instance_for(cfg, cfg->q_hidden);
+    if (general && (qact_of(cfg) < 0 || !env_shape_compiled(cfg->sd, cfg->ad))) { le_set_error("le_td_update: unsupported Q-network"); return LE_EUNSUPPORTED; }
+    if (!general && !ops) return LE_EUNSUPPORTED;
     cudaStream_t st = (cudaStream_t)stream;
     le_lane_cfg* cfg_dev = nullptr;
     LE_CUDA_CHECK(cudaMallocAsync((void**)&cfg_dev, sizeof(le_lane_cfg), st));
@@ -559,11 +740,11 @@ int le_td_update(const le_lane_cfg* cfg, float* q_theta_dev, float* q_target_dev
 
 // ---- fused hot path -----------------------------------------------------------------------------------
 int64_t le_inner_loop_workspace_bytes(const le_lane_cfg* cfg, int n_lanes, int n_env) {
-    Plan pl;
     if (!cfg) { le_set_error("le_inner_loop_workspace_bytes: cfg is NULL"); return LE_EINVAL; }
-    int rc = make_plan(cfg, n_lanes, n_env, &pl);
-    if (rc != LE_OK) return rc;
-    return pl.total_bytes;
+    LanePlan pl;
+    int rc = check_lanes(cfg, nullptr, n_lanes, "le_inner_loop_workspace_bytes", &pl);
+    if (rc == LE_OK) rc = plan_lanes(cfg, nullptr, n_lanes, n_env, &pl);
+    return rc == LE_OK ? pl.total_bytes : rc;
 }
 
 int le_inner_loop_run(const le_lane_cfg* cfg_dev, int n_cfg, const le_lane_cfg* cfg_host0, const float* env_theta_dev, int n_env,
@@ -575,57 +756,52 @@ int le_inner_loop_run(const le_lane_cfg* cfg_dev, int n_cfg, const le_lane_cfg* 
         le_set_error("le_inner_loop_run: bad arguments (n_cfg must be 1 or n_lanes; no NULL outputs)");
         return LE_EINVAL;
     }
-    Plan pl;
-    int rc = make_plan(cfg_host0, n_lanes, n_env, &pl);
+    const le_lane_cfg* c = cfg_host0;
+    LanePlan pl;
+    int rc = check_lanes(c, nullptr, n_lanes, "le_inner_loop_run", &pl);
     if (rc != LE_OK) return rc;
-    if (cfg_host0->env_kind != LE_ENV_REAL && (!env_theta_dev || n_env < 1)) { le_set_error("le_inner_loop_run: env_theta is required for SE/RN lanes"); return LE_EINVAL; }
+    if (c->env_kind != LE_ENV_REAL && (!env_theta_dev || n_env < 1)) { le_set_error("le_inner_loop_run: env_theta is required for SE/RN lanes"); return LE_EINVAL; }
+    rc = plan_lanes(c, nullptr, n_lanes, n_env, &pl);
+    if (rc != LE_OK) return rc;
     if (workspace_bytes < pl.total_bytes) {
         le_set_error("le_inner_loop_run: workspace too small (%lld < %lld bytes)", (long long)workspace_bytes, (long long)pl.total_bytes);
         return LE_EINVAL;
     }
     cudaStream_t st = (cudaStream_t)stream;
     char* ws = (char*)workspace_dev;
-    float* pack = (float*)ws;
-    const le_lane_cfg* c = cfg_host0;
-    LE_CUDA_CHECK(pack_env(pl.ops, c, env_theta_dev, n_env, pack, pl.pack_stride_f, st));
-    int* counter = (int*)(ws + pl.off_counter);
-    LE_CUDA_CHECK(cudaMemsetAsync(counter, 0, sizeof(int), st));
     RunParams P;
-    memset(&P, 0, sizeof(P));
+    rc = start_lanes(pl, c, env_theta_dev, n_env, env_index_dev, keys_dev, n_lanes, out_dev, rewards_dev, lengths_dev, test_rewards_dev, ws,
+                     trace_host, trace_lane, st, &P);
+    if (rc != LE_OK) return rc;
     P.cfg = cfg_dev; P.n_cfg = n_cfg;
-    P.env_pack = (const float4*)pack; P.env_pack_stride = pl.pack_stride_f / 4;
-    P.env_index = env_index_dev; P.keys = keys_dev;
-    P.q_init = q_init_dev; P.q_final = q_final_dev;
-    P.q_stride = q_params_of(c);
-    P.n_lanes = n_lanes; P.out = out_dev; P.rewards = rewards_dev; P.lengths = lengths_dev; P.test_rewards = test_rewards_dev; P.test_lengths = test_lengths_dev;
-    P.rew_stride = c->train_episodes > 0 ? c->train_episodes : 1;
-    P.test_stride = c->test_episodes;
-    P.rings = (float*)(ws + pl.off_rings); P.ring_stride = pl.ring_stride_f; P.ring_cap = pl.ring_cap;
-    P.work_counter = counter;
-    if (trace_host && trace_host->cap > 0) { P.trace = *trace_host; P.trace_lane = trace_lane; }
-    if (pl.general) LE_CUDA_CHECK(general_launch(c, P, P.rings, pl.gp, st));
-    else if (pl.mw) {
+    P.q_init = q_init_dev; P.q_final = q_final_dev; P.q_stride = q_params_of(c);
+    P.test_lengths = test_lengths_dev;
+    P.rings = (float*)(ws + pl.off_slots); P.ring_stride = pl.slot_bytes / 4;
+    if (pl.family == LaneFamily::General) LE_CUDA_CHECK(general_launch(c, P, P.rings, pl.gp, st));
+    else if (pl.family == LaneFamily::Warp) LE_CUDA_CHECK(pl.ops->launch_inner(P, pl.grid, st));
+    else {
         // the member's SE / RN pack is staged in the CTA's shared memory by one TMA bulk copy per lane when it fits beside the lane state
+        const bool cluster = pl.family == LaneFamily::Cluster;
         const int64_t pack_bytes = c->env_kind == LE_ENV_REAL ? 0 : pl.pack_stride_f * 4;
-        const int64_t lane_smem = pl.mwc ? pl.ops->mwc_smem_bytes : pl.ops->mw_smem_bytes;
+        const int64_t lane_smem = cluster ? pl.ops->mwc_smem_bytes : pl.ops->mw_smem_bytes;
         if (pack_bytes > 0 && lane_smem + pack_bytes <= 227 * 1024) P.mw_pack_f4 = (int)(pack_bytes / 16);
-        if (pl.mwc) LE_CUDA_CHECK(pl.ops->launch_inner_mwc(P, pl.slots, st));
+        if (cluster) LE_CUDA_CHECK(pl.ops->launch_inner_mwc(P, pl.slots, st));
         else LE_CUDA_CHECK(pl.ops->launch_inner_mw(P, pl.grid, st));
     }
-    else LE_CUDA_CHECK(pl.ops->launch_inner(P, pl.grid, st));
     return LE_OK;
 }
 
 int le_inner_loop_plan(const le_lane_cfg* cfg, int n_lanes, int n_env, int* grid, int* slots, int* ring_cap, int* units,
                        int64_t* ring_offset_bytes) {
-    Plan pl;
-    int rc = make_plan(cfg, n_lanes, n_env, &pl);
+    LanePlan pl;
+    int rc = check_lanes(cfg, nullptr, n_lanes, "le_inner_loop_plan", &pl);
+    if (rc == LE_OK) rc = plan_lanes(cfg, nullptr, n_lanes, n_env, &pl);
     if (rc != LE_OK) return rc;
     if (grid) *grid = pl.grid;
     if (slots) *slots = pl.slots;
     if (ring_cap) *ring_cap = pl.ring_cap;
-    if (units) *units = pl.ops->units;
-    if (ring_offset_bytes) *ring_offset_bytes = pl.off_rings;
+    if (units) *units = pl.ops ? pl.ops->units : 0;
+    if (ring_offset_bytes) *ring_offset_bytes = pl.off_slots;
     return LE_OK;
 }
 
@@ -636,31 +812,26 @@ int le_inner_loop_run_host(const le_lane_cfg* cfgs, int n_cfg, const float* env_
         le_set_error("le_inner_loop_run_host: bad arguments");
         return LE_EINVAL;
     }
-    LE_CUDA_CHECK(cudaSetDevice(device));
     const le_lane_cfg* c = &cfgs[0];
-    Plan pl;
-    int rc = make_plan(c, n_lanes, n_env, &pl);
+    LanePlan pl;
+    int rc = check_lanes(c, nullptr, n_lanes, "le_inner_loop_run_host", &pl);
+    if (rc != LE_OK) return rc;
+    LE_CUDA_CHECK(cudaSetDevice(device));
+    rc = plan_lanes(c, nullptr, n_lanes, n_env, &pl);
     if (rc != LE_OK) return rc;
     const int Pq = q_params_of(c);
-    const int rs = c->train_episodes > 0 ? c->train_episodes : 1;
     HostCall hc;
-    const size_t i_cfg = hc.add(cfgs, nullptr, sizeof(le_lane_cfg) * n_cfg);
-    const size_t i_th = hc.add(env_theta, nullptr, env_theta ? sizeof(float) * (size_t)env_param_count(c) * n_env : 0);
-    const size_t i_ei = hc.add(env_index, nullptr, env_index ? sizeof(int32_t) * n_lanes : 0);
-    const size_t i_key = hc.add(keys, nullptr, sizeof(uint32_t) * 2 * n_lanes);
+    const LaneSegs s = add_lane_segs(hc, cfgs, sizeof(le_lane_cfg) * n_cfg, c, env_theta, n_env, env_index, keys, n_lanes, out, rewards,
+                                     lengths, test_rewards, nullptr);
     const size_t i_qi = hc.add(q_init, nullptr, q_init ? sizeof(float) * (size_t)Pq * n_lanes : 0);
     const size_t i_qf = hc.add(nullptr, q_final, q_final ? sizeof(float) * (size_t)Pq * n_lanes : 0);
-    const size_t i_out = hc.add(nullptr, out, sizeof(le_lane_out) * n_lanes);
-    const size_t i_rw = hc.add(nullptr, rewards, sizeof(double) * (size_t)rs * n_lanes);
-    const size_t i_ln = hc.add(nullptr, lengths, sizeof(int32_t) * (size_t)rs * n_lanes);
-    const size_t i_tr = hc.add(nullptr, test_rewards, sizeof(double) * (size_t)c->test_episodes * n_lanes);
     const size_t off_ws = hc.reserve((size_t)pl.total_bytes);
-    rc = hc.stage_in();
+    le_trace tr;
+    rc = stage_lane_segs(hc, s, &tr);
     if (rc != LE_OK) return rc;
-    LE_CUDA_CHECK(cudaMemsetAsync(hc.arena + hc.segs[i_rw].off, 0, hc.segs[i_rw].bytes + hc.segs[i_ln].bytes, hc.st));
-    rc = le_inner_loop_run((const le_lane_cfg*)hc.dp(i_cfg), n_cfg, c, (const float*)hc.dp(i_th), n_env, (const int32_t*)hc.dp(i_ei),
-                           (const uint32_t*)hc.dp(i_key), (const float*)hc.dp(i_qi), (float*)hc.dp(i_qf), n_lanes, (le_lane_out*)hc.dp(i_out),
-                           (double*)hc.dp(i_rw), (int32_t*)hc.dp(i_ln), (double*)hc.dp(i_tr), nullptr, hc.arena + off_ws, pl.total_bytes, nullptr, 0,
+    rc = le_inner_loop_run((const le_lane_cfg*)hc.dp(s.cfg), n_cfg, c, (const float*)hc.dp(s.th), n_env, (const int32_t*)hc.dp(s.ei),
+                           (const uint32_t*)hc.dp(s.key), (const float*)hc.dp(i_qi), (float*)hc.dp(i_qf), n_lanes, (le_lane_out*)hc.dp(s.out),
+                           (double*)hc.dp(s.rw), (int32_t*)hc.dp(s.ln), (double*)hc.dp(s.tr), nullptr, hc.arena + off_ws, pl.total_bytes, nullptr, 0,
                            hc.st);
     return hc.stage_out(rc, "le_inner_loop_run_host");   // ~HostCall frees the arena and destroys the stream
 }
@@ -672,31 +843,6 @@ int le_td3_param_counts(const le_td3_cfg* cfg, int* p_actor, int* p_critic) {
     if (p_actor) *p_actor = sd * H + H + (L - 1) * (H * H + H) + H * ad + ad;
     if (p_critic) *p_critic = (sd + ad) * H + H + (L - 1) * (H * H + H) + H + 1;
     return LE_OK;
-}
-
-// the checks of the fields a learn() step reads (nets, minibatch, TD3 hyper-parameters); no CUDA call
-static int td3_learn_check(const le_td3_cfg* cfg, const char* who) {
-    const le_lane_cfg* c = &cfg->base;
-    if (qact_of(c) < 0 || c->q_hidden < 1 || c->q_layers > 3 || cfg->policy_delay < 1 || !(cfg->gumbel_temp > 0.0) || c->ad > 4 ||
-        c->batch_size < 1) {
-        le_set_error("%s: configuration outside the compiled kernel set", who);
-        return LE_EUNSUPPORTED;
-    }
-    if (!le_find_instance(c->sd, c->ad, 1, QACT_TANH)) { le_set_error("no compiled kernel set for state_dim=%d action_dim=%d", c->sd, c->ad); return LE_EUNSUPPORTED; }
-    return LE_OK;
-}
-
-// the checks shared by the TD3 lane entry points, on the (maxima) configuration; no CUDA call
-static int td3_check(const le_td3_cfg* cfg, const char* who) {
-    const le_lane_cfg* c = &cfg->base;
-    int rc = check_env_cfg(c);
-    if (rc != LE_OK) return rc;
-    if (c->env_kind == LE_ENV_RN) { le_set_error("%s: reward-network training envs are not built for TD3 lanes", who); return LE_EUNSUPPORTED; }
-    if (c->train_episodes < 0 || c->test_episodes < 1 || c->max_steps < 1) {
-        le_set_error("%s: configuration outside the compiled kernel set", who);
-        return LE_EUNSUPPORTED;
-    }
-    return td3_learn_check(cfg, who);
 }
 
 int le_td3_learn(const le_td3_cfg* cfg, float* actor_dev, float* actor_target_dev, float* critic1_dev, float* critic1_target_dev,
@@ -715,45 +861,12 @@ int le_td3_learn(const le_td3_cfg* cfg, float* actor_dev, float* actor_target_de
                      (cudaStream_t)stream);
 }
 
-// workspace layout of the TD3 entry points: [SE pack | lane queue counter | resident lane slots]
-struct Td3Layout {
-    Td3Plan tp;
-    const InstanceOps* ops;
-    int ring_cap;
-    int64_t pack_stride_f, off_counter, off_slots, slot_bytes;
-};
-
-static int td3_layout(const le_td3_cfg* cfg, int n_lanes, int n_env, const char* who, Td3Layout* L) {
-    const le_lane_cfg* c = &cfg->base;
-    int rc = td3_check(cfg, who);
-    if (rc != LE_OK) return rc;
-    L->ops = le_find_instance(c->sd, c->ad, 1, QACT_TANH);
-    int dev = 0, sms = 0;
-    LE_CUDA_CHECK(cudaGetDevice(&dev));
-    LE_CUDA_CHECK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
-    L->ring_cap = ring_capacity(c);
-    rc = td3_plan(cfg, n_lanes, L->ring_cap, sms, &L->tp);
-    if (rc != LE_OK) return rc;
-    L->pack_stride_f = (c->env_kind == LE_ENV_SE ? L->ops->se_pack_vec4(c->env_hidden) : 1) * 4;
-    L->off_counter = ((int64_t)(n_env > 0 ? n_env : 1) * L->pack_stride_f * 4 + 255) / 256 * 256;
-    L->off_slots = L->off_counter + 256;
-    L->slot_bytes = L->tp.slot_floats * (int64_t)sizeof(float);
-    return LE_OK;
-}
-
 int64_t le_td3_workspace_bytes(const le_td3_cfg* cfg_host0, int n_lanes, int n_env) {
     if (!cfg_host0 || n_lanes < 1) { le_set_error("le_td3_workspace_bytes: bad arguments"); return LE_EINVAL; }
-    Td3Layout L;
-    const int rc = td3_layout(cfg_host0, n_lanes, n_env, "le_td3_workspace_bytes", &L);
-    if (rc != LE_OK) return rc;
-    // a slot of the widest vary_hp shapes (hidden 1530 x 3 layers) is ~0.3 GB: when every resident lane's slot does not fit
-    // 90 % of the free device memory, ask for fewer slots (the lane queue runs the rest on them)
-    size_t free_b = 0, total_b = 0;
-    LE_CUDA_CHECK(cudaMemGetInfo(&free_b, &total_b));
-    const int64_t room = (int64_t)(0.9 * (double)free_b) - L.off_slots;
-    int64_t slots = L.tp.grid;
-    if (slots * L.slot_bytes > room) slots = room / L.slot_bytes > 1 ? room / L.slot_bytes : 1;
-    return L.off_slots + slots * L.slot_bytes;
+    LanePlan pl;
+    int rc = check_lanes(&cfg_host0->base, cfg_host0, n_lanes, "le_td3_workspace_bytes", &pl);
+    if (rc == LE_OK) rc = plan_lanes(&cfg_host0->base, cfg_host0, n_lanes, n_env, &pl);
+    return rc == LE_OK ? td3_workspace_bytes(pl) : rc;
 }
 
 int le_td3_run(const le_td3_cfg* cfg_dev, int n_cfg, const le_td3_cfg* cfg_host0, const float* env_theta_dev, int n_env,
@@ -768,33 +881,28 @@ int le_td3_run(const le_td3_cfg* cfg_dev, int n_cfg, const le_td3_cfg* cfg_host0
         le_set_error("le_td3_run: bad arguments (n_cfg and n_init must be 1 or n_lanes; all three init arrays or none; no NULL outputs)");
         return LE_EINVAL;
     }
-    Td3Layout L;
-    int rc = td3_layout(cfg_host0, n_lanes, n_env, "le_td3_run", &L);
-    if (rc != LE_OK) return rc;
     const le_lane_cfg* c = &cfg_host0->base;
+    LanePlan pl;
+    int rc = check_lanes(c, cfg_host0, n_lanes, "le_td3_run", &pl);
+    if (rc != LE_OK) return rc;
     if (c->env_kind == LE_ENV_SE && (!env_theta_dev || n_env < 1)) { le_set_error("le_td3_run: env_theta is required for SE lanes"); return LE_EINVAL; }
+    rc = plan_lanes(c, cfg_host0, n_lanes, n_env, &pl);
+    if (rc != LE_OK) return rc;
     // resident lanes: as many slots as the workspace holds, up to the occupancy-bound grid
-    const int64_t fit = workspace_bytes > L.off_slots ? (workspace_bytes - L.off_slots) / L.slot_bytes : 0;
+    const int64_t fit = workspace_bytes > pl.off_slots ? (workspace_bytes - pl.off_slots) / pl.slot_bytes : 0;
     if (fit < 1) {
-        le_set_error("le_td3_run: workspace too small (%lld < %lld bytes)", (long long)workspace_bytes, (long long)(L.off_slots + L.slot_bytes));
+        le_set_error("le_td3_run: workspace too small (%lld < %lld bytes)", (long long)workspace_bytes, (long long)(pl.off_slots + pl.slot_bytes));
         return LE_EINVAL;
     }
-    if (fit < L.tp.grid) L.tp.grid = (int)fit;
+    if (fit < pl.tp.grid) pl.tp.grid = (int)fit;
     cudaStream_t st = (cudaStream_t)stream;
     char* ws = (char*)workspace_dev;
-    LE_CUDA_CHECK(cudaMemsetAsync(ws + L.off_counter, 0, 256, st));
-    LE_CUDA_CHECK(pack_env(L.ops, c, env_theta_dev, n_env, (float*)ws, L.pack_stride_f, st));
     RunParams P;
-    memset(&P, 0, sizeof(P));
-    P.env_pack = (const float4*)ws; P.env_pack_stride = L.pack_stride_f / 4;
-    P.env_index = env_index_dev; P.keys = keys_dev;
-    P.n_lanes = n_lanes; P.out = out_dev; P.rewards = rewards_dev; P.lengths = lengths_dev; P.test_rewards = test_rewards_dev;
-    P.rew_stride = c->train_episodes > 0 ? c->train_episodes : 1; P.test_stride = c->test_episodes;
-    P.ring_cap = L.ring_cap;
-    P.work_counter = (int*)(ws + L.off_counter);
-    if (trace_host && trace_host->cap > 0) { P.trace = *trace_host; P.trace_lane = trace_lane; }
-    cudaError_t le = td3_launch(cfg_dev, n_cfg, cfg_host0, P, (float*)(ws + L.off_slots), L.tp, actor_init_dev, critic1_init_dev, critic2_init_dev,
-                                all_init && n_init == n_lanes && n_lanes > 1, actor_final_dev, st);
+    rc = start_lanes(pl, c, env_theta_dev, n_env, env_index_dev, keys_dev, n_lanes, out_dev, rewards_dev, lengths_dev, test_rewards_dev, ws,
+                     trace_host, trace_lane, st, &P);
+    if (rc != LE_OK) return rc;
+    cudaError_t le = td3_launch(cfg_dev, n_cfg, cfg_host0, P, (float*)(ws + pl.off_slots), pl.tp, actor_init_dev, critic1_init_dev,
+                                critic2_init_dev, all_init && n_init == n_lanes && n_lanes > 1, actor_final_dev, st);
     if (le != cudaSuccess) { le_set_error("td3 launch failed: %s", cudaGetErrorString(le)); return LE_ECUDA; }
     return LE_OK;
 }
@@ -809,52 +917,30 @@ int le_td3_run_host(const le_td3_cfg* cfg, const float* env_theta, int n_env, co
         return LE_EINVAL;
     }
     const le_lane_cfg* c = &cfg->base;
-    int rc = td3_check(cfg, "le_td3_run_host");
-    if (rc != LE_OK) return rc;
-    LE_CUDA_CHECK(cudaSetDevice(device));
-    Td3Layout L;
-    rc = td3_layout(cfg, n_lanes, n_env, "le_td3_run_host", &L);
+    LanePlan pl;
+    int rc = check_lanes(c, cfg, n_lanes, "le_td3_run_host", &pl);
     if (rc != LE_OK) return rc;
     if (c->env_kind == LE_ENV_SE && (!env_theta || n_env < 1)) { le_set_error("le_td3_run_host: env_theta is required for SE lanes"); return LE_EINVAL; }
-    const int64_t ws_bytes = le_td3_workspace_bytes(cfg, n_lanes, n_env);
-    if (ws_bytes < 0) return (int)ws_bytes;
-    const int rs = c->train_episodes > 0 ? c->train_episodes : 1;
-    const int tcap = trace_host ? trace_host->cap : 0;
-    HostCall hc;
-    const size_t i_cfg = hc.add(cfg, nullptr, sizeof(le_td3_cfg));
-    const size_t i_th = hc.add(env_theta, nullptr, sizeof(float) * (size_t)env_param_count(c) * n_env);
-    const size_t i_ei = hc.add(env_index, nullptr, env_index ? sizeof(int32_t) * n_lanes : 0);
-    const size_t i_key = hc.add(keys, nullptr, sizeof(uint32_t) * 2 * n_lanes);
-    const size_t i_a = hc.add(actor_init, nullptr, sizeof(float) * (size_t)L.tp.p_actor * n_init);
-    const size_t i_c1 = hc.add(critic1_init, nullptr, sizeof(float) * (size_t)L.tp.p_critic * n_init);
-    const size_t i_c2 = hc.add(critic2_init, nullptr, sizeof(float) * (size_t)L.tp.p_critic * n_init);
-    const size_t i_af = hc.add(nullptr, actor_final, actor_final ? sizeof(float) * (size_t)L.tp.p_actor * n_lanes : 0);
-    const size_t i_out = hc.add(nullptr, out, sizeof(le_lane_out) * n_lanes);
-    const size_t i_rw = hc.add(nullptr, rewards, sizeof(double) * (size_t)rs * n_lanes);
-    const size_t i_ln = hc.add(nullptr, lengths, sizeof(int32_t) * (size_t)rs * n_lanes);
-    const size_t i_tr = hc.add(nullptr, test_rewards, sizeof(double) * (size_t)c->test_episodes * n_lanes);
-    const size_t i_ta = hc.add(nullptr, tcap ? trace_host->action : nullptr, sizeof(int32_t) * (size_t)tcap);
-    const size_t i_te = hc.add(nullptr, tcap ? trace_host->explore : nullptr, sizeof(int32_t) * (size_t)tcap);
-    const size_t i_tn = hc.add(nullptr, tcap ? trace_host->next_state : nullptr, sizeof(float) * (size_t)tcap * c->sd);
-    const size_t i_trw = hc.add(nullptr, tcap ? trace_host->reward : nullptr, sizeof(float) * (size_t)tcap);
-    const size_t i_td = hc.add(nullptr, tcap ? trace_host->done : nullptr, sizeof(float) * (size_t)tcap);
-    const size_t i_tl = hc.add(nullptr, tcap ? trace_host->loss : nullptr, sizeof(float) * (size_t)tcap);
-    const size_t off_ws = hc.reserve((size_t)ws_bytes);
-    rc = hc.stage_in();
+    LE_CUDA_CHECK(cudaSetDevice(device));
+    rc = plan_lanes(c, cfg, n_lanes, n_env, &pl);
     if (rc != LE_OK) return rc;
-    char* arena = hc.arena;
-    LE_CUDA_CHECK(cudaMemsetAsync(arena + hc.segs[i_rw].off, 0, hc.segs[i_rw].bytes + hc.segs[i_ln].bytes, hc.st));
+    const int64_t ws_bytes = td3_workspace_bytes(pl);
+    if (ws_bytes < 0) return (int)ws_bytes;
+    HostCall hc;
+    const LaneSegs s = add_lane_segs(hc, cfg, sizeof(le_td3_cfg), c, env_theta, n_env, env_index, keys, n_lanes, out, rewards, lengths,
+                                     test_rewards, trace_host);
+    const size_t i_a = hc.add(actor_init, nullptr, sizeof(float) * (size_t)pl.tp.p_actor * n_init);
+    const size_t i_c1 = hc.add(critic1_init, nullptr, sizeof(float) * (size_t)pl.tp.p_critic * n_init);
+    const size_t i_c2 = hc.add(critic2_init, nullptr, sizeof(float) * (size_t)pl.tp.p_critic * n_init);
+    const size_t i_af = hc.add(nullptr, actor_final, actor_final ? sizeof(float) * (size_t)pl.tp.p_actor * n_lanes : 0);
+    const size_t off_ws = hc.reserve((size_t)ws_bytes);
     le_trace tr;
-    memset(&tr, 0, sizeof(tr));
-    if (tcap) {
-        LE_CUDA_CHECK(cudaMemsetAsync(arena + hc.segs[i_ta].off, 0xff, off_ws - hc.segs[i_ta].off, hc.st));   /* untouched trace slots: -1 / NaN */
-        tr.cap = tcap; tr.action = (int32_t*)hc.dp(i_ta); tr.explore = (int32_t*)hc.dp(i_te); tr.next_state = (float*)hc.dp(i_tn);
-        tr.reward = (float*)hc.dp(i_trw); tr.done = (float*)hc.dp(i_td); tr.loss = (float*)hc.dp(i_tl);
-    }
-    rc = le_td3_run((const le_td3_cfg*)hc.dp(i_cfg), 1, cfg, (const float*)hc.dp(i_th), n_env, (const int32_t*)hc.dp(i_ei),
-                    (const uint32_t*)hc.dp(i_key), (const float*)hc.dp(i_a), (const float*)hc.dp(i_c1), (const float*)hc.dp(i_c2), n_init,
-                    (float*)hc.dp(i_af), n_lanes, (le_lane_out*)hc.dp(i_out), (double*)hc.dp(i_rw), (int32_t*)hc.dp(i_ln), (double*)hc.dp(i_tr),
-                    arena + off_ws, ws_bytes, tcap ? &tr : nullptr, trace_lane, hc.st);
+    rc = stage_lane_segs(hc, s, &tr);
+    if (rc != LE_OK) return rc;
+    rc = le_td3_run((const le_td3_cfg*)hc.dp(s.cfg), 1, cfg, (const float*)hc.dp(s.th), n_env, (const int32_t*)hc.dp(s.ei),
+                    (const uint32_t*)hc.dp(s.key), (const float*)hc.dp(i_a), (const float*)hc.dp(i_c1), (const float*)hc.dp(i_c2), n_init,
+                    (float*)hc.dp(i_af), n_lanes, (le_lane_out*)hc.dp(s.out), (double*)hc.dp(s.rw), (int32_t*)hc.dp(s.ln), (double*)hc.dp(s.tr),
+                    hc.arena + off_ws, ws_bytes, tr.cap ? &tr : nullptr, trace_lane, hc.st);
     return hc.stage_out(rc, "le_td3_run_host");   // ~HostCall frees the arena and destroys the stream
 }
 

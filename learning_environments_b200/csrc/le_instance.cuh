@@ -1,6 +1,8 @@
-// le_instance.cuh — launchers for one compiled (SD, AD, U, ACT) kernel set.  The instantiations live in
-// le_inst_*.cu (one translation unit per environment shape x activation so they compile in parallel);
-// le_api.cu looks them up with le_find_instance().
+// le_instance.cuh — launchers for one compiled (SD, AD, U, ACT) register Q-net kernel set: the warp, multi-warp and
+// cluster lane kernels and the Q-net unit operators.  The instantiations live in le_inst_*.cu (one translation unit per
+// environment shape x activation so they compile in parallel); le_api.cu looks up the kernel set of a lane with
+// le_find_instance().  The environment kernels (packing, SE / RN unit operators) depend on the shape only and are compiled
+// once, in le_api.cu.
 #pragma once
 #include "le_inner_loop.cuh"
 
@@ -17,21 +19,7 @@ struct InstanceOps {
     // fused persistent kernel
     int (*inner_max_ctas_per_sm)();
     cudaError_t (*launch_inner)(const RunParams& P, int grid, cudaStream_t st);
-    int64_t (*ring_row_floats)();
-    // environment packing
-    int64_t (*se_pack_vec4)(int H);
-    int64_t (*rn_pack_vec4)(int H);
-    cudaError_t (*launch_pack_se)(const float* theta, int P_env, int n_env, int H, const float* slopes, float* out,
-                                  int64_t out_stride_f, cudaStream_t st);
-    cudaError_t (*launch_pack_rn)(const float* theta, int P_env, int n_env, int H, float slope, float* out,
-                                  int64_t out_stride_f, cudaStream_t st);
     // unit operators
-    cudaError_t (*launch_se_forward)(const float4* pack, int64_t pack_stride, int H, int is_tanh, int lanes_per_member,
-                                     const float* state, const int32_t* action, float* ns, float* reward, float* done, int n,
-                                     cudaStream_t st);
-    cudaError_t (*launch_rn_reward)(const float4* pack, int64_t pack_stride, int H, int is_tanh, int rn_type, float gamma,
-                                    int lanes_per_member, const float* s, const float* s2, const float* rr, float* out, int n,
-                                    cudaStream_t st);
     cudaError_t (*launch_qnet_forward)(const float* q_theta, int q_stride, int H, float slope, const float* state, float* q_out,
                                        int32_t* argmax, int n, cudaStream_t st);
     cudaError_t (*launch_td_update)(const le_lane_cfg* cfg_dev, float* th, float* thT, float* m, float* v, int32_t* t, int q_stride,
@@ -42,41 +30,7 @@ const InstanceOps* le_find_instance(int sd, int ad, int units_needed, int act);
 void le_register_instance(const InstanceOps* ops);
 
 // ------------------------------------------------------------------------------------------------------
-// unit kernels (one warp per row / lane), sharing the device code of the fused kernel
-
-template <int SD, int AD>
-__global__ void se_forward_kernel(const float4* __restrict__ pack, int64_t pack_stride, int H, int is_tanh, int lanes_per_member,
-                                  const float* __restrict__ state, const int32_t* __restrict__ action, float* __restrict__ ns_out,
-                                  float* __restrict__ reward, float* __restrict__ done, int n) {
-    const int lane = threadIdx.x & 31;
-    const int row = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
-    if (row >= n) return;
-    float s[SD], ns[SD], r, d;
-#pragma unroll
-    for (int i = 0; i < SD; ++i) s[i] = state[(int64_t)row * SD + i];
-    se_step_row<SD, AD>(pack + (int64_t)(row / lanes_per_member) * pack_stride, H, is_tanh != 0, s, action[row], lane, ns, r, d);
-    if (lane == 0) {
-#pragma unroll
-        for (int i = 0; i < SD; ++i) ns_out[(int64_t)row * SD + i] = ns[i];
-        reward[row] = r;
-        done[row] = d;
-    }
-}
-
-template <int SD>
-__global__ void rn_reward_kernel(const float4* __restrict__ pack, int64_t pack_stride, int H, int is_tanh, int rn_type, float gamma,
-                                 int lanes_per_member, const float* __restrict__ s_in, const float* __restrict__ s2_in,
-                                 const float* __restrict__ rr, float* __restrict__ out, int n) {
-    const int lane = threadIdx.x & 31;
-    const int row = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
-    if (row >= n) return;
-    float s[SD], s2[SD];
-#pragma unroll
-    for (int i = 0; i < SD; ++i) { s[i] = s_in[(int64_t)row * SD + i]; s2[i] = s2_in[(int64_t)row * SD + i]; }
-    float ps = 0.f, ps2 = 0.f;
-    if (rn_type != 0) rn_phi2<SD>(pack + (int64_t)(row / lanes_per_member) * pack_stride, H, is_tanh != 0, s, s2, lane, ps, ps2);
-    if (lane == 0) out[row] = rn_combine(rn_type, gamma, rr[row], ps, ps2);
-}
+// Q-net unit kernels (one warp per row / lane), sharing the device code of the fused kernel
 
 template <int SD, int AD, int U, int ACT>
 __global__ void qnet_forward_kernel(const float* __restrict__ q_theta, int q_stride, int H, float slope,
@@ -214,37 +168,6 @@ struct InstanceImpl {
             return cudaLaunchKernelEx(&cfg, inner_loop_mwc_kernel<SD, AD, U, ACT>, P);
         } else return cudaErrorInvalidConfiguration;
     }
-    static int64_t ring_row_floats() { return RowLayout<SD>::ROWF; }
-    static int64_t se_pack_vec4(int H) { return SePack<SD, AD>::pack_vec4(H); }
-    static int64_t rn_pack_vec4(int H) { return RnPack<SD>::pack_vec4(H); }
-    static cudaError_t launch_pack_se(const float* theta, int P_env, int n_env, int H, const float* slopes, float* out,
-                                      int64_t out_stride_f, cudaStream_t st) {
-        const int64_t total = SePack<SD, AD>::pack_vec4(H) * 4 * n_env;
-        const int grid = (int)((total + 255) / 256 < 4096 ? (total + 255) / 256 : 4096);
-        pack_se_kernel<SD, AD><<<grid, 256, 0, st>>>(theta, P_env, n_env, H, slopes[0], slopes[1], slopes[2], out, out_stride_f);
-        return cudaGetLastError();
-    }
-    static cudaError_t launch_pack_rn(const float* theta, int P_env, int n_env, int H, float slope, float* out, int64_t out_stride_f,
-                                      cudaStream_t st) {
-        const int64_t total = RnPack<SD>::pack_vec4(H) * 4 * n_env;
-        const int grid = (int)((total + 255) / 256 < 4096 ? (total + 255) / 256 : 4096);
-        pack_rn_kernel<SD><<<grid, 256, 0, st>>>(theta, P_env, n_env, H, slope, out, out_stride_f);
-        return cudaGetLastError();
-    }
-    static cudaError_t launch_se_forward(const float4* pack, int64_t pack_stride, int H, int is_tanh, int lanes_per_member,
-                                         const float* state, const int32_t* action, float* ns, float* reward, float* done, int n,
-                                         cudaStream_t st) {
-        const int grid = (n + 3) / 4;
-        se_forward_kernel<SD, AD><<<grid, 128, 0, st>>>(pack, pack_stride, H, is_tanh, lanes_per_member, state, action, ns, reward, done, n);
-        return cudaGetLastError();
-    }
-    static cudaError_t launch_rn_reward(const float4* pack, int64_t pack_stride, int H, int is_tanh, int rn_type, float gamma,
-                                        int lanes_per_member, const float* s, const float* s2, const float* rr, float* out, int n,
-                                        cudaStream_t st) {
-        const int grid = (n + 3) / 4;
-        rn_reward_kernel<SD><<<grid, 128, 0, st>>>(pack, pack_stride, H, is_tanh, rn_type, gamma, lanes_per_member, s, s2, rr, out, n);
-        return cudaGetLastError();
-    }
     static cudaError_t launch_qnet_forward(const float* q_theta, int q_stride, int H, float slope, const float* state, float* q_out,
                                            int32_t* argmax, int n, cudaStream_t st) {
         const int grid = (n + 3) / 4;
@@ -260,8 +183,7 @@ struct InstanceImpl {
         return cudaGetLastError();
     }
     static const InstanceOps* ops() {
-        static const InstanceOps o = {SD, AD, U, ACT, kInnerWarps, kMwOk ? mw_warps<U>() : 0, (int64_t)kMwSmemBytes, kMwcOk ? (int64_t)kMwcSmemBytes : 0, launch_inner_mwc, launch_inner_mw, inner_max_ctas_per_sm, launch_inner, ring_row_floats, se_pack_vec4,
-                                      rn_pack_vec4, launch_pack_se, launch_pack_rn, launch_se_forward, launch_rn_reward,
+        static const InstanceOps o = {SD, AD, U, ACT, kInnerWarps, kMwOk ? mw_warps<U>() : 0, (int64_t)kMwSmemBytes, kMwcOk ? (int64_t)kMwcSmemBytes : 0, launch_inner_mwc, launch_inner_mw, inner_max_ctas_per_sm, launch_inner,
                                       launch_qnet_forward, launch_td_update};
         return &o;
     }

@@ -163,29 +163,28 @@ def lane_out_dtype():
                      ("test_steps", np.int64), ("score", np.float64)])
 
 
-class InnerLoopBuffers(object):
-    """Device buffers of one le_inner_loop_run call (allocated once, reusable across generations)."""
+class _LaneBuffers(object):
+    """Device buffers every lane launch uses, allocated once and reusable across generations: the workspace of `ws` bytes (a
+    negative `ws` is the error code of the workspace query `who`), per-lane results, reward / length histories, final test
+    rewards, n_cfg device copies of the lane configuration `cfg` (`base`: its LaneCfg) and an optional trace of trace_cap steps."""
 
-    def __init__(self, cfg, n_lanes, n_env, device, n_cfg=1, trace_cap=0, want_q_final=False):
+    def __init__(self, cfg, base, n_lanes, n_env, device, n_cfg, trace_cap, ws, who):
         self.cfg, self.n_lanes, self.n_env, self.device = cfg, n_lanes, n_env, device
-        ws = _lib().le_inner_loop_workspace_bytes(C.byref(cfg), C.c_int(n_lanes), C.c_int(n_env))
         if ws < 0:
-            check(int(ws), "le_inner_loop_workspace_bytes")
+            check(int(ws), who)
         self.workspace = torch.empty(int(ws), dtype=torch.uint8, device=device)
-        rs = max(cfg.train_episodes, 1)
+        rs = max(base.train_episodes, 1)
         self.out = torch.zeros((n_lanes, C.sizeof(LaneOut)), dtype=torch.uint8, device=device)
         self.rewards = torch.zeros((n_lanes, rs), dtype=_F64, device=device)
         self.lengths = torch.zeros((n_lanes, rs), dtype=_I32, device=device)
-        self.test_rewards = torch.zeros((n_lanes, cfg.test_episodes), dtype=_F64, device=device)
-        self.test_lengths = torch.zeros((n_lanes, cfg.test_episodes), dtype=_I32, device=device)
-        self.q_final = torch.zeros((n_lanes, cfg.q_params()), dtype=_F32, device=device) if want_q_final else None
-        self.cfg_dev = torch.zeros((n_cfg, C.sizeof(LaneCfg)), dtype=torch.uint8, device=device)
+        self.test_rewards = torch.zeros((n_lanes, base.test_episodes), dtype=_F64, device=device)
+        self.cfg_dev = torch.zeros((n_cfg, C.sizeof(cfg)), dtype=torch.uint8, device=device)
         self.trace = None
         if trace_cap > 0:
             self.trace = dict(cap=trace_cap,
                               action=torch.full((trace_cap,), -1, dtype=_I32, device=device),
                               explore=torch.zeros(trace_cap, dtype=_I32, device=device),
-                              next_state=torch.zeros((trace_cap, cfg.sd), dtype=_F32, device=device),
+                              next_state=torch.zeros((trace_cap, base.sd), dtype=_F32, device=device),
                               reward=torch.zeros(trace_cap, dtype=_F32, device=device),
                               done=torch.zeros(trace_cap, dtype=_F32, device=device),
                               loss=torch.full((trace_cap,), float("nan"), dtype=_F32, device=device),
@@ -193,8 +192,36 @@ class InnerLoopBuffers(object):
 
     def results(self):
         """One D2H read of the per-lane results."""
-        o = np.frombuffer(self.out.cpu().numpy().tobytes(), dtype=lane_out_dtype())
-        return o
+        return np.frombuffer(self.out.cpu().numpy().tobytes(), dtype=lane_out_dtype())
+
+    def _launch_args(self, cfgs, keys):
+        """The arguments a launch on these buffers shares: n_cfg, after uploading the configurations when they changed (they
+        rarely do between generations); the checked keys; the trace (by reference) or None."""
+        n_cfg = len(cfgs)
+        assert n_cfg in (1, self.n_lanes) and self.cfg_dev.shape[0] == n_cfg
+        raw = b"".join(bytes(c) for c in cfgs)
+        if getattr(self, "_cfg_raw", None) != raw:
+            self.cfg_dev.copy_(torch.frombuffer(bytearray(raw), dtype=torch.uint8).reshape(n_cfg, -1), non_blocking=False)
+            self._cfg_raw = raw
+        keys = _dev(keys, _I32)
+        assert keys.numel() == 2 * self.n_lanes
+        tr = None
+        if self.trace is not None:
+            tr = Trace()
+            tr.cap = self.trace["cap"]
+            for n in ("action", "explore", "next_state", "reward", "done", "loss", "qgap"):
+                setattr(tr, n, self.trace[n].data_ptr())
+        return n_cfg, keys, C.byref(tr) if tr is not None else None
+
+
+class InnerLoopBuffers(_LaneBuffers):
+    """Device buffers of one le_inner_loop_run call (allocated once, reusable across generations)."""
+
+    def __init__(self, cfg, n_lanes, n_env, device, n_cfg=1, trace_cap=0, want_q_final=False):
+        ws = _lib().le_inner_loop_workspace_bytes(C.byref(cfg), C.c_int(n_lanes), C.c_int(n_env))
+        super().__init__(cfg, cfg, n_lanes, n_env, device, n_cfg, trace_cap, ws, "le_inner_loop_workspace_bytes")
+        self.test_lengths = torch.zeros((n_lanes, cfg.test_episodes), dtype=_I32, device=device)
+        self.q_final = torch.zeros((n_lanes, cfg.q_params()), dtype=_F32, device=device) if want_q_final else None
 
 
 def inner_loop_run(bufs, cfgs, env_theta, env_index, keys, q_init=None, trace_lane=0, cfg0=None):
@@ -204,30 +231,14 @@ def inner_loop_run(bufs, cfgs, env_theta, env_index, keys, q_init=None, trace_la
     (None for ENV_REAL); env_index [n_lanes] int32 or None; keys [n_lanes, 2] (uint32 values in an int64/int32 tensor).
     """
     cfg0 = bufs.cfg if cfg0 is None else cfg0     # shapes / strides / kernel set: the maxima under per-lane configurations
-    if isinstance(cfgs, LaneCfg):
-        cfgs = [cfgs]
-    n_cfg = len(cfgs)
-    assert n_cfg in (1, bufs.n_lanes) and bufs.cfg_dev.shape[0] == n_cfg
-    raw = b"".join(bytes(c) for c in cfgs)
-    if getattr(bufs, "_cfg_raw", None) != raw:      # lane configurations rarely change between generations: upload once
-        bufs.cfg_dev.copy_(torch.frombuffer(bytearray(raw), dtype=torch.uint8).reshape(n_cfg, -1), non_blocking=False)
-        bufs._cfg_raw = raw
-    keys = _dev(keys, _I32)
-    assert keys.numel() == 2 * bufs.n_lanes
-    tr = None
-    if bufs.trace is not None:
-        tr = Trace()
-        tr.cap = bufs.trace["cap"]
-        for n in ("action", "explore", "next_state", "reward", "done", "loss", "qgap"):
-            setattr(tr, n, bufs.trace[n].data_ptr())
+    n_cfg, keys, tr = bufs._launch_args([cfgs] if isinstance(cfgs, LaneCfg) else cfgs, keys)
     n_env = 0 if env_theta is None else env_theta.reshape(-1, max(cfg0.env_params(), 1)).shape[0]
     with _on(bufs.workspace) as stream:
         check(_lib().le_inner_loop_run(
-            _ptr(bufs.cfg_dev), C.c_int(n_cfg), C.byref(cfg0), _ptr(env_theta) if env_theta is not None else None, C.c_int(n_env),
-            _ptr(env_index) if env_index is not None else None, _ptr(keys), _ptr(q_init) if q_init is not None else None,
-            _ptr(bufs.q_final) if bufs.q_final is not None else None, C.c_int(bufs.n_lanes), _ptr(bufs.out), _ptr(bufs.rewards),
-            _ptr(bufs.lengths), _ptr(bufs.test_rewards), _ptr(bufs.test_lengths), _ptr(bufs.workspace), C.c_int64(bufs.workspace.numel()),
-            C.byref(tr) if tr is not None else None, C.c_int(trace_lane), stream), "le_inner_loop_run")
+            _ptr(bufs.cfg_dev), C.c_int(n_cfg), C.byref(cfg0), _ptr(env_theta), C.c_int(n_env), _ptr(env_index), _ptr(keys), _ptr(q_init),
+            _ptr(bufs.q_final), C.c_int(bufs.n_lanes), _ptr(bufs.out), _ptr(bufs.rewards), _ptr(bufs.lengths), _ptr(bufs.test_rewards),
+            _ptr(bufs.test_lengths), _ptr(bufs.workspace), C.c_int64(bufs.workspace.numel()), tr, C.c_int(trace_lane), stream),
+            "le_inner_loop_run")
 
 
 def keys_tensor(keys, device):
@@ -236,34 +247,40 @@ def keys_tensor(keys, device):
     return torch.from_numpy(k.view(np.int32).copy()).to(device)
 
 
+def _host_lane_arrays(base, env_theta, env_index, keys):
+    """The HOST arrays both *_run_host calls pass: keys [n, 2] uint32, env_theta [n_env, P_env] and env_index (or None), and the
+    zeroed result arrays of n lanes of the LaneCfg `base`."""
+    keys = np.ascontiguousarray(np.asarray(keys, dtype=np.uint32).reshape(-1, 2))
+    n = keys.shape[0]
+    th = None if env_theta is None else np.ascontiguousarray(env_theta, np.float32).reshape(-1, base.env_params())
+    ei = None if env_index is None else np.ascontiguousarray(env_index, np.int32)
+    rs = max(base.train_episodes, 1)
+    res = dict(out=np.zeros(n, dtype=lane_out_dtype()), rewards=np.zeros((n, rs), np.float64), lengths=np.zeros((n, rs), np.int32),
+               test_rewards=np.zeros((n, base.test_episodes), np.float64))
+    return keys, th, ei, res
+
+
+def _hptr(a):
+    return a.ctypes.data_as(C.c_void_p) if a is not None else None
+
+
+def _res_ptrs(res):
+    return _hptr(res["out"]), _hptr(res["rewards"]), _hptr(res["lengths"]), _hptr(res["test_rewards"])
+
+
 def inner_loop_run_host(cfgs, env_theta, env_index, keys, q_init=None, want_q_final=False, device=0):
     """le_inner_loop_run_host: everything in HOST numpy buffers, H2D/D2H inside the call. Returns dict of arrays."""
     if isinstance(cfgs, LaneCfg):
         cfgs = [cfgs]
     c0 = cfgs[0]
-    n_cfg = len(cfgs)
-    arr = (LaneCfg * n_cfg)(*cfgs)
-    keys = np.ascontiguousarray(np.asarray(keys, dtype=np.uint32).reshape(-1, 2))
+    keys, th, ei, res = _host_lane_arrays(c0, env_theta, env_index, keys)
     n = keys.shape[0]
-    n_env = 0
-    th = None
-    if env_theta is not None:
-        th = np.ascontiguousarray(env_theta, np.float32).reshape(-1, c0.env_params())
-        n_env = th.shape[0]
-    ei = None if env_index is None else np.ascontiguousarray(env_index, np.int32)
     qi = None if q_init is None else np.ascontiguousarray(q_init, np.float32)
-    qf = np.zeros((n, c0.q_params()), np.float32) if want_q_final else None
-    out = np.zeros(n, dtype=lane_out_dtype())
-    rs = max(c0.train_episodes, 1)
-    rewards = np.zeros((n, rs), np.float64)
-    lengths = np.zeros((n, rs), np.int32)
-    test_rewards = np.zeros((n, c0.test_episodes), np.float64)
-
-    def p(a):
-        return a.ctypes.data_as(C.c_void_p) if a is not None else None
-    check(_lib().le_inner_loop_run_host(arr, C.c_int(n_cfg), p(th), C.c_int(n_env), p(ei), p(keys), p(qi), p(qf), C.c_int(n), p(out),
-                                        p(rewards), p(lengths), p(test_rewards), C.c_int(device)), "le_inner_loop_run_host")
-    return dict(out=out, rewards=rewards, lengths=lengths, test_rewards=test_rewards, q_final=qf)
+    res["q_final"] = np.zeros((n, c0.q_params()), np.float32) if want_q_final else None
+    check(_lib().le_inner_loop_run_host((LaneCfg * len(cfgs))(*cfgs), C.c_int(len(cfgs)), _hptr(th), C.c_int(0 if th is None else th.shape[0]),
+                                        _hptr(ei), _hptr(keys), _hptr(qi), _hptr(res["q_final"]), C.c_int(n), *_res_ptrs(res),
+                                        C.c_int(device)), "le_inner_loop_run_host")
+    return res
 
 
 # ---------------------------------------------------------------------------------------------------------
@@ -338,39 +355,16 @@ def td3_learn(tcfg, nets, adam, counters, rows, policy_noise, expo_target, expo_
     return loss
 
 
-class Td3Buffers(object):
+class Td3Buffers(_LaneBuffers):
     """Device buffers of one le_td3_run call, sized for `tcfg0` (the maxima configuration of the launch); the counterpart of
     InnerLoopBuffers for TD3_discrete_vary lanes."""
 
     def __init__(self, tcfg0, n_lanes, n_env, device, n_cfg=1, trace_cap=0, want_actor_final=False):
         assert isinstance(tcfg0, Td3Cfg)
-        self.cfg, self.n_lanes, self.n_env, self.device = tcfg0, n_lanes, n_env, device
-        c = tcfg0.base
         ws = _lib().le_td3_workspace_bytes(C.byref(tcfg0), C.c_int(n_lanes), C.c_int(n_env))
-        if ws < 0:
-            check(int(ws), "le_td3_workspace_bytes")
-        self.workspace = torch.empty(int(ws), dtype=torch.uint8, device=device)
+        super().__init__(tcfg0, tcfg0.base, n_lanes, n_env, device, n_cfg, trace_cap, ws, "le_td3_workspace_bytes")
         self.p_actor, self.p_critic = td3_param_counts(tcfg0)
-        rs = max(c.train_episodes, 1)
-        self.out = torch.zeros((n_lanes, C.sizeof(LaneOut)), dtype=torch.uint8, device=device)
-        self.rewards = torch.zeros((n_lanes, rs), dtype=_F64, device=device)
-        self.lengths = torch.zeros((n_lanes, rs), dtype=_I32, device=device)
-        self.test_rewards = torch.zeros((n_lanes, c.test_episodes), dtype=_F64, device=device)
         self.actor_final = torch.zeros((n_lanes, self.p_actor), dtype=_F32, device=device) if want_actor_final else None
-        self.cfg_dev = torch.zeros((n_cfg, C.sizeof(Td3Cfg)), dtype=torch.uint8, device=device)
-        self.trace = None
-        if trace_cap > 0:
-            self.trace = dict(cap=trace_cap,
-                              action=torch.full((trace_cap,), -1, dtype=_I32, device=device),
-                              explore=torch.zeros(trace_cap, dtype=_I32, device=device),
-                              next_state=torch.zeros((trace_cap, c.sd), dtype=_F32, device=device),
-                              reward=torch.zeros(trace_cap, dtype=_F32, device=device),
-                              done=torch.zeros(trace_cap, dtype=_F32, device=device),
-                              loss=torch.full((trace_cap,), float("nan"), dtype=_F32, device=device),
-                              qgap=torch.full((trace_cap,), float("nan"), dtype=_F32, device=device))
-
-    def results(self):
-        return np.frombuffer(self.out.cpu().numpy().tobytes(), dtype=lane_out_dtype())
 
 
 def td3_run(bufs, tcfgs, env_theta, env_index, keys, inits=None, trace_lane=0):
@@ -382,18 +376,11 @@ def td3_run(bufs, tcfgs, env_theta, env_index, keys, inits=None, trace_lane=0):
     in its row."""
     if isinstance(tcfgs, Td3Cfg):
         tcfgs = [tcfgs]
-    n_cfg = len(tcfgs)
-    assert n_cfg in (1, bufs.n_lanes) and bufs.cfg_dev.shape[0] == n_cfg
     m = bufs.cfg.base
     for t in tcfgs:
         if t.base.q_hidden > m.q_hidden or t.base.q_layers > m.q_layers or t.base.batch_size > m.batch_size:
             raise ValueError("a lane configuration exceeds the maxima the buffers were sized for")
-    raw = b"".join(bytes(t) for t in tcfgs)
-    if getattr(bufs, "_cfg_raw", None) != raw:
-        bufs.cfg_dev.copy_(torch.frombuffer(bytearray(raw), dtype=torch.uint8).reshape(n_cfg, -1), non_blocking=False)
-        bufs._cfg_raw = raw
-    keys = _dev(keys, _I32)
-    assert keys.numel() == 2 * bufs.n_lanes
+    n_cfg, keys, tr = bufs._launch_args(tcfgs, keys)
     a0 = q1 = q2 = None
     n_init = 0
     if inits is not None:
@@ -401,19 +388,13 @@ def td3_run(bufs, tcfgs, env_theta, env_index, keys, inits=None, trace_lane=0):
         n_init = a0.shape[0]
         assert a0.shape == (n_init, bufs.p_actor) and q1.shape == q2.shape == (n_init, bufs.p_critic) and n_init in (1, bufs.n_lanes)
         a0, q1, q2 = (_dev(x, _F32) for x in (a0, q1, q2))
-    tr = None
-    if bufs.trace is not None:
-        tr = Trace()
-        tr.cap = bufs.trace["cap"]
-        for n in ("action", "explore", "next_state", "reward", "done", "loss", "qgap"):
-            setattr(tr, n, bufs.trace[n].data_ptr())
     n_env = 0 if env_theta is None else env_theta.reshape(-1, max(m.env_params(), 1)).shape[0]
     with _on(bufs.workspace) as stream:
         check(_lib().le_td3_run(
             _ptr(bufs.cfg_dev), C.c_int(n_cfg), C.byref(bufs.cfg), _ptr(env_theta), C.c_int(n_env), _ptr(env_index), _ptr(keys),
             _ptr(a0), _ptr(q1), _ptr(q2), C.c_int(n_init), _ptr(bufs.actor_final), C.c_int(bufs.n_lanes), _ptr(bufs.out),
             _ptr(bufs.rewards), _ptr(bufs.lengths), _ptr(bufs.test_rewards), _ptr(bufs.workspace), C.c_int64(bufs.workspace.numel()),
-            C.byref(tr) if tr is not None else None, C.c_int(trace_lane), stream), "le_td3_run")
+            tr, C.c_int(trace_lane), stream), "le_td3_run")
 
 
 def td3_run_host(tcfg, env_theta, env_index, keys, actor_init, critic1_init, critic2_init, trace_cap=0, trace_lane=0, device=0):
@@ -421,35 +402,23 @@ def td3_run_host(tcfg, env_theta, env_index, keys, actor_init, critic1_init, cri
     actor_init [1 or n, P_actor], critic*_init [1 or n, P_critic].  Returns a dict of arrays (+ 'trace' when trace_cap > 0)."""
     assert isinstance(tcfg, Td3Cfg)
     c = tcfg.base
-    keys = np.ascontiguousarray(np.asarray(keys, dtype=np.uint32).reshape(-1, 2))
+    keys, th, ei, res = _host_lane_arrays(c, env_theta, env_index, keys)
     n = keys.shape[0]
     Pa, Pc = td3_param_counts(tcfg)
     a0 = np.ascontiguousarray(actor_init, np.float32).reshape(-1, Pa)
     q1 = np.ascontiguousarray(critic1_init, np.float32).reshape(-1, Pc)
     q2 = np.ascontiguousarray(critic2_init, np.float32).reshape(-1, Pc)
     assert a0.shape[0] == q1.shape[0] == q2.shape[0] and a0.shape[0] in (1, n)
-    th, n_env = None, 0
-    if env_theta is not None:
-        th = np.ascontiguousarray(env_theta, np.float32).reshape(-1, c.env_params())
-        n_env = th.shape[0]
-    ei = None if env_index is None else np.ascontiguousarray(env_index, np.int32)
-    af = np.zeros((n, Pa), np.float32)
-    out = np.zeros(n, dtype=lane_out_dtype())
-    rs = max(c.train_episodes, 1)
-    rewards, lengths = np.zeros((n, rs), np.float64), np.zeros((n, rs), np.int32)
-    test_rewards = np.zeros((n, c.test_episodes), np.float64)
-    tr, trace = None, None
+    res["actor_final"] = np.zeros((n, Pa), np.float32)
+    tr, res["trace"] = None, None
     if trace_cap > 0:
-        trace = dict(action=np.zeros(trace_cap, np.int32), explore=np.zeros(trace_cap, np.int32), next_state=np.zeros((trace_cap, c.sd), np.float32),
-                     reward=np.zeros(trace_cap, np.float32), done=np.zeros(trace_cap, np.float32), loss=np.zeros(trace_cap, np.float32))
+        res["trace"] = dict(action=np.zeros(trace_cap, np.int32), explore=np.zeros(trace_cap, np.int32), next_state=np.zeros((trace_cap, c.sd), np.float32),
+                            reward=np.zeros(trace_cap, np.float32), done=np.zeros(trace_cap, np.float32), loss=np.zeros(trace_cap, np.float32))
         tr = Trace()
         tr.cap = trace_cap
-        for k, v in trace.items():
+        for k, v in res["trace"].items():
             setattr(tr, k, v.ctypes.data)
-
-    def p(a):
-        return a.ctypes.data_as(C.c_void_p) if a is not None else None
-    check(_lib().le_td3_run_host(C.byref(tcfg), p(th), C.c_int(n_env), p(ei), p(keys), p(a0), p(q1), p(q2), C.c_int(a0.shape[0]), p(af),
-                                 C.c_int(n), p(out), p(rewards), p(lengths), p(test_rewards), C.byref(tr) if tr is not None else None,
-                                 C.c_int(trace_lane), C.c_int(device)), "le_td3_run_host")
-    return dict(out=out, rewards=rewards, lengths=lengths, test_rewards=test_rewards, actor_final=af, trace=trace)
+    check(_lib().le_td3_run_host(C.byref(tcfg), _hptr(th), C.c_int(0 if th is None else th.shape[0]), _hptr(ei), _hptr(keys), _hptr(a0),
+                                 _hptr(q1), _hptr(q2), C.c_int(a0.shape[0]), _hptr(res["actor_final"]), C.c_int(n), *_res_ptrs(res),
+                                 C.byref(tr) if tr is not None else None, C.c_int(trace_lane), C.c_int(device)), "le_td3_run_host")
+    return res
